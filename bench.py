@@ -4,6 +4,7 @@
   python bench.py --gpus 1 --steps K --warmup W                  # this repo (CUDA, sm_100a)
   python bench.py --impl reference --gpus N --steps K --warmup W  # the reference algorithm on the host cores
   torchrun ... bench.py --gpus N ...                              # N > 1: pixel-column shards, NCCL Gram all-reduce
+  python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR # also write what the last timed step computed (dump_outputs)
 
 A "step" is one complete decomposition of the resident clip: init norms, all ALM iterations, materialisation of L and
 the foreground mask.  `value` is timed with CUDA events with D already in HBM; `e2e` is the same job through the
@@ -42,6 +43,8 @@ WORKLOADS = {
     "synthetic_1080p_300_graph": (1080, 1920, 300, 0, 6),
     "synthetic_1080p_30_graph": (1080, 1920, 30, 0, 6),       # the first 10th of the period of that clip (the prox cost is per frame)
 }
+FLOW_WORKLOADS = ("highway_flow", "batch64_qvga_200")         # and every *_graph workload: scripts/bench_flows.py
+DUMP_SAMPLE = 1 << 22          # --dump-outputs: entries kept per matrix (3 x 16 MB of float32, within a 64 MB budget)
 
 
 def parse():
@@ -57,7 +60,14 @@ def parse():
                     help="CPU baseline: keep rows/div x cols/(2 div) of every frame (0 = 4: a 1/32 window of 1080p, ~20 s of CPU work)")
     ap.add_argument("--tile-rows", type=int, default=0)
     ap.add_argument("--cluster-frames", type=int, default=0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write L, S and the mask of the last timed step to DIR/<name>.npy (a fixed seeded sample of "
+                         "%d entries each, plus float64 per-frame sums), so that two builds can be compared output for output "
+                         "(one GPU, --impl b200; not the *_graph, highway_flow and batch64_qvga_200 workloads)" % DUMP_SAMPLE)
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -173,6 +183,25 @@ def load_video(workload):
     return synth.make_clip(rows, cols, frames, seed=seed, n_rect=nrect)[0]
 
 
+def dump_outputs(path, outputs):
+    """--dump-outputs: `outputs` maps a name to a device matrix [frames][pixels].  Each is written as DIR/<name>.npy
+    (float32): whole when it has at most DUMP_SAMPLE entries, else the entries at one seeded sample of (frame, pixel)
+    positions that is the same for every output and every run.  DIR/<name>_frame_sums.npy (float64 [frames]) holds the
+    per-frame sums of the whole matrix, so that a difference outside the sample shows too; they are device reductions
+    whose summation order is not fixed, so compare them with a tolerance, not bit for bit."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    n, m = next(iter(outputs.values())).shape
+    idx = None
+    if n * m > DUMP_SAMPLE:
+        idx = torch.from_numpy(np.sort(np.random.default_rng(0).choice(n * m, size=DUMP_SAMPLE, replace=False))).cuda()
+    for name, x in outputs.items():
+        entries = x.reshape(-1) if idx is None else x[idx // m, idx % m]
+        sums = torch.cat([x[f0:f0 + 16].to(torch.float64).sum(1) for f0 in range(0, n, 16)])
+        np.save(os.path.join(path, name + ".npy"), entries.to(torch.float32).cpu().numpy())
+        np.save(os.path.join(path, name + "_frame_sums.npy"), sums.cpu().numpy())
+
+
 def run_reference(args, rank, world):
     """--impl reference: the reference's CPU algorithm (oracle port; the reference itself is pure Python and is not
     present on the GPU box) on all host cores, bounded sample, same metric/config."""
@@ -207,6 +236,10 @@ def main():
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    flow = args.workload in FLOW_WORKLOADS or args.workload.endswith("_graph")
+    if args.dump_outputs and (args.impl != "b200" or world > 1 or flow):
+        raise SystemExit("bench.py: --dump-outputs is implemented for --impl b200 on one GPU, workloads %s"
+                         % ", ".join(w for w in sorted(WORKLOADS) if w not in FLOW_WORKLOADS and not w.endswith("_graph")))
     if args.impl == "reference":
         out = run_reference(args, rank, world)
         if out is not None:
@@ -224,7 +257,7 @@ def main():
     torch.cuda.set_device(local_rank)
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
-    if args.workload in ("highway_flow", "batch64_qvga_200") or args.workload.endswith("_graph"):
+    if flow:
         sys.path.insert(0, os.path.join(ROOT, "scripts"))
         import bench_flows
         if args.workload == "highway_flow":
@@ -332,6 +365,8 @@ def main():
     ms_step = float(tmax.item()) / args.steps
     st = solver.status()
     iters = int(st.iter)
+    if args.dump_outputs:                   # before the e2e leg below reloads this solver handle
+        dump_outputs(args.dump_outputs, {"L": solver.dec.device_tensor('L'), "S": solver.dec.device_tensor('S'), "mask": mask})
 
     info = solver.dec.debug_info()
 
