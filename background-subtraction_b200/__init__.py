@@ -8,7 +8,7 @@ from .api import (BLOCK_SIZE, Decomposition, center_window_decomposition, LSD, a
                   get_proximal_graph_group_centers, gram,
                   group_sparse_decomposition, inexact_alm_group_sparse_RPCA, inexact_alm_lsd,
                   inexact_alm_lsd_batch, inexact_alm_lsd_with_background, inexact_alm_rpca,
-                  labels_from_blocks, lsd_decomposition, make_config, normalizeImage, prox, prox_by_frame, prox_flat,
+                  labels_from_blocks, lsd_decomposition, make_config, normalizeImage, pack_graphs, prox, prox_by_frame, prox_flat,
                   resize_with_cv2, svd_k_largest, window_csc, with_background_decomposition)
 from .flow import (LSD_improved, apply_morph_ops, compute_RPCA, executeSaliencyRPCA, inexact_alm_rpca_batch, build_improved_LSD_graphs, calc_mask_percent, computeSCube, connected_components,
                    filter_sparse_map, gkern, improved_LSD_weight_mask, merge_masks, motion_saliency_blocks,

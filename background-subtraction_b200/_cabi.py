@@ -35,7 +35,7 @@ class IterLog(ctypes.Structure):
                 ("err", ctypes.c_double), ("mu", ctypes.c_double), ("nnz", ctypes.c_uint64)]
 
 
-PROX_FLAT_LINF, PROX_GRAPH_LINF, PROX_BLOCK_L2, PROX_L1, PROX_GRAPH_CENTER_BG = 0, 1, 2, 3, 4
+PROX_FLAT_LINF, PROX_GRAPH_LINF, PROX_BLOCK_L2, PROX_L1, PROX_GRAPH_CENTER_BG, PROX_GRAPH_GENERIC = 0, 1, 2, 3, 4, 5
 FLAG_ALWAYS_STORE_S = 1
 
 # every symbol include/bsub_b200.h declares: name -> (restype, argtypes)
@@ -50,6 +50,8 @@ SIGNATURES = {
     "bsub_set_graph_windows": (ctypes.c_int, [vp, c_double_p, ctypes.c_int64]),
     "bsub_set_blocks": (ctypes.c_int, [vp, c_uint8_p, c_int32_p, c_double_p]),
     "bsub_set_center_windows": (ctypes.c_int, [vp, c_float_p, c_uint8_p]),
+    "bsub_set_graphs": (ctypes.c_int, [vp, ctypes.c_int32, c_int32_p, c_int64_p, ctypes.POINTER(c_int32_p), ctypes.POINTER(c_int32_p),
+                                       ctypes.POINTER(c_double_p), c_uint8_p]),
     "bsub_load_D_f64_host": (ctypes.c_int, [vp, vp, ctypes.c_int64, vp]),
     "bsub_load_D_f32_host": (ctypes.c_int, [vp, vp, ctypes.c_int64, vp]),
     "bsub_load_D_f32_dev": (ctypes.c_int, [vp, vp, ctypes.c_int64, vp]),
@@ -93,6 +95,9 @@ SIGNATURES = {
                                             c_double_p, ctypes.c_int32, ctypes.c_double, c_int32_p, vp]),
     "bsub_prox_center3_dev": (ctypes.c_int, [vp, vp, ctypes.c_int64, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_double,
                               c_float_p, ctypes.c_int32, ctypes.c_double, c_int32_p, vp]),
+    "bsub_prox_graph_dev": (ctypes.c_int, [vp, vp, ctypes.c_int64, ctypes.c_int64, ctypes.c_int32, ctypes.c_double, ctypes.c_int32, c_int32_p,
+                                           c_int64_p, ctypes.POINTER(c_int32_p), ctypes.POINTER(c_int32_p), ctypes.POINTER(c_double_p),
+                                           ctypes.c_int32, ctypes.c_double, c_int32_p, vp]),
     "bsub_block_shrink_dev": (ctypes.c_int, [vp, vp, ctypes.c_int64, ctypes.c_int64, ctypes.c_int32, c_uint8_p, c_int32_p, c_double_p,
                                              ctypes.c_double, ctypes.c_double, vp]),
     "bsub_gram_dev": (ctypes.c_int, [vp, vp, vp, ctypes.c_int64, ctypes.c_int64, ctypes.c_int32, ctypes.c_double, c_double_p, vp]),

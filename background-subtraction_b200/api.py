@@ -135,6 +135,8 @@ def detect_center_windows(graph, m, img_shape=None):
             continue
         if ng == 0:
             return (rows, cols), np.zeros(m, dtype=np.float32)
+        if np.any(np.diff(ptr) == 0):                  # a centre window is never empty (e.g. the 1 x k windows of the last row)
+            return None
         first, size = idx[ptr[:-1]], np.diff(ptr)
         i0, j0 = first % rows, first // rows
         # height of the window = length of the first run of consecutive indices
@@ -144,7 +146,7 @@ def detect_center_windows(graph, m, img_shape=None):
         ww = size // np.maximum(hh, 1)
         ci = np.where(hh == 3, i0 + 1, np.where(i0 == 0, 0, rows - 1)) if rows > 2 else None
         cj = np.where(ww == 3, j0 + 1, np.where(j0 == 0, 0, cols - 1)) if cols > 2 else None
-        if ci is None or cj is None:
+        if ci is None or cj is None or np.any(ci >= rows) or np.any(cj >= cols):   # the latter: not a centre-window graph
             continue
         emap = np.zeros((rows, cols), dtype=np.float64)
         emap[ci, cj] = eta
@@ -201,6 +203,66 @@ def detect_window_graph(graph, m, img_shape=None):
                 return None
             return rows, cols, np.ascontiguousarray(graph['eta_g'], dtype=np.float64)
     return None
+
+
+def _is_graph_list(graphs):
+    return isinstance(graphs, (list, tuple)) or (isinstance(graphs, np.ndarray) and graphs.dtype == object)
+
+
+def pack_graphs(graphs, m, n):
+    """SPAMS graph dict, or a list of them with one per frame -> (csc, frame_graph): csc = list of distinct
+    (indptr int32, indices int32, eta float64) triples, frame_graph int32[n] = which of them each frame uses.  A graph shared
+    by several frames (the same object, or equal CSC arrays) is stored once.  Raises on nested groups (SPAMS DAG semantics
+    are not restated), a variable count other than m, pixel indices out of range or twice in a group, and eta that is
+    negative, non-finite or of the wrong length."""
+    import hashlib
+    glist = list(graphs) if _is_graph_list(graphs) else [graphs] * n
+    if len(glist) != n:
+        raise Exception("graphs must hold one graph per frame (%d graphs, %d frames)" % (len(glist), n))
+    csc, frame_graph, by_id, by_hash = [], np.empty(n, dtype=np.int32), {}, {}
+    for f, g in enumerate(glist):
+        if id(g) in by_id:
+            frame_graph[f] = by_id[id(g)]
+            continue
+        nested = g.get('groups', None)
+        if nested is not None and getattr(nested, 'nnz', 0) != 0:
+            raise Exception("frame %d: the graph has nested groups (graph['groups'] is not empty); only flat group "
+                            "structures are implemented" % f)
+        gv = g['groups_var'].tocsc()
+        if gv.shape[0] != m:
+            raise Exception("graph has %d variables, matrix has %d rows" % (gv.shape[0], m))
+        ip = np.ascontiguousarray(gv.indptr, dtype=np.int32)
+        ix = np.ascontiguousarray(gv.indices, dtype=np.int32)
+        eta = np.ascontiguousarray(np.asarray(g['eta_g'], dtype=np.float64).ravel())
+        ng = len(ip) - 1
+        if eta.size != ng:
+            raise Exception("frame %d: eta_g has %d entries, the graph has %d groups" % (f, eta.size, ng))
+        if not np.all(np.isfinite(eta) & (eta >= 0)):
+            raise Exception("frame %d: eta_g must be finite and >= 0" % f)
+        if ix.size and (ix.min() < 0 or ix.max() >= m):
+            raise Exception("frame %d: group pixel index out of range [0, %d)" % (f, m))
+        owner = np.repeat(np.arange(ng, dtype=np.int64), np.diff(ip))
+        if np.unique(owner * m + ix).size != ix.size:
+            raise Exception("frame %d: a group holds the same pixel twice" % f)
+        key = hashlib.sha1(ip.tobytes() + b'|' + ix.tobytes() + b'|' + eta.tobytes()).digest()
+        k = by_hash.get(key)
+        if k is None or not all(np.array_equal(a, b) for a, b in zip(csc[k], (ip, ix, eta))):
+            k = len(csc)
+            csc.append((ip, ix, eta))
+            by_hash[key] = k
+        by_id[id(g)] = k
+        frame_graph[f] = k
+    return csc, frame_graph
+
+
+def _graph_pointers(csc):
+    """ctypes arrays of bsub_set_graphs / bsub_prox_graph_dev for the triples of pack_graphs (which must stay alive)."""
+    k = len(csc)
+    ng = np.array([len(c[0]) - 1 for c in csc], dtype=np.int64)
+    ip = (C.c_int32_p * k)(*[c[0].ctypes.data_as(C.c_int32_p) for c in csc])
+    ix = (C.c_int32_p * k)(*[c[1].ctypes.data_as(C.c_int32_p) for c in csc])
+    et = (C.c_double_p * k)(*[c[2].ctypes.data_as(C.c_double_p) for c in csc])
+    return ng, ip, ix, et
 
 
 # --------------------------------------------------------------------------------------------------------------
@@ -332,6 +394,14 @@ class Decomposition:
             e = np.ascontiguousarray(eta, dtype=np.float64)
             C.check(self.lib.bsub_set_graph_windows(self.h, e.ctypes.data_as(C.c_double_p), e.size))
 
+    def set_graphs(self, csc, frame_graph, background=None):
+        """Any graphs (PROX_GRAPH_GENERIC): csc / frame_graph as returned by pack_graphs; background uint8[n][m] or None."""
+        fg = np.ascontiguousarray(frame_graph, dtype=np.int32)
+        ng, ip, ix, et = _graph_pointers(csc)
+        bg = None if background is None else np.ascontiguousarray(background, dtype=np.uint8)
+        C.check(self.lib.bsub_set_graphs(self.h, len(csc), fg.ctypes.data_as(C.c_int32_p), ng.ctypes.data_as(C.c_int64_p), ip, ix, et,
+                                         None if bg is None else bg.ctypes.data_as(C.c_uint8_p)))
+
     def set_blocks(self, labels, lam_ptr, lam):
         labels = np.ascontiguousarray(labels, dtype=np.uint8)
         lam_ptr = np.ascontiguousarray(lam_ptr, dtype=np.int32)
@@ -442,6 +512,13 @@ def _shape_of(D0):
     return np.shape(D0)
 
 
+def _geometry(img_shape, m):
+    """(rows, cols) of img_shape when it describes the m pixels, else (0, 0) (the generic graph mode needs no geometry)."""
+    if img_shape is not None and int(img_shape[0]) * int(img_shape[1]) == m:
+        return int(img_shape[0]), int(img_shape[1])
+    return 0, 0
+
+
 def _finish(dec, D0, verbose):
     st = dec.status()
     if verbose:
@@ -478,7 +555,7 @@ def lsd_decomposition(D0, graphs=None, groups=None, delta=10, img_shape=None, ma
         dec = Decomposition(cfg)
         dec.set_flat_groups(groups)
     else:
-        if isinstance(graphs, (list, tuple)) or (isinstance(graphs, np.ndarray) and graphs.dtype == object):
+        if _is_graph_list(graphs):
             glist = list(graphs)
             if len(glist) != n:
                 raise Exception("graphs must hold one graph per frame")
@@ -486,14 +563,19 @@ def lsd_decomposition(D0, graphs=None, groups=None, delta=10, img_shape=None, ma
             same = first is not None and all(
                 (g is glist[0]) or (detect_window_graph(g, m, img_shape) is not None and
                                     np.array_equal(g['eta_g'], glist[0]['eta_g'])) for g in glist[1:])
-            if not same:
-                raise Exception("per-frame graphs that differ between frames (inexact_alm_lsd_with_background) are not "
-                                "implemented in this build")
-            geo = first
+            geo = first if same else None
         else:
             geo = detect_window_graph(graphs, m, img_shape)
-        if geo is None:
-            raise Exception("only the overlapping 3x3 all-windows graph of getGraphSPAMS_all_groups is implemented")
+        if geo is None:                                  # any other graph, or per-frame graphs that differ
+            csc, frame_graph = pack_graphs(graphs, m, n)
+            rows, cols = _geometry(img_shape, m)
+            cfg = make_config(m, n, C.PROX_GRAPH_GENERIC, rows, cols, delta=delta, max_iter=max_iter, tile_rows=tile_rows,
+                              cluster_frames=cluster_frames, graph_max_sweeps=graph_max_sweeps, graph_tol=graph_tol)
+            dec = Decomposition(cfg)
+            dec.set_graphs(csc, frame_graph)
+            dec.load(D0)
+            dec.run()
+            return dec
         rows, cols, eta = geo
         cfg = make_config(m, n, C.PROX_GRAPH_LINF, rows, cols, delta=delta, max_iter=max_iter, tile_rows=tile_rows,
                           cluster_frames=cluster_frames, graph_max_sweeps=graph_max_sweeps, graph_tol=graph_tol)
@@ -557,11 +639,12 @@ def with_background_decomposition(D0, graphs, background_masks, delta=10, img_sh
         raise Exception("graphs and background_masks must have one entry per frame")
     eta = np.empty((n, m), dtype=np.float32)
     shape = tuple(img_shape) if img_shape is not None else None
+    generic = False
     for f in range(n):
         det = detect_center_windows(graphs[f], m, shape)
-        if det is None:
-            raise Exception("frame %d: only the radius-1 centre-window graphs of get_proximal_graph_group_centers are "
-                            "implemented in this build" % f)
+        if det is None:                                  # not a radius-1 centre-window graph: the generic graph mode
+            generic = True
+            break
         if shape is None or graphs[f].get('_group_centers', None) is not None:
             shape = det[0] if shape is None else shape
         if det[0] != tuple(shape):
@@ -570,6 +653,14 @@ def with_background_decomposition(D0, graphs, background_masks, delta=10, img_sh
     bg = np.ascontiguousarray(np.stack([np.asarray(b, dtype=bool).ravel() for b in background_masks]).astype(np.uint8))
     if bg.shape != (n, m):
         raise Exception("background_masks must hold %d boolean masks of %d pixels" % (n, m))
+    if generic:
+        csc, frame_graph = pack_graphs(graphs, m, n)
+        rows, cols = _geometry(img_shape, m)
+        dec = Decomposition(make_config(m, n, C.PROX_GRAPH_GENERIC, rows, cols, delta=delta, **tuning))
+        dec.set_graphs(csc, frame_graph, bg)
+        dec.load(D0)
+        dec.run()
+        return dec
     cfg = make_config(m, n, C.PROX_GRAPH_CENTER_BG, shape[0], shape[1], delta=delta, **tuning)
     dec = Decomposition(cfg)
     C.check(dec.lib.bsub_set_center_windows(dec.h, eta.ctypes.data_as(C.c_float_p), bg.ctypes.data_as(C.c_uint8_p)))
@@ -752,15 +843,15 @@ def prox_flat(G_S, lambda1, groups, num_threads=None, img_shape=None):
 
 
 def prox(G_S, lambda1, graph, num_threads=None, img_shape=None, max_sweeps=20000, tol=1e-7, return_sweeps=False):
-    """/root/reference/inexact_alm_lsd.py:49-57 (overlapping 3x3 all-windows graph)."""
+    """/root/reference/inexact_alm_lsd.py:49-57: the 3x3 all-windows graph and the radius-1 centre-window graphs on their
+    dedicated kernels, any other graph on the generic one."""
     torch = _require_cuda()
     m, n = _shape_of(G_S)
     geo = detect_window_graph(graph, m, img_shape)
     if geo is None:
         ctr = detect_center_windows(graph, m, img_shape)           # a per-frame graph of get_proximal_graph_group_centers
         if ctr is None:
-            raise Exception("only the overlapping 3x3 all-windows graph of getGraphSPAMS_all_groups and the radius-1 "
-                            "centre-window graphs of get_proximal_graph_group_centers are implemented")
+            return _prox_generic(G_S, lambda1, graph, max_sweeps, tol, return_sweeps)
         return _prox_center(G_S, lambda1, ctr[0], np.tile(ctr[1], (n, 1)), max_sweeps, tol, return_sweeps)
     rows, cols, eta = geo
     lib = C.load()
@@ -791,13 +882,34 @@ def _prox_center(G_S, lambda1, shape, eta_nm, max_sweeps=20000, tol=1e-7, return
     return (out, sw.value) if return_sweeps else out
 
 
+def _prox_generic(G_S, lambda1, graphs, max_sweeps=20000, tol=1e-7, return_sweeps=False):
+    """Any graph, or one graph per frame (pack_graphs); all frames in one launch."""
+    torch = _require_cuda()
+    m, n = _shape_of(G_S)
+    csc, frame_graph = pack_graphs(graphs, m, n)
+    ng, ip, ix, et = _graph_pointers(csc)
+    lib = C.load()
+    u, ld = _to_device_f32(G_S, m, n)
+    v = torch.zeros_like(u)
+    sw = ctypes.c_int32(0)
+    C.check(lib.bsub_prox_graph_dev(ctypes.c_void_p(u.data_ptr()), ctypes.c_void_p(v.data_ptr()), ld, m, n, float(lambda1), len(csc),
+                                    frame_graph.ctypes.data_as(C.c_int32_p), ng.ctypes.data_as(C.c_int64_p), ip, ix, et,
+                                    int(max_sweeps), float(tol) * float(lambda1), ctypes.byref(sw), _stream_ptr()))
+    out = _op_out(v, m, G_S)
+    return (out, sw.value) if return_sweeps else out
+
+
 def prox_by_frame(G_S, lambda1, graphs, img_shape=None):
     """/root/reference/inexact_alm_lsd.py:60-68: one graph per column.  Centre-window graphs (the per-frame graphs the
-    reference builds) go through one launch for all frames; anything else frame by frame through prox()."""
+    reference builds) go through one launch for all frames, as does any list with a graph the dedicated kernels do not take;
+    lists of 3x3 all-window and radius-1 centre-window graphs go frame by frame through prox()."""
     m, n = _shape_of(G_S)
-    dets = [detect_center_windows(g, m, img_shape) if detect_window_graph(g, m, img_shape) is None else None for g in graphs]
+    win = [detect_window_graph(g, m, img_shape) is not None for g in graphs]
+    dets = [detect_center_windows(g, m, img_shape) if not w else None for g, w in zip(graphs, win)]
     if len(dets) == n and all(d is not None for d in dets) and len({d[0] for d in dets}) == 1:
         return _prox_center(G_S, lambda1, dets[0][0], np.stack([d[1] for d in dets]))
+    if len(dets) != n or not all(w or d is not None for w, d in zip(win, dets)):
+        return _prox_generic(G_S, lambda1, list(graphs))
     cols = [prox(G_S[:, [f]], lambda1, graphs[f], img_shape=img_shape) for f in range(n)]
     return np.column_stack(cols)
 

@@ -187,4 +187,32 @@ int launch_prox_graph3(const float* U, float* V, float* xi, long long xi_floats,
                        int cols, int n, float lam, int max_sweeps, float tol, int* sweeps_out, const DevState* st,
                        cudaStream_t s, int center = 0, long long eta_stride = 0);
 
+// ---------------------------------------------------------------- prox_graph.cu (any non-nested graph, one graph per frame)
+// Graphs coloured and stored colour-major by pack_generic_graphs: graph gr owns colours [gcol[gr], gcol[gr+1]); colour c owns
+// groups [cbeg[c], cbeg[c+1]), of which [cbig[c], cbeg[c+1]) have more than 32 pixels; group g owns gidx[gptr[g] .. gptr[g+1])
+// and its dual entries are the same positions minus gnz0[gr].
+struct GenericGraphHost {
+    std::vector<int> frame_graph, gcol, cbeg, cbig, gptr, gidx, gnz0;
+    std::vector<float> eta;
+    long long max_nnz = 0; int max_colours = 0;
+};
+struct GenericGraphDev {
+    const int *frame_graph, *gcol, *cbeg, *cbig, *gptr, *gidx, *gnz0;
+    const float* eta;
+    long long max_nnz;
+};
+// where the per-pixel dual sums live (cs CTAs per cluster, 1 << shift pixels each, or global rows) and the workspace that takes
+struct GenericGraphLayout { int cs, shift, slots; bool tot_global; long long xi_floats, tot_floats; size_t smem; };
+// validates every input (bad input: error message, nothing launched), colours each graph and lays it out
+int pack_generic_graphs(long long m, int n, int n_graphs, const int32_t* frame_graph, const int64_t* n_groups,
+                        const int32_t* const* indptr, const int32_t* const* indices, const double* const* eta, GenericGraphHost* out,
+                        const char* who);
+// one device allocation for the index arrays (*ints) and one for eta; frees what the pointers held before
+int upload_generic_graphs(const GenericGraphHost& H, int** ints, float** eta_dev, GenericGraphDev* dev);
+// duals: BSUB_GRAPH_XI_MB cap (default 8 GB) on the clusters in flight
+GenericGraphLayout prox_graph_generic_layout(long long m, long long ld, int n, long long max_nnz);
+// status: the caller's zeroed int[8] ([0] sweeps of the last call, [4..6] running totals as for launch_prox_graph3)
+int launch_prox_graph_generic(const float* U, float* V, long long ld, long long m, int n, const GenericGraphDev& g, const GenericGraphLayout& L,
+                              float* xi, float* totg, float lam, int max_sweeps, float tol, int* status, const DevState* st, cudaStream_t s);
+
 }  // namespace bsub

@@ -67,6 +67,8 @@ struct bsub_solver {
     float* eta_dev = nullptr; float* xi = nullptr; long long xi_floats = 0; float* tot = nullptr;
     float* xi2 = nullptr; float* tot2 = nullptr; int* sweeps2 = nullptr; long long xi2_floats = 0, tot2_floats = 0;   // bsub_step_prox_frames
     int* sweeps_dev = nullptr; bool graph_set = false;
+    // any graphs (BSUB_PROX_GRAPH_GENERIC): packed index arrays + eta on the device, where tot lives; xi / tot / sweeps_dev above
+    int* pg_ints = nullptr; float* pg_eta = nullptr; GenericGraphDev pg_dev; GenericGraphLayout pg_layout; bool pg_bg = false;
     // l2 blocks
     unsigned char* labels_dev = nullptr; double* lam_table = nullptr; double* bsums = nullptr; int nlab = 0; bool blocks_set = false;
     unsigned char* mask_stage = nullptr;      // bsub_mask_host staging
@@ -135,7 +137,8 @@ int bsub_destroy(bsub_solver* s) {
     void* ptrs[] = {s->D, s->S, s->Y, s->T, s->L, s->U, s->st, s->log, s->comm_sum, s->comm_max, s->tasks_dev, s->gram_partial,
                     s->eb.work, s->eb.lam, s->eb.Z, s->eb.Vr, s->eb.VC, s->tpart, s->part_zz, s->part_nnz, s->part_max, s->gptr,
                     s->gidx, s->eta_dev, s->xi, s->tot, s->sweeps_dev, s->labels_dev, s->lam_table, s->bsums, s->Wq, s->Gint,
-                    s->gi_info, s->gi_blkn, s->part_wmax, s->mask_stage, s->mask_scratch, s->stage64, s->Tt, s->xi2, s->tot2, s->sweeps2};
+                    s->gi_info, s->gi_blkn, s->part_wmax, s->mask_stage, s->mask_scratch, s->stage64, s->Tt, s->xi2, s->tot2, s->sweeps2,
+                    s->pg_ints, s->pg_eta};
     for (void* p : ptrs) if (p) cudaFree(p);
     if (s->mirror) cudaFreeHost((void*)s->mirror);
     for (int i = 0; i <= kRunAhead; ++i) if (s->ev[i]) cudaEventDestroy(s->ev[i]);
@@ -148,7 +151,7 @@ int bsub_destroy(bsub_solver* s) {
 int bsub_create(const bsub_config* cfg, bsub_solver** out) {
     if (!cfg || !out) { set_error("bsub_create: null argument"); return -1; }
     if (cfg->m <= 0 || cfg->n <= 0) { set_error("bsub_create: empty matrix (m=%lld, n=%d)", (long long)cfg->m, cfg->n); return -1; }
-    if (cfg->prox < 0 || cfg->prox > 4) { set_error("bsub_create: unknown prox %d", cfg->prox); return -1; }
+    if (cfg->prox < 0 || cfg->prox > 5) { set_error("bsub_create: unknown prox %d", cfg->prox); return -1; }
     if ((cfg->prox == BSUB_PROX_FLAT_LINF || cfg->prox == BSUB_PROX_GRAPH_LINF || cfg->prox == BSUB_PROX_GRAPH_CENTER_BG) &&
         ((long long)cfg->rows * cfg->cols != cfg->m)) {
         set_error("bsub_create: rows*cols (%d*%d) != m (%lld)", cfg->rows, cfg->cols, (long long)cfg->m); return -1;
@@ -371,6 +374,34 @@ int bsub_set_center_windows(bsub_solver* s, const float* eta, const uint8_t* bac
     return 0;
 }
 
+int bsub_set_graphs(bsub_solver* s, int32_t n_graphs, const int32_t* frame_graph, const int64_t* n_groups, const int32_t* const* indptr,
+                    const int32_t* const* indices, const double* const* eta, const uint8_t* background) {
+    if (!s) { set_error("bsub_set_graphs: null solver"); return -1; }
+    if (s->cfg.prox != BSUB_PROX_GRAPH_GENERIC) { set_error("bsub_set_graphs: solver was not created with BSUB_PROX_GRAPH_GENERIC"); return -1; }
+    GenericGraphHost H;
+    RET_IF(pack_generic_graphs(s->m, s->n, n_graphs, frame_graph, n_groups, indptr, indices, eta, &H, "bsub_set_graphs"));
+    RET_IF(upload_generic_graphs(H, &s->pg_ints, &s->pg_eta, &s->pg_dev));
+    s->pg_layout = prox_graph_generic_layout(s->m, s->ld, s->n, H.max_nnz);
+    if (s->xi) { cudaFree(s->xi); s->xi = nullptr; }
+    if (s->tot) { cudaFree(s->tot); s->tot = nullptr; }
+    CK(cudaMalloc((void**)&s->xi, sizeof(float) * (size_t)s->pg_layout.xi_floats));
+    if (s->pg_layout.tot_floats > 0) CK(cudaMalloc((void**)&s->tot, sizeof(float) * (size_t)s->pg_layout.tot_floats));
+    s->xi_floats = s->pg_layout.xi_floats;
+    s->pg_bg = background != nullptr;
+    if (s->pg_bg) {           // label 0 = background (the complement group of the l2 kernels), 255 = keeps the graph prox result
+        const size_t nm = (size_t)s->n * s->m;
+        std::vector<unsigned char> lab(nm);
+        for (size_t i = 0; i < nm; ++i) lab[i] = background[i] ? 0 : 255;
+        if (!s->labels_dev) CK(cudaMalloc((void**)&s->labels_dev, nm));
+        if (!s->bsums) CK(cudaMalloc((void**)&s->bsums, sizeof(double) * s->n));
+        CK(cudaMemcpy(s->labels_dev, lab.data(), nm, cudaMemcpyHostToDevice));
+        s->nlab = 1;
+    }
+    if (!s->sweeps_dev) { CK(cudaMalloc((void**)&s->sweeps_dev, sizeof(int) * 8)); CK(cudaMemset(s->sweeps_dev, 0, sizeof(int) * 8)); }
+    s->graph_set = true;
+    return 0;
+}
+
 int bsub_set_blocks(bsub_solver* s, const uint8_t* labels, const int32_t* lam_ptr, const double* lam) {
     if (!s || !labels || !lam_ptr) { set_error("bsub_set_blocks: null argument"); return -1; }
     if (s->cfg.prox != BSUB_PROX_BLOCK_L2) { set_error("bsub_set_blocks: solver was not created with BSUB_PROX_BLOCK_L2"); return -1; }
@@ -509,7 +540,8 @@ static int check_ready(bsub_solver* s) {
     if (!s) { set_error("null solver"); return -1; }
     if (!s->loaded) { set_error("no data loaded (call bsub_load_* first)"); return -1; }
     if (s->cfg.prox == BSUB_PROX_FLAT_LINF && !s->groups_set) { set_error("one of graphs or groups must not be None"); return -1; }
-    if ((s->cfg.prox == BSUB_PROX_GRAPH_LINF || s->cfg.prox == BSUB_PROX_GRAPH_CENTER_BG) && !s->graph_set) { set_error("one of graphs or groups must not be None"); return -1; }
+    if ((s->cfg.prox == BSUB_PROX_GRAPH_LINF || s->cfg.prox == BSUB_PROX_GRAPH_CENTER_BG || s->cfg.prox == BSUB_PROX_GRAPH_GENERIC) &&
+        !s->graph_set) { set_error("one of graphs or groups must not be None"); return -1; }
     if (s->cfg.prox == BSUB_PROX_BLOCK_L2 && !s->blocks_set) { set_error("blocks_by_frame / lambdas_by_frame not set"); return -1; }
     return 0;
 }
@@ -652,6 +684,13 @@ static int step_shrink_impl(bsub_solver* s, void* stream, int part) {
                                       s->cfg.graph_max_sweeps, (float)s->cfg.graph_tol, s->sweeps_dev, s->st, st, 1, s->m));
             RET_IF(launch_block_l2_sums(s->U, s->labels_dev, s->ld, s->m, s->n, 1, s->bsums, s->st, st));
             RET_IF(launch_block_l2_apply(s->U, s->S, s->labels_dev, s->ld, s->m, s->n, 1, s->bsums, nullptr, s->st, 0.0, 0.0, st, 1));
+        } else if (s->cfg.prox == BSUB_PROX_GRAPH_GENERIC) {
+            RET_IF(launch_prox_graph_generic(s->U, s->S, s->ld, s->m, s->n, s->pg_dev, s->pg_layout, s->xi, s->tot, 0.f, s->cfg.graph_max_sweeps,
+                                             (float)s->cfg.graph_tol, s->sweeps_dev, s->st, st));
+            if (s->pg_bg) {
+                RET_IF(launch_block_l2_sums(s->U, s->labels_dev, s->ld, s->m, s->n, 1, s->bsums, s->st, st));
+                RET_IF(launch_block_l2_apply(s->U, s->S, s->labels_dev, s->ld, s->m, s->n, 1, s->bsums, nullptr, s->st, 0.0, 0.0, st, 1));
+            }
         } else {   // BSUB_PROX_BLOCK_L2
             RET_IF(launch_block_l2_sums(s->U, s->labels_dev, s->ld, s->m, s->n, s->nlab, s->bsums, s->st, st));
             if (part == 1) return 0;                       // the driver all-reduces bsums, then calls part 2
@@ -1024,6 +1063,34 @@ int bsub_prox_center3_dev(const float* U, float* V, int64_t ld, int32_t rows, in
     CK(cudaMemcpy(eta, eta_host, sizeof(float) * (size_t)n * m, cudaMemcpyHostToDevice));
     RET_IF(launch_prox_graph3(U, V, xi, xi_floats, tot, eta, ld, rows, cols, n, (float)lambda1, max_sweeps > 0 ? max_sweeps : 4000, (float)tol, sw,
                               nullptr, st, 1, m));
+    int sw_h = 0;
+    CK(cudaMemcpyAsync(&sw_h, sw, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if (sweeps_used) *sweeps_used = sw_h;
+    return 0;
+}
+
+int bsub_prox_graph_dev(const float* U, float* V, int64_t ld, int64_t m, int32_t n, double lambda1, int32_t n_graphs, const int32_t* frame_graph,
+                        const int64_t* n_groups, const int32_t* const* indptr, const int32_t* const* indices, const double* const* eta,
+                        int32_t max_sweeps, double tol, int32_t* sweeps_used, void* stream) {
+    GenericGraphHost H;                                   // validation first: bad input never reaches the device
+    RET_IF(pack_generic_graphs(m, n, n_graphs, frame_graph, n_groups, indptr, indices, eta, &H, "bsub_prox_graph_dev"));
+    if (!U || !V || ld < m) { set_error("bsub_prox_graph_dev: bad argument"); return -1; }
+    cudaStream_t st = as_stream(stream);
+    DevScope mem;
+    int* ints = nullptr; float* eta_d = nullptr;
+    GenericGraphDev gd;
+    const int rc = upload_generic_graphs(H, &ints, &eta_d, &gd);
+    mem.ptrs.push_back(ints); mem.ptrs.push_back(eta_d);
+    if (rc != 0) return rc;
+    const GenericGraphLayout L = prox_graph_generic_layout(m, ld, n, H.max_nnz);
+    float *xi = nullptr, *tot = nullptr; int* sw = nullptr;
+    RET_IF(mem.alloc(&xi, sizeof(float) * (size_t)L.xi_floats));
+    if (L.tot_floats > 0) RET_IF(mem.alloc(&tot, sizeof(float) * (size_t)L.tot_floats));
+    RET_IF(mem.alloc(&sw, sizeof(int) * 8));
+    CK(cudaMemsetAsync(sw, 0, sizeof(int) * 8, st));
+    RET_IF(launch_prox_graph_generic(U, V, ld, m, n, gd, L, xi, tot, (float)lambda1, max_sweeps > 0 ? max_sweeps : 4000, (float)tol, sw,
+                                     nullptr, st));
     int sw_h = 0;
     CK(cudaMemcpyAsync(&sw_h, sw, sizeof(int), cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));

@@ -31,9 +31,12 @@ enum {
     BSUB_PROX_GRAPH_LINF = 1,  /* spams.proximalGraph 'graph' (overlapping)   inexact_alm_lsd.py:49-57,159     */
     BSUB_PROX_BLOCK_L2 = 2,    /* block_shrinkage_operator                    group_sparse_RPCA.py:13-42       */
     BSUB_PROX_L1 = 3,          /* elementwise soft threshold                  lsd_improvement.py:176           */
-    BSUB_PROX_GRAPH_CENTER_BG = 4 /* per-frame windows centred on weighted pixels (prox_by_frame, inexact_alm_lsd.py:60-68,
+    BSUB_PROX_GRAPH_CENTER_BG = 4, /* per-frame windows centred on weighted pixels (prox_by_frame, inexact_alm_lsd.py:60-68,
                                   graphs of lsd_improvement.py:74-120) + l2 shrink of each frame's background
                                   (lsd_improvement.py:199-212): inexact_alm_lsd_with_background, lsd_improvement.py:215-304 */
+    BSUB_PROX_GRAPH_GENERIC = 5   /* spams.proximalGraph 'graph' for ANY non-nested graph, one graph per frame (bsub_set_graphs),
+                                     optionally + the l2 shrink of each frame's background: every graph the reference accepts in
+                                     inexact_alm_lsd / prox_by_frame / inexact_alm_lsd_with_background */
 };
 
 /* Replaces the hard-coded constants of inexact_alm_lsd.py:102-125 / group_sparse_RPCA.py:53-77. */
@@ -111,6 +114,14 @@ int bsub_set_blocks(bsub_solver* s, const uint8_t* labels_host, const int32_t* l
  * centred on that pixel in that frame (<= 0: no window; get_proximal_graph_group_centers, lsd_improvement.py:74-120),
  * background_host uint8[n][m] != 0 where the pixel belongs to the frame's background mask (lsd_improvement.py:434). */
 int bsub_set_center_windows(bsub_solver* s, const float* eta_host, const uint8_t* background_host);
+/* any graphs (BSUB_PROX_GRAPH_GENERIC): n_graphs SPAMS-style CSC groups_var matrices as the reference builds them -- graph k has
+ * n_groups[k] groups, group g of it holds the pixels indices[k][indptr[k][g] .. indptr[k][g+1]) (0-based, < m, no pixel twice) and
+ * weighs eta[k][g] (finite, >= 0); frame f uses graph frame_graph[f] (NULL: all frames use graph 0, n_graphs must be 1).
+ * background_host uint8[n][m] (may be NULL): != 0 marks the frame's background pixels, which get the l2 shrink at
+ * 100 lambda / mu after the prox (inexact_alm_lsd_with_background).  The library colours the graphs itself; the arrays are
+ * copied, and every entry is validated before anything reaches the device. */
+int bsub_set_graphs(bsub_solver* s, int32_t n_graphs, const int32_t* frame_graph, const int64_t* n_groups, const int32_t* const* indptr,
+                    const int32_t* const* indices, const double* const* eta, const uint8_t* background_host);
 
 /* ---- data in ---------------------------------------------------------------------------------------------- */
 int bsub_load_D_f64_host(bsub_solver* s, const double* D, int64_t ld, void* stream);      /* host float64 (NumPy)   */
@@ -172,7 +183,7 @@ int bsub_debug_info(bsub_solver* s, int32_t* out16);   /* ..., [12] plane projec
  * [4] Gram mode of the next iteration (0 fp64 DMMA, 1 int8 tcgen05), [5] last digit pass saturated, [6] the solve has switched
  * to the fp64 Gram for accuracy, [7] 1e6 * bound of the int8 Gram's truncation error relative to (1/mu)^2 */
 int bsub_debug_counters(bsub_solver* s, int64_t* out8);
-/* overlapping-window prox of this handle: out4 = {outer iterations of the last call, their total over all calls, calls, calls that hit graph_max_sweeps} */
+/* overlapping-window / generic graph prox of this handle: out4 = {outer iterations of the last call, their total over all calls, calls, calls that hit graph_max_sweeps} */
 int bsub_debug_graph(bsub_solver* s, int64_t* out4);
 /* foreground_mask(D, L, S, sigmas) of utils.py:139-149 on the solver's own D, L, S; mask uint8[n][m] on the host */
 int bsub_mask_stats_local(bsub_solver* s, int phase /*0: max|S|, 1: count/sum/sumsq*/, void* stream);
@@ -196,6 +207,12 @@ int bsub_prox_graph3_dev(const float* U, float* V, int64_t ld, int32_t rows, int
  * that pixel of that frame (<= 0: no window) */
 int bsub_prox_center3_dev(const float* U, float* V, int64_t ld, int32_t rows, int32_t cols, int32_t n, double lambda1,
                           const float* eta_host, int32_t max_sweeps, double tol, int32_t* sweeps_used, void* stream);
+/* prox / prox_by_frame (inexact_alm_lsd.py:49-68) for any non-nested graphs, all frames in one launch: graphs and frame_graph as for
+ * bsub_set_graphs; stop when the largest dual change of a sweep <= tol (absolute), at most max_sweeps (<= 0: 4000) per frame;
+ * sweeps_used = the largest sweep count over the frames.  Synchronises the stream. */
+int bsub_prox_graph_dev(const float* U, float* V, int64_t ld, int64_t m, int32_t n, double lambda1, int32_t n_graphs, const int32_t* frame_graph,
+                        const int64_t* n_groups, const int32_t* const* indptr, const int32_t* const* indices, const double* const* eta,
+                        int32_t max_sweeps, double tol, int32_t* sweeps_used, void* stream);
 /* block_shrinkage_operator(G, blocks_by_frame, lambdas_by_frame, mu, non_block_lambda)   group_sparse_RPCA.py:13-42 */
 int bsub_block_shrink_dev(const float* G, float* R, int64_t ld, int64_t m, int32_t n, const uint8_t* labels_host,
                           const int32_t* lam_ptr, const double* lam, double mu, double non_block_lambda, void* stream);
