@@ -426,7 +426,8 @@ def LSD_improved(ImData0, frame_start=0, frame_end=47, downsample_ratio=1, delta
 # --------------------------------------------------------------------------------------------------------------
 def inexact_alm_rpca_batch(slices, delta=1.0, max_rank=1, tol=1e-7, tol_l1=0.0, max_iter=500, rho=1.2, return_info=False):
     """inexact_alm_rpca (/root/reference/lsd_improvement.py:123-196) on every slices[i, :, :] at once, the rank of L capped at
-    max_rank = 1: one thread-block cluster per slice, state resident in shared memory (csrc/rpca_batch.cu).  -> (L, S) like the
+    max_rank = 1: one thread-block cluster per slice (csrc/rpca_batch.cu), its state resident in shared memory when the slice fits a
+    cluster of 8 CTAs (at most 640 columns), otherwise iterated in global memory (any slice up to 4096 x 4096).  -> (L, S) like the
     input ([slices, rows, cols]); with return_info also the per-slice iteration counts (negative: not converged), errors, ranks."""
     if max_rank != 1:
         raise Exception("inexact_alm_rpca_batch: the batched kernel caps the rank at 1 (use inexact_alm_rpca for a free rank)")
@@ -450,23 +451,26 @@ def inexact_alm_rpca_batch(slices, delta=1.0, max_rank=1, tol=1e-7, tol_l1=0.0, 
     return L, S
 
 
-def compute_RPCA(image_array, grayscale=True, max_error=None, max_iter=200000):
+def compute_RPCA(image_array, grayscale=True, max_error=None, max_iter=200000, return_info=False):
     """Drop-in for /root/reference/computeRPCADecomposition.py:12-48 (grayscale branch) -> (L_array, S_array): a max_rank = 1
     robust PCA of every image_array[i, :, :].  The reference hands each slice to RobustPCA(max_rank=1, tol=max_error) -- a package
     that is not vendored, pinned or installable (parity unpinned there); here every slice goes through the reference's own
     inexact_alm_rpca iteration with the rank capped at 1, stopped by the same residual test sum|M - L - S| <= max_error (or the
-    iteration's own 1e-7 relative tolerance, whichever comes first; 500 iterations at most, like inexact_alm_rpca)."""
+    iteration's own 1e-7 relative tolerance, whichever comes first; 500 iterations at most, like inexact_alm_rpca).
+    return_info=True appends inexact_alm_rpca_batch's info dict (per-slice iters, negative where the cap was hit; err; rank)."""
     if not grayscale:
         raise Exception("compute_RPCA: only the grayscale work mode (the reference's default) is implemented in this build")
     if max_error is None:
         max_error = image_array.shape[1] * image_array.shape[2] * 0.0001
-    return inexact_alm_rpca_batch(image_array, delta=1.0, tol_l1=float(max_error), max_iter=min(int(max_iter), 500))
+    return inexact_alm_rpca_batch(image_array, delta=1.0, tol_l1=float(max_error), max_iter=min(int(max_iter), 500),
+                                  return_info=return_info)
 
 
 def executeSaliencyRPCA(ImData, downsample_ratio, grayscale_workmode=True, grayscale_input=True):
     """Drop-in for /root/reference/computeRPCADecomposition.py:52-95 -> (xt_lowrank, xt_sparse, yt_lowrank, yt_sparse): the video
     [t, h, w] cut into X-T planes ([w, h, t]) and Y-T planes ([h, w, t]), each resized by 1/downsample_ratio over its first two
-    axes (resize_with_cv2) and decomposed slice by slice."""
+    axes (resize_with_cv2) and decomposed slice by slice.  Frames up to 4096 x 4096 pixels and clips up to 4096 frames; the X-T and
+    Y-T stacks may take different kernels (inexact_alm_rpca_batch), with no effect on the result beyond float32 rounding."""
     if not (grayscale_workmode and grayscale_input):
         raise Exception("executeSaliencyRPCA: only the grayscale mode is implemented in this build")
     torch = _torch()

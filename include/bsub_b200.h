@@ -271,7 +271,9 @@ int bsub_morph_disk_dev(const uint8_t* src, int64_t ld_src, uint8_t* dst, int64_
  * (lsd_improvement.py:123-196: lambda = 1/(sqrt(max(rows, cols)) delta), Y0 = D/max(||D||_2, ||D||_inf/lambda), mu0 = 1.25/||D||_2,
  * mu *= rho) with the rank of L capped at 1; stops when ||Z||_F/||D||_F < tol or (tol_l1 > 0) sum|Z| <= tol_l1 or after max_iter.
  * iters[b] > 0: iterations used; < 0: -max_iter, tolerance not met.  err[b] = last ||Z||_F/||D||_F, rank[b] in {0, 1}.
- * cols <= 640 and 4 * ceil(rows/8) * cols floats must fit the shared memory of one CTA (csrc/rpca_batch.cu). */
+ * Two kernels, chosen by shape (csrc/rpca_batch.cu): a slice whose state fits the shared memory of a cluster of <= 8 CTAs (cols <= 640
+ * and 4 * ceil(rows/C) * cols floats per CTA) is solved there; any other slice up to 4096 x 4096 iterates in global memory, S in S and
+ * Y/mu in L (L holds the low-rank part on return).  A larger slice is an error before any launch. */
 int bsub_rpca_rank1_batch_dev(const float* D, int32_t batch, int32_t rows, int32_t cols, double delta, double rho, double tol,
                               double tol_l1, int32_t max_iter, float* L, float* S, int32_t* iters, float* err, int32_t* rank, void* stream);
 
