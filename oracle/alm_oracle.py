@@ -272,7 +272,8 @@ def foreground_mask(D, L, S, sigmas_from_mean=2):
 # the ALM loops
 # --------------------------------------------------------------------------
 def _alm(D0, prox_fn, mu_scale, delta, rho=1.6, tol_out=1e-7, max_iter=500, sv0=10,
-         break_on_rank0=False, use_sv_prediction=True, L0=False, log=None):
+         break_on_rank0=False, use_sv_prediction=True, L0=False, log=None, return_Y=False):
+    """(L, S, iterations, converged), and the final multiplier Y after them when return_Y is set."""
     D = np.asfortranarray(D0, dtype=np.float64)
     m, n = D.shape
     d = min(m, n)
@@ -314,7 +315,7 @@ def _alm(D0, prox_fn, mu_scale, delta, rho=1.6, tol_out=1e-7, max_iter=500, sv0=
             converged = True
         elif it >= max_iter:
             break
-    return L, S, it, converged
+    return (L, S, it, converged, Y) if return_Y else (L, S, it, converged)
 
 
 def inexact_alm_lsd(D0, graphs=None, groups=None, delta=10, log=None, prox_tol=1e-13, prox_max_sweeps=20000,
