@@ -265,6 +265,78 @@ def _graph_pointers(csc):
     return ng, ip, ix, et
 
 
+class GraphRoute:
+    """Which prox kernel runs a graph description -- the one decision shared by the solvers below and the sharded driver
+    (dist.CudaStepSolver).  prox = C.PROX_GRAPH_LINF: the 3x3 all-window graph on the tile kernel, eta = float64 window weights
+    or None (unit weights); C.PROX_GRAPH_CENTER_BG: radius-1 centre windows on the tile kernel, eta = float32 [n][m] map;
+    C.PROX_GRAPH_GENERIC: any other graph on the generic kernel, csc / frame_graph as pack_graphs returns them.  background =
+    uint8 [n][m] (non-zero: the frame's background pixels, l2-shrunk after the prox) or None; rows, cols = image geometry
+    (0, 0 when the generic graphs came without one)."""
+
+    def __init__(self, prox, rows, cols, eta=None, csc=None, frame_graph=None, background=None):
+        self.prox, self.rows, self.cols = prox, int(rows), int(cols)
+        self.eta, self.csc, self.frame_graph, self.background = eta, csc, frame_graph, background
+
+
+def route_graphs(graphs, m, n, img_shape=None, background_masks=None):
+    """GraphRoute of inexact_alm_lsd(graphs=...) (background_masks None: all-window graph or any other) or of
+    inexact_alm_lsd_with_background (radius-1 centre windows or any other graphs, plus the background)."""
+    if background_masks is None:
+        if _is_graph_list(graphs):
+            glist = list(graphs)
+            if len(glist) != n:
+                raise Exception("graphs must hold one graph per frame")
+            first = detect_window_graph(glist[0], m, img_shape)
+            same = first is not None and all(
+                (g is glist[0]) or (detect_window_graph(g, m, img_shape) is not None and
+                                    np.array_equal(g['eta_g'], glist[0]['eta_g'])) for g in glist[1:])
+            geo = first if same else None
+        else:
+            geo = detect_window_graph(graphs, m, img_shape)
+        if geo is None:                                  # any other graph, or per-frame graphs that differ
+            csc, frame_graph = pack_graphs(graphs, m, n)
+            return GraphRoute(C.PROX_GRAPH_GENERIC, *_geometry(img_shape, m), csc=csc, frame_graph=frame_graph)
+        rows, cols, eta = geo
+        return GraphRoute(C.PROX_GRAPH_LINF, rows, cols, eta=None if np.all(eta == 1.0) else eta)
+    if not isinstance(graphs, list) and not isinstance(graphs, np.ndarray):
+        raise Exception('graphs must be list/array')                       # lsd_improvement.py:223-224
+    if len(graphs) != n or len(background_masks) != n:
+        raise Exception("graphs and background_masks must have one entry per frame")
+    eta = np.empty((n, m), dtype=np.float32)
+    shape = tuple(img_shape) if img_shape is not None else None
+    generic = False
+    for f in range(n):
+        det = detect_center_windows(graphs[f], m, shape)
+        if det is None:                                  # not a radius-1 centre-window graph: the generic graph mode
+            generic = True
+            break
+        if shape is None or graphs[f].get('_group_centers', None) is not None:
+            shape = det[0] if shape is None else shape
+        if det[0] != tuple(shape):
+            raise Exception("frame %d: graph built for image shape %s, expected %s" % (f, det[0], tuple(shape)))
+        eta[f] = det[1]
+    bg = np.ascontiguousarray(np.stack([np.asarray(b, dtype=bool).ravel() for b in background_masks]).astype(np.uint8))
+    if bg.shape != (n, m):
+        raise Exception("background_masks must hold %d boolean masks of %d pixels" % (n, m))
+    if generic:
+        csc, frame_graph = pack_graphs(graphs, m, n)
+        return GraphRoute(C.PROX_GRAPH_GENERIC, *_geometry(img_shape, m), csc=csc, frame_graph=frame_graph, background=bg)
+    return GraphRoute(C.PROX_GRAPH_CENTER_BG, shape[0], shape[1], eta=eta, background=bg)
+
+
+def route_weight_mask(weight_mask, m, n, img_shape=None):
+    """GraphRoute of the [h, w, t] weight map of build_improved_LSD_graphs (center_window_decomposition): radius-1 centre windows
+    weighted by the positive entries, background where an entry is negative."""
+    wm = np.asarray(weight_mask)
+    h, w = (int(v) for v in (img_shape if img_shape is not None else wm.shape[:2]))
+    if wm.shape != (h, w, n) or h * w != m:
+        raise Exception("weight_mask must be [h, w, t] with h*w = %d pixels and t = %d frames" % (m, n))
+    flat = np.ascontiguousarray(wm.transpose(2, 1, 0)).reshape(n, m)          # [t][p], p = j*rows + i
+    eta = np.where(flat > 0, flat, 0).astype(np.float32)
+    bg = np.ascontiguousarray((flat < 0).astype(np.uint8))
+    return GraphRoute(C.PROX_GRAPH_CENTER_BG, h, w, eta=eta, background=bg)
+
+
 # --------------------------------------------------------------------------------------------------------------
 # marshalling helpers
 # --------------------------------------------------------------------------------------------------------------
@@ -401,6 +473,37 @@ class Decomposition:
         bg = None if background is None else np.ascontiguousarray(background, dtype=np.uint8)
         C.check(self.lib.bsub_set_graphs(self.h, len(csc), fg.ctypes.data_as(C.c_int32_p), ng.ctypes.data_as(C.c_int64_p), ip, ix, et,
                                          None if bg is None else bg.ctypes.data_as(C.c_uint8_p)))
+
+    def set_route(self, route):
+        """The whole-clip description of a GraphRoute (this handle's pixels are whole frames)."""
+        if route.prox == C.PROX_GRAPH_LINF:
+            self.set_graph_windows(route.eta)
+        elif route.prox == C.PROX_GRAPH_GENERIC:
+            self.set_graphs(route.csc, route.frame_graph, route.background)
+        else:
+            C.check(self.lib.bsub_set_center_windows(self.h, route.eta.ctypes.data_as(C.c_float_p),
+                                                     route.background.ctypes.data_as(C.c_uint8_p)))
+
+    def set_frame_route(self, route, f0, f1):
+        """Frame-range description of a GraphRoute: the prox of whole frames [f0, f1) (bsub_set_frame_*, run by
+        bsub_step_prox_block).  Only those frames' graphs, weights and background are uploaded."""
+        rows, cols, nf = route.rows, route.cols, f1 - f0
+        bg = None if route.background is None else np.ascontiguousarray(route.background[f0:f1])
+        bgp = None if bg is None else bg.ctypes.data_as(C.c_uint8_p)
+        if route.prox == C.PROX_GRAPH_LINF:
+            e = None if route.eta is None else np.ascontiguousarray(route.eta, dtype=np.float64)
+            C.check(self.lib.bsub_set_frame_windows(self.h, rows, cols, f0, nf, None if e is None else e.ctypes.data_as(C.c_double_p),
+                                                    0 if e is None else e.size))
+        elif route.prox == C.PROX_GRAPH_CENTER_BG:
+            eta = np.ascontiguousarray(route.eta[f0:f1], dtype=np.float32)
+            C.check(self.lib.bsub_set_frame_center_windows(self.h, rows, cols, f0, nf, eta.ctypes.data_as(C.c_float_p), bgp))
+        else:
+            used, fg = np.unique(np.asarray(route.frame_graph[f0:f1]), return_inverse=True)
+            csc = [route.csc[k] for k in used]
+            fg = np.ascontiguousarray(fg, dtype=np.int32)
+            ng, ip, ix, et = _graph_pointers(csc)
+            C.check(self.lib.bsub_set_frame_graphs(self.h, rows, cols, f0, nf, len(csc), fg.ctypes.data_as(C.c_int32_p),
+                                                   ng.ctypes.data_as(C.c_int64_p), ip, ix, et, bgp))
 
     def set_blocks(self, labels, lam_ptr, lam):
         labels = np.ascontiguousarray(labels, dtype=np.uint8)
@@ -555,32 +658,11 @@ def lsd_decomposition(D0, graphs=None, groups=None, delta=10, img_shape=None, ma
         dec = Decomposition(cfg)
         dec.set_flat_groups(groups)
     else:
-        if _is_graph_list(graphs):
-            glist = list(graphs)
-            if len(glist) != n:
-                raise Exception("graphs must hold one graph per frame")
-            first = detect_window_graph(glist[0], m, img_shape)
-            same = first is not None and all(
-                (g is glist[0]) or (detect_window_graph(g, m, img_shape) is not None and
-                                    np.array_equal(g['eta_g'], glist[0]['eta_g'])) for g in glist[1:])
-            geo = first if same else None
-        else:
-            geo = detect_window_graph(graphs, m, img_shape)
-        if geo is None:                                  # any other graph, or per-frame graphs that differ
-            csc, frame_graph = pack_graphs(graphs, m, n)
-            rows, cols = _geometry(img_shape, m)
-            cfg = make_config(m, n, C.PROX_GRAPH_GENERIC, rows, cols, delta=delta, max_iter=max_iter, tile_rows=tile_rows,
-                              cluster_frames=cluster_frames, graph_max_sweeps=graph_max_sweeps, graph_tol=graph_tol)
-            dec = Decomposition(cfg)
-            dec.set_graphs(csc, frame_graph)
-            dec.load(D0)
-            dec.run()
-            return dec
-        rows, cols, eta = geo
-        cfg = make_config(m, n, C.PROX_GRAPH_LINF, rows, cols, delta=delta, max_iter=max_iter, tile_rows=tile_rows,
+        route = route_graphs(graphs, m, n, img_shape)
+        cfg = make_config(m, n, route.prox, route.rows, route.cols, delta=delta, max_iter=max_iter, tile_rows=tile_rows,
                           cluster_frames=cluster_frames, graph_max_sweeps=graph_max_sweeps, graph_tol=graph_tol)
         dec = Decomposition(cfg)
-        dec.set_graph_windows(None if np.all(eta == 1.0) else eta)
+        dec.set_route(route)
     dec.load(D0)
     dec.run()
     return dec
@@ -632,38 +714,10 @@ def inexact_alm_lsd_batch(clips, groups=None, graphs=None, delta=10, img_shape=N
 
 
 def with_background_decomposition(D0, graphs, background_masks, delta=10, img_shape=None, **tuning):
-    if not isinstance(graphs, list) and not isinstance(graphs, np.ndarray):
-        raise Exception('graphs must be list/array')                       # lsd_improvement.py:223-224
     m, n = _shape_of(D0)
-    if len(graphs) != n or len(background_masks) != n:
-        raise Exception("graphs and background_masks must have one entry per frame")
-    eta = np.empty((n, m), dtype=np.float32)
-    shape = tuple(img_shape) if img_shape is not None else None
-    generic = False
-    for f in range(n):
-        det = detect_center_windows(graphs[f], m, shape)
-        if det is None:                                  # not a radius-1 centre-window graph: the generic graph mode
-            generic = True
-            break
-        if shape is None or graphs[f].get('_group_centers', None) is not None:
-            shape = det[0] if shape is None else shape
-        if det[0] != tuple(shape):
-            raise Exception("frame %d: graph built for image shape %s, expected %s" % (f, det[0], tuple(shape)))
-        eta[f] = det[1]
-    bg = np.ascontiguousarray(np.stack([np.asarray(b, dtype=bool).ravel() for b in background_masks]).astype(np.uint8))
-    if bg.shape != (n, m):
-        raise Exception("background_masks must hold %d boolean masks of %d pixels" % (n, m))
-    if generic:
-        csc, frame_graph = pack_graphs(graphs, m, n)
-        rows, cols = _geometry(img_shape, m)
-        dec = Decomposition(make_config(m, n, C.PROX_GRAPH_GENERIC, rows, cols, delta=delta, **tuning))
-        dec.set_graphs(csc, frame_graph, bg)
-        dec.load(D0)
-        dec.run()
-        return dec
-    cfg = make_config(m, n, C.PROX_GRAPH_CENTER_BG, shape[0], shape[1], delta=delta, **tuning)
-    dec = Decomposition(cfg)
-    C.check(dec.lib.bsub_set_center_windows(dec.h, eta.ctypes.data_as(C.c_float_p), bg.ctypes.data_as(C.c_uint8_p)))
+    route = route_graphs(graphs, m, n, img_shape, background_masks=background_masks)
+    dec = Decomposition(make_config(m, n, route.prox, route.rows, route.cols, delta=delta, **tuning))
+    dec.set_route(route)
     dec.load(D0)
     dec.run()
     return dec
@@ -674,16 +728,9 @@ def center_window_decomposition(D0, weight_mask, delta=10, img_shape=None, **tun
     (/root/reference/lsd_improvement.py:406-436): a positive entry is the weight of the 3x3 window centred on that pixel of that
     frame, a negative one marks a background pixel -- the per-frame SPAMS graphs are never built."""
     m, n = _shape_of(D0)
-    wm = np.asarray(weight_mask)
-    h, w = (int(v) for v in (img_shape if img_shape is not None else wm.shape[:2]))
-    if wm.shape != (h, w, n) or h * w != m:
-        raise Exception("weight_mask must be [h, w, t] with h*w = %d pixels and t = %d frames" % (m, n))
-    flat = np.ascontiguousarray(wm.transpose(2, 1, 0)).reshape(n, m)          # [t][p], p = j*rows + i
-    eta = np.where(flat > 0, flat, 0).astype(np.float32)
-    bg = np.ascontiguousarray((flat < 0).astype(np.uint8))
-    cfg = make_config(m, n, C.PROX_GRAPH_CENTER_BG, h, w, delta=delta, **tuning)
-    dec = Decomposition(cfg)
-    C.check(dec.lib.bsub_set_center_windows(dec.h, eta.ctypes.data_as(C.c_float_p), bg.ctypes.data_as(C.c_uint8_p)))
+    route = route_weight_mask(weight_mask, m, n, img_shape)
+    dec = Decomposition(make_config(m, n, route.prox, route.rows, route.cols, delta=delta, **tuning))
+    dec.set_route(route)
     dec.load(D0)
     dec.run()
     return dec

@@ -8,6 +8,7 @@
 // host only limits how far ahead it enqueues by watching a mapped status word.
 #include <math.h>
 #include <stdarg.h>
+#include <cmath>
 #include <stdlib.h>
 #include <string.h>
 #include <vector>
@@ -65,10 +66,16 @@ struct bsub_solver {
     int* gptr = nullptr; int* gidx = nullptr; int ngroups = 0; bool groups_set = false;
     // overlapping graph
     float* eta_dev = nullptr; float* xi = nullptr; long long xi_floats = 0; float* tot = nullptr;
-    float* xi2 = nullptr; float* tot2 = nullptr; int* sweeps2 = nullptr; long long xi2_floats = 0, tot2_floats = 0;   // bsub_step_prox_frames
+    float* xi2 = nullptr; float* tot2 = nullptr; int* sweeps2 = nullptr; long long xi2_floats = 0, tot2_floats = 0;   // bsub_step_prox_frames / _prox_block
     int* sweeps_dev = nullptr; bool graph_set = false;
     // any graphs (BSUB_PROX_GRAPH_GENERIC): packed index arrays + eta on the device, where tot lives; xi / tot / sweeps_dev above
     int* pg_ints = nullptr; float* pg_eta = nullptr; GenericGraphDev pg_dev; GenericGraphLayout pg_layout; bool pg_bg = false;
+    // frame-range description (bsub_set_frame_*): the prox of whole rows x cols frames [fr_f0, fr_f0 + fr_nf) of the clip, run by
+    // bsub_step_prox_block on the frames a pixel-sharded driver has gathered; workspaces xi2 / tot2 above
+    bool fr_set = false; int fr_rows = 0, fr_cols = 0, fr_f0 = 0, fr_nf = 0;
+    float* fr_eta = nullptr; long long fr_eta_stride = 0;           // tile kernel: window weights (stride 0) or centre map [nf][m]
+    int* fr_ints = nullptr; float* fr_geta = nullptr; GenericGraphDev fr_graph; long long fr_max_nnz = 0;   // generic kernel
+    unsigned char* fr_labels = nullptr; double* fr_bsums = nullptr;   // background (label 0) [nf][m] and its sums, or none
     // l2 blocks
     unsigned char* labels_dev = nullptr; double* lam_table = nullptr; double* bsums = nullptr; int nlab = 0; bool blocks_set = false;
     unsigned char* mask_stage = nullptr;      // bsub_mask_host staging
@@ -93,6 +100,16 @@ static int ensure_stage64(bsub_solver* s, size_t doubles) {
     s->stage64_doubles = doubles;
     return 0;
 }
+// whole-frame prox workspaces: allocated once, grown when a call needs more
+static int grow_floats(float** p, long long* have, long long want) {
+    if (want <= *have) return 0;
+    if (*p) cudaFree(*p);
+    *p = nullptr; *have = 0;
+    CK(cudaMalloc((void**)p, sizeof(float) * (size_t)want));
+    *have = want;
+    return 0;
+}
+
 // frees whatever a stand-alone operator allocated, on every return path
 struct DevScope {
     std::vector<void*> ptrs;
@@ -138,7 +155,7 @@ int bsub_destroy(bsub_solver* s) {
                     s->eb.work, s->eb.lam, s->eb.Z, s->eb.Vr, s->eb.VC, s->tpart, s->part_zz, s->part_nnz, s->part_max, s->gptr,
                     s->gidx, s->eta_dev, s->xi, s->tot, s->sweeps_dev, s->labels_dev, s->lam_table, s->bsums, s->Wq, s->Gint,
                     s->gi_info, s->gi_blkn, s->part_wmax, s->mask_stage, s->mask_scratch, s->stage64, s->Tt, s->xi2, s->tot2, s->sweeps2,
-                    s->pg_ints, s->pg_eta};
+                    s->pg_ints, s->pg_eta, s->fr_eta, s->fr_ints, s->fr_geta, s->fr_labels, s->fr_bsums};
     for (void* p : ptrs) if (p) cudaFree(p);
     if (s->mirror) cudaFreeHost((void*)s->mirror);
     for (int i = 0; i <= kRunAhead; ++i) if (s->ev[i]) cudaEventDestroy(s->ev[i]);
@@ -402,6 +419,90 @@ int bsub_set_graphs(bsub_solver* s, int32_t n_graphs, const int32_t* frame_graph
     return 0;
 }
 
+// ---------------------------------------------------------------------------- frame-range descriptions (bsub_step_prox_block)
+static int frame_range_check(bsub_solver* s, int prox, const char* prox_name, int32_t rows, int32_t cols, int32_t f0, int32_t nf,
+                             const char* who) {
+    if (!s) { set_error("%s: null solver", who); return -1; }
+    if (s->cfg.prox != prox) { set_error("%s: solver was not created with %s", who, prox_name); return -1; }
+    if (rows <= 0 || cols <= 0 || (long long)rows * cols > (1LL << 30)) { set_error("%s: bad frame geometry %d x %d", who, rows, cols); return -1; }
+    if (f0 < 0 || nf < 0 || (long long)f0 + nf > s->n) {
+        set_error("%s: frames [%d, %lld) are not a range of the %d frames of the clip", who, f0, (long long)f0 + nf, s->n); return -1;
+    }
+    return 0;
+}
+
+// drops the previous description; the new one takes effect once everything has been uploaded
+static void frame_range_clear(bsub_solver* s) {
+    for (void* p : {(void*)s->fr_eta, (void*)s->fr_ints, (void*)s->fr_geta, (void*)s->fr_labels, (void*)s->fr_bsums}) if (p) cudaFree(p);
+    s->fr_eta = nullptr; s->fr_ints = nullptr; s->fr_geta = nullptr; s->fr_labels = nullptr; s->fr_bsums = nullptr;
+    s->fr_set = false; s->fr_eta_stride = 0; s->fr_max_nnz = 0;
+}
+
+// background uint8[nf][m] (may be NULL) -> label 0 (the complement group of the l2 kernels) / 255 (keeps the graph prox result)
+static int frame_range_finish(bsub_solver* s, int32_t rows, int32_t cols, int32_t f0, int32_t nf, const uint8_t* background) {
+    const size_t nm = (size_t)nf * rows * cols;
+    if (background != nullptr && nf > 0) {
+        std::vector<unsigned char> lab(nm);
+        for (size_t i = 0; i < nm; ++i) lab[i] = background[i] ? 0 : 255;
+        CK(cudaMalloc((void**)&s->fr_labels, nm));
+        CK(cudaMalloc((void**)&s->fr_bsums, sizeof(double) * nf));
+        CK(cudaMemcpy(s->fr_labels, lab.data(), nm, cudaMemcpyHostToDevice));
+    }
+    if (!s->sweeps_dev) { CK(cudaMalloc((void**)&s->sweeps_dev, sizeof(int) * 8)); CK(cudaMemset(s->sweeps_dev, 0, sizeof(int) * 8)); }
+    s->fr_rows = rows; s->fr_cols = cols; s->fr_f0 = f0; s->fr_nf = nf;
+    s->fr_set = true;
+    return 0;
+}
+
+int bsub_set_frame_windows(bsub_solver* s, int32_t rows, int32_t cols, int32_t f0, int32_t nf, const double* eta, int64_t n_eta) {
+    RET_IF(frame_range_check(s, BSUB_PROX_GRAPH_LINF, "BSUB_PROX_GRAPH_LINF", rows, cols, f0, nf, "bsub_set_frame_windows"));
+    const long long nw = (long long)(rows - std::min(3, rows) + 1) * (cols - std::min(3, cols) + 1);
+    std::vector<float> ef;
+    if (eta != nullptr) {
+        if (n_eta != nw) { set_error("bsub_set_frame_windows: eta has %lld entries, the %dx%d image has %lld windows", (long long)n_eta, rows, cols, nw); return -1; }
+        ef.resize((size_t)nw);
+        for (long long i = 0; i < nw; ++i) {
+            if (!(std::isfinite(eta[i]) && eta[i] >= 0.0)) { set_error("bsub_set_frame_windows: eta[%lld] = %g is not finite and >= 0", i, eta[i]); return -1; }
+            ef[i] = (float)eta[i];
+        }
+    }
+    frame_range_clear(s);
+    if (eta != nullptr) {                  // the same weights in every frame
+        CK(cudaMalloc((void**)&s->fr_eta, sizeof(float) * nw));
+        CK(cudaMemcpy(s->fr_eta, ef.data(), sizeof(float) * nw, cudaMemcpyHostToDevice));
+    }
+    return frame_range_finish(s, rows, cols, f0, nf, nullptr);
+}
+
+int bsub_set_frame_center_windows(bsub_solver* s, int32_t rows, int32_t cols, int32_t f0, int32_t nf, const float* eta, const uint8_t* background) {
+    RET_IF(frame_range_check(s, BSUB_PROX_GRAPH_CENTER_BG, "BSUB_PROX_GRAPH_CENTER_BG", rows, cols, f0, nf, "bsub_set_frame_center_windows"));
+    const size_t nm = (size_t)nf * rows * cols;
+    if (nf > 0 && (!eta || !background)) { set_error("bsub_set_frame_center_windows: null argument"); return -1; }
+    for (size_t i = 0; i < nm; ++i)
+        if (!std::isfinite(eta[i])) { set_error("bsub_set_frame_center_windows: eta[%zu] = %g is not finite", i, (double)eta[i]); return -1; }
+    frame_range_clear(s);
+    if (nf > 0) {
+        CK(cudaMalloc((void**)&s->fr_eta, sizeof(float) * nm));
+        CK(cudaMemcpy(s->fr_eta, eta, sizeof(float) * nm, cudaMemcpyHostToDevice));
+    }
+    s->fr_eta_stride = (long long)rows * cols;
+    return frame_range_finish(s, rows, cols, f0, nf, background);
+}
+
+int bsub_set_frame_graphs(bsub_solver* s, int32_t rows, int32_t cols, int32_t f0, int32_t nf, int32_t n_graphs, const int32_t* frame_graph,
+                          const int64_t* n_groups, const int32_t* const* indptr, const int32_t* const* indices, const double* const* eta,
+                          const uint8_t* background) {
+    RET_IF(frame_range_check(s, BSUB_PROX_GRAPH_GENERIC, "BSUB_PROX_GRAPH_GENERIC", rows, cols, f0, nf, "bsub_set_frame_graphs"));
+    GenericGraphHost H;
+    if (nf > 0) RET_IF(pack_generic_graphs((long long)rows * cols, nf, n_graphs, frame_graph, n_groups, indptr, indices, eta, &H, "bsub_set_frame_graphs"));
+    frame_range_clear(s);
+    if (nf > 0) {
+        RET_IF(upload_generic_graphs(H, &s->fr_ints, &s->fr_geta, &s->fr_graph));
+        s->fr_max_nnz = H.max_nnz;
+    }
+    return frame_range_finish(s, rows, cols, f0, nf, background);
+}
+
 int bsub_set_blocks(bsub_solver* s, const uint8_t* labels, const int32_t* lam_ptr, const double* lam) {
     if (!s || !labels || !lam_ptr) { set_error("bsub_set_blocks: null argument"); return -1; }
     if (s->cfg.prox != BSUB_PROX_BLOCK_L2) { set_error("bsub_set_blocks: solver was not created with BSUB_PROX_BLOCK_L2"); return -1; }
@@ -541,7 +642,7 @@ static int check_ready(bsub_solver* s) {
     if (!s->loaded) { set_error("no data loaded (call bsub_load_* first)"); return -1; }
     if (s->cfg.prox == BSUB_PROX_FLAT_LINF && !s->groups_set) { set_error("one of graphs or groups must not be None"); return -1; }
     if ((s->cfg.prox == BSUB_PROX_GRAPH_LINF || s->cfg.prox == BSUB_PROX_GRAPH_CENTER_BG || s->cfg.prox == BSUB_PROX_GRAPH_GENERIC) &&
-        !s->graph_set) { set_error("one of graphs or groups must not be None"); return -1; }
+        !s->graph_set && !s->fr_set) { set_error("one of graphs or groups must not be None"); return -1; }
     if (s->cfg.prox == BSUB_PROX_BLOCK_L2 && !s->blocks_set) { set_error("blocks_by_frame / lambdas_by_frame not set"); return -1; }
     return 0;
 }
@@ -614,9 +715,14 @@ static int step_shrink_impl(bsub_solver* s, void* stream, int part) {
     if (!s || !s->initialised) { set_error("bsub_step_shrink: solver not initialised"); return -1; }
     cudaStream_t st = use_stream(s, stream);
     // the overlapping-window mode splits too: between the halves the driver re-shards G_S by FRAMES (the prox of a frame needs the
-    // whole image, bsub_step_prox_frames) and brings S back
-    const bool split = s->shrink_mode == SHRINK_SPILL && (s->cfg.prox == BSUB_PROX_BLOCK_L2 || s->cfg.prox == BSUB_PROX_GRAPH_LINF);
+    // whole image) and brings S back
+    // (bsub_step_prox_frames), and so does every graph mode once the handle has a frame-range description (bsub_step_prox_block)
+    const bool split = s->shrink_mode == SHRINK_SPILL && (s->cfg.prox == BSUB_PROX_BLOCK_L2 || s->cfg.prox == BSUB_PROX_GRAPH_LINF || s->fr_set);
     if (part == 2 && !split) return 0;
+    if (part == 0 && s->fr_set && !s->graph_set) {
+        set_error("bsub_step_shrink: the handle holds only a frame-range description; use _shrink_a, bsub_step_prox_block, _shrink_b");
+        return -1;
+    }
     if (part == 2) {
         if (s->cfg.prox == BSUB_PROX_BLOCK_L2)
             RET_IF(launch_block_l2_apply(s->U, s->S, s->labels_dev, s->ld, s->m, s->n, s->nlab, s->bsums, s->lam_table, s->st, 0.0, 0.0, st));
@@ -678,6 +784,8 @@ static int step_shrink_impl(bsub_solver* s, void* stream, int part) {
             if (part == 1) return 0;                       // the driver runs the prox on frame shards, then calls part 2
             RET_IF(launch_prox_graph3(s->U, s->S, s->xi, s->xi_floats, s->tot, s->eta_dev, s->ld, s->cfg.rows, s->cfg.cols, s->n, 0.f,
                                       s->cfg.graph_max_sweeps, (float)s->cfg.graph_tol, s->sweeps_dev, s->st, st));
+        } else if (part == 1 && s->fr_set) {
+            return 0;                                      // the driver runs the prox on frame shards (bsub_step_prox_block)
         } else if (s->cfg.prox == BSUB_PROX_GRAPH_CENTER_BG) {
             // S = prox_by_frame(G_S) then the background pixels of every frame are overwritten by their l2 shrink of G_S
             RET_IF(launch_prox_graph3(s->U, s->S, s->xi, s->xi_floats, s->tot, s->eta_dev, s->ld, s->cfg.rows, s->cfg.cols, s->n, 0.f,
@@ -727,12 +835,52 @@ int bsub_step_prox_frames(bsub_solver* s, const float* Uf, float* Vf, int64_t ld
     cudaStream_t st = use_stream(s, stream);
     long long xf = 0, tf = 0;
     prox_graph3_workspace(rows, cols, nf, ldf, 0, &xf, &tf);
-    if (xf > s->xi2_floats) { if (s->xi2) cudaFree(s->xi2); s->xi2 = nullptr; CK(cudaMalloc((void**)&s->xi2, sizeof(float) * (size_t)xf)); s->xi2_floats = xf; }
-    if (tf > s->tot2_floats) { if (s->tot2) cudaFree(s->tot2); s->tot2 = nullptr; CK(cudaMalloc((void**)&s->tot2, sizeof(float) * (size_t)tf)); s->tot2_floats = tf; }
+    RET_IF(grow_floats(&s->xi2, &s->xi2_floats, xf));
+    RET_IF(grow_floats(&s->tot2, &s->tot2_floats, tf));
     if (!s->sweeps2) { CK(cudaMalloc((void**)&s->sweeps2, sizeof(int) * 8)); CK(cudaMemset(s->sweeps2, 0, sizeof(int) * 8)); }
     // lambda / mu and the stop flag come from the device state, exactly as in the unsharded pass
     return launch_prox_graph3(Uf, Vf, s->xi2, xf, s->tot2, nullptr, ldf, rows, cols, nf, 0.f, s->cfg.graph_max_sweeps, (float)s->cfg.graph_tol,
                               s->sweeps2, s->st, st);
+}
+
+int bsub_step_prox_block(bsub_solver* s, const float* Uf, float* Vf, int64_t ldf, int32_t f0, int32_t nf, void* stream) {
+    if (!s || !s->initialised) { set_error("bsub_step_prox_block: solver not initialised"); return -1; }
+    if (!s->fr_set) { set_error("bsub_step_prox_block: the handle has no frame-range description (bsub_set_frame_*)"); return -1; }
+    if (nf < 0 || f0 < s->fr_f0 || (long long)f0 + nf > (long long)s->fr_f0 + s->fr_nf) {
+        set_error("bsub_step_prox_block: frames [%d, %lld) are outside the described range [%d, %d)", f0, (long long)f0 + nf, s->fr_f0,
+                  s->fr_f0 + s->fr_nf);
+        return -1;
+    }
+    if (nf == 0) return 0;
+    const int rows = s->fr_rows, cols = s->fr_cols, lf = f0 - s->fr_f0;
+    const long long m = (long long)rows * cols;
+    if (!Uf || !Vf || ldf < m) { set_error("bsub_step_prox_block: bad argument"); return -1; }
+    cudaStream_t st = use_stream(s, stream);
+    // lambda / mu and the stop flag come from the device state, exactly as in the unsharded pass
+    if (s->cfg.prox == BSUB_PROX_GRAPH_GENERIC) {
+        const GenericGraphLayout L = prox_graph_generic_layout(m, ldf, nf, s->fr_max_nnz);
+        RET_IF(grow_floats(&s->xi2, &s->xi2_floats, L.xi_floats));
+        RET_IF(grow_floats(&s->tot2, &s->tot2_floats, L.tot_floats));
+        GenericGraphDev g = s->fr_graph;
+        g.frame_graph += lf;
+        RET_IF(launch_prox_graph_generic(Uf, Vf, ldf, m, nf, g, L, s->xi2, s->tot2, 0.f, s->cfg.graph_max_sweeps, (float)s->cfg.graph_tol,
+                                         s->sweeps_dev, s->st, st));
+    } else {
+        const int center = s->cfg.prox == BSUB_PROX_GRAPH_CENTER_BG ? 1 : 0;
+        long long xf = 0, tf = 0;
+        prox_graph3_workspace(rows, cols, nf, ldf, center, &xf, &tf);
+        RET_IF(grow_floats(&s->xi2, &s->xi2_floats, xf));
+        RET_IF(grow_floats(&s->tot2, &s->tot2_floats, tf));
+        const float* eta = s->fr_eta ? s->fr_eta + (size_t)lf * s->fr_eta_stride : nullptr;
+        RET_IF(launch_prox_graph3(Uf, Vf, s->xi2, xf, s->tot2, eta, ldf, rows, cols, nf, 0.f, s->cfg.graph_max_sweeps, (float)s->cfg.graph_tol,
+                                  s->sweeps_dev, s->st, st, center, s->fr_eta_stride));
+    }
+    if (s->fr_labels) {       // background pixels: their frame's l2 shrink of G_S at non_block_lambda / mu, over the graph prox result
+        const unsigned char* lab = s->fr_labels + (size_t)lf * m;
+        RET_IF(launch_block_l2_sums(Uf, lab, ldf, m, nf, 1, s->fr_bsums, s->st, st));
+        RET_IF(launch_block_l2_apply(Uf, Vf, lab, ldf, m, nf, 1, s->fr_bsums, nullptr, s->st, 0.0, 0.0, st, 1));
+    }
+    return 0;
 }
 
 int bsub_block_sums_buffer(bsub_solver* s, double** sums, int64_t* count) {
@@ -780,6 +928,10 @@ int bsub_sync_status(bsub_solver* s, bsub_status* out, void* stream) {
 }
 
 int bsub_run(bsub_solver* s, void* stream) {
+    if (s && s->fr_set && !s->graph_set) {
+        set_error("bsub_run: the handle holds only a frame-range description (bsub_set_frame_*), not the graphs of its own pixels");
+        return -1;
+    }
     for (int attempt = 0; attempt < 2; ++attempt) {
         RET_IF(bsub_step_init_local(s, stream));
         RET_IF(bsub_step_init_finish(s, stream));

@@ -2,7 +2,7 @@
 
 The path shards by image columns (pixel index p = j*rows + i, so a block of whole columns is a contiguous pixel
 range of every frame): rank r owns the column triples [t0, t1) so that no 3x3 tile straddles two ranks
-(SURVEY.md section 8e).  Per ALM iteration there is ONE exchange (two in the l2-block mode, see ShardedLSD): an all-reduce(SUM) of a single buffer that holds the
+(SURVEY.md section 8e).  Per ALM iteration there is ONE exchange (two in the l2-block and graph modes, see ShardedLSD): an all-reduce(SUM) of a single buffer that holds the
 frames x frames fp64 Gram partial of iteration k+1 followed by the 4 scalars of iteration k (sum Z^2, ||S||_0, ...).  The
 shrink pass of iteration k advances mu itself (local data only), the Gram of k+1 is enqueued right behind it, and the
 residual / stop test of iteration k is evaluated after the joint message has arrived; an iteration that turns out to be
@@ -84,21 +84,64 @@ class TorchComm:
 class CudaStepSolver:
     """Thin object view of the bsub_step_* C entry points for one shard."""
 
-    def __init__(self, rows, cols_local, n, m_global, delta=10, max_iter=500, tile_rows=0, cluster_frames=0, store_S_lazily=True,
-                 blocks=None, use_sv_prediction=True, graph_cols=None):
+    def __init__(self, rows, cols_local, n, m_global, delta=None, max_iter=500, tile_rows=0, cluster_frames=0, store_S_lazily=True,
+                 blocks=None, use_sv_prediction=True, graph_cols=None, graphs=None, background_masks=None, weight_mask=None, l1=False,
+                 frames=None):
         """blocks = (labels uint8 [n][rows * cols_local] of THIS shard's pixels, lam_ptr int32 [n + 1], lam float64) selects the
         group-sparse solver (inexact_alm_group_sparse_RPCA, /root/reference/group_sparse_RPCA.py:45-126: l2 blocks per frame,
         mu0 = 1.25 / ||D||_2, stop on rank 0); lam_ptr / lam are the same on every rank.  graph_cols = number of image columns of the
-        WHOLE frame selects the reference's default LSD() mode (overlapping 3x3 windows with unit weights,
+        WHOLE frame alone selects the reference's default LSD() mode (overlapping 3x3 windows with unit weights,
         /root/reference/inexact_alm_lsd.py:13-57): the prox then runs on whole frames after a frame-wise re-sharding (ShardedLSD).
-        Default: flat 3x3 l_inf groups (LSD)."""
+        The other graph modes also run their prox on whole frames, those of `frames` = (f0, f1), which must be
+        shard_frames(n, world, rank) (default: all n frames, one rank); they take the public solvers' descriptions of the WHOLE
+        frame (rows x graph_cols pixels), and api.route_graphs / api.route_weight_mask pick the kernel as those solvers do:
+          graphs = SPAMS graph dict or per-frame list, with graph_cols: inexact_alm_lsd(graphs=...);
+          graphs + background_masks (list of n boolean masks of the whole frame): inexact_alm_lsd_with_background;
+          weight_mask = [h, w, t] map of build_improved_LSD_graphs: center_window_decomposition (LSD_improved's second pass).
+        l1=True: inexact_alm_rpca (elementwise soft threshold, /root/reference/lsd_improvement.py:123-196: delta 1.0, mu0 =
+        1.25 / ||D||_2, rho 1.2, no sv prediction), which shards without any exchange.  Default: flat 3x3 l_inf groups (LSD)."""
+        if sum(x is not None for x in (blocks, graphs, weight_mask)) + bool(l1) > 1:
+            raise Exception("CudaStepSolver: blocks, graphs, weight_mask and l1 are mutually exclusive")
+        if background_masks is not None and graphs is None:
+            raise Exception("CudaStepSolver: background_masks needs graphs")
+        route = None
+        if weight_mask is not None:
+            gc = int(np.shape(weight_mask)[1])
+            if graph_cols is not None and graph_cols != gc:
+                raise Exception("CudaStepSolver: weight_mask has %d columns, graph_cols = %d" % (gc, graph_cols))
+            route = api.route_weight_mask(weight_mask, rows * gc, n, (rows, gc))
+        elif graphs is not None:
+            if graph_cols is None:
+                raise Exception("CudaStepSolver: graphs needs graph_cols, the number of columns of the whole frame")
+            route = api.route_graphs(graphs, rows * graph_cols, n, (rows, graph_cols), background_masks=background_masks)
+        if route is not None:
+            graph_cols = route.cols
+        self.frame_range = None
+        if route is not None:
+            self.frame_range = (0, n) if frames is None else (int(frames[0]), int(frames[1]))
+        elif frames is not None:
+            raise Exception("CudaStepSolver: frames applies to the graph modes given by graphs or weight_mask")
+        if delta is None:
+            delta = 1.0 if l1 else 10
         self.rows, self.cols_local, self.graph_cols = rows, cols_local, graph_cols
         # store_S_lazily: let the single-pass shrink kernel skip the store of S in iterations that cannot be the last (it is
         # rebuilt from D, Y and the digit planes at the end).  A clipped digit pass in such an iteration stops EVERY rank with
         # done == 5 in the same iteration (the flag is part of the all-reduced scalars); ShardedLSD then repeats the solve
         # with S stored every time.
         self.m = rows * cols_local
-        if graph_cols is not None:
+        if route is not None:
+            cfg = api.make_config(self.m, n, route.prox, rows, cols_local, delta=delta, m_global=m_global, d_global=min(m_global, n),
+                                  max_iter=max_iter)
+            self.lazy_S = False
+            self.dec = api.Decomposition(cfg)
+            self.dec.set_frame_route(route, *self.frame_range)
+        elif l1:
+            cfg = api.make_config(self.m, n, C.PROX_L1, 0, 0, delta=delta, mu_scale=1.25, rho=1.2, use_sv_prediction=False,
+                                  m_global=m_global, d_global=min(m_global, n), max_iter=max_iter, tile_rows=tile_rows,
+                                  cluster_frames=cluster_frames, flags=0 if store_S_lazily else C.FLAG_ALWAYS_STORE_S)
+            self.lazy_S = bool(store_S_lazily)
+            self.dec = api.Decomposition(cfg)
+        elif graph_cols is not None:
             if blocks is not None:
                 raise Exception("CudaStepSolver: blocks and graph_cols are mutually exclusive")
             cfg = api.make_config(self.m, n, C.PROX_GRAPH_LINF, rows, cols_local, delta=delta, m_global=m_global,
@@ -182,10 +225,23 @@ class CudaStepSolver:
         return torch.empty((max(nf, 1), ldf), dtype=torch.float32, device="cuda")
 
     def prox_frames(self, Uf, Vf, rows, cols, nf):
-        """Overlapping-window prox of nf whole frames (rows of Uf / Vf, row stride Uf.stride(0)) at this handle's lambda / mu."""
-        if nf > 0:
+        """Prox of this rank's nf whole frames (rows of Uf / Vf, row stride Uf.stride(0)) at this handle's lambda / mu."""
+        if self.frame_range is not None:
+            self.prox_block(Uf, Vf, self.frame_range[0], nf)
+        elif nf > 0:
             C.check(self.lib.bsub_step_prox_frames(self.h, ctypes.c_void_p(Uf.data_ptr()), ctypes.c_void_p(Vf.data_ptr()),
                                                    int(Uf.stride(0)), rows, cols, nf, self._s()))
+
+    def prox_block(self, Uf, Vf, f0, nf):
+        """Prox of the whole frames [f0, f0 + nf) of the clip, held in the rows of Uf / Vf: any block of this solver's frame range."""
+        C.check(self.lib.bsub_step_prox_block(self.h, ctypes.c_void_p(Uf.data_ptr()), ctypes.c_void_p(Vf.data_ptr()), int(Uf.stride(0)),
+                                              int(f0), int(nf), self._s()))
+
+    def debug_graph(self):
+        """bsub_debug_graph: outer iterations of the last prox call, their total, calls, calls that hit graph_max_sweeps."""
+        out = (ctypes.c_int64 * 4)()
+        C.check(self.lib.bsub_debug_graph(self.h, out))
+        return list(out)
 
     def block_sums_view(self):
         """l2-block mode: per-(frame, group) sums of squares of this shard, to be all-reduced between shrink_a and shrink_b."""
@@ -250,9 +306,10 @@ class CudaStepSolver:
 
 
 class ShardedLSD:
-    """inexact_alm_lsd (flat 3x3 groups) or inexact_alm_group_sparse_RPCA (l2 blocks, one more all-reduce per iteration: the
-    per-(frame, group) sums of squares) or the overlapping-window LSD (the prox runs on whole frames after an all-to-all to a frame
-    sharding, _prox_on_frames) over `comm.world` shards -- the step solver decides which.  hooks: optional callbacks
+    """inexact_alm_lsd (flat 3x3 groups), inexact_alm_rpca (l1), inexact_alm_group_sparse_RPCA (l2 blocks, one more all-reduce per
+    iteration: the per-(frame, group) sums of squares) or a graph mode -- any graph, with or without the background shrink (the
+    prox runs on whole frames after an all-to-all to a frame sharding, _prox_on_frames) -- over `comm.world` shards; the step
+    solver decides which.  A step solver with a `frame_range` must describe the frames shard_frames gives this rank.  hooks: optional callbacks
     hooks[name](phase) with phase in {'begin', 'end'} around 'gram', 'solve', 'shrink' for timing."""
 
     def __init__(self, solver, comm, run_ahead=3, max_iter=500, fence=None):
@@ -262,6 +319,10 @@ class ShardedLSD:
             fence = cuda_fence
         self.fence = fence
         self.iters_enqueued = 0
+        fr = getattr(solver, "frame_range", None)           # the frames this rank's prox gets from the exchange
+        if fr is not None and tuple(fr) != shard_frames(solver.n, comm.world, comm.rank):
+            raise Exception("ShardedLSD: the step solver describes frames [%d, %d), but rank %d of %d owns [%d, %d) (shard_frames)"
+                            % ((fr[0], fr[1], comm.rank, comm.world) + shard_frames(solver.n, comm.world, comm.rank)))
 
     def solve(self, hooks=None):
         s, comm = self.s, self.comm

@@ -154,14 +154,40 @@ int bsub_step_finish_iter(bsub_solver* s, void* stream);   /* err, mu update, st
 int bsub_step_shrink_a(bsub_solver* s, void* stream);
 int bsub_step_shrink_b(bsub_solver* s, void* stream);
 int bsub_block_sums_buffer(bsub_solver* s, double** sums, int64_t* count);
-/* Overlapping-window mode (inexact_alm_lsd.py:49-57) on pixel shards: the prox of a frame needs the whole image, so between the two
- * halves of the pass the driver re-shards G_S by FRAMES (all-to-all), runs the prox of its frames and brings S back:
- *   _shrink_a (G_S of this pixel shard into the buffer _prox_buffers returns) -> exchange -> _prox_frames (nf whole frames of
- *   rows x cols pixels, device pointers, lambda/mu and the stop flag from this handle's device state) -> exchange (result into the S
- *   pointer of _prox_buffers) -> _shrink_b.  All-window graphs with unit weights only. */
+/* Graph modes on pixel shards: the prox of a frame needs the whole image but no other frame, so between the two halves of the pass
+ * the driver re-shards G_S by FRAMES (all-to-all), runs the prox of its frames and brings S back:
+ *   _shrink_a (G_S of this pixel shard into the buffer _prox_buffers returns) -> exchange -> prox of nf whole frames of rows x cols
+ *   pixels (device pointers, lambda/mu and the stop flag from this handle's device state) -> exchange (result into the S pointer of
+ *   _prox_buffers) -> _shrink_b.
+ * bsub_step_prox_frames: all-window graphs with unit weights, on a handle set up with bsub_set_graph_windows (whose _shrink_a always
+ * stops before the prox).
+ * bsub_step_prox_block: every graph mode, on a handle that holds a frame-range description (bsub_set_frame_*, below); once it has
+ * one, _shrink_a stops before the prox and _shrink_b finishes the pass in BSUB_PROX_GRAPH_CENTER_BG / _GENERIC too.  The l1 mode
+ * (BSUB_PROX_L1) is elementwise and shards with bsub_step_shrink alone. */
 int bsub_step_prox_buffers(bsub_solver* s, float** G_S, float** S, int64_t* ld);
 int bsub_step_prox_frames(bsub_solver* s, const float* U_frames, float* V_frames, int64_t ld_frames, int32_t rows, int32_t cols,
                           int32_t n_frames, void* stream);
+/* Frame-range descriptions: the prox of whole rows x cols frames [f0, f0 + nf) of the clip (the frames this rank owns after the
+ * exchange; nf may be 0).  Only those frames' data is copied, every entry is validated before anything reaches the device, and a new
+ * description replaces the previous one.  A handle that holds only such a description has no graph for its own pixels: bsub_run and
+ * bsub_step_shrink refuse it.
+ *   _windows (BSUB_PROX_GRAPH_LINF): the 3x3 all-window graph, eta double[n_eta] one weight per window as bsub_set_graph_windows
+ *     takes it (finite, >= 0), the same in every frame; NULL: unit weights.
+ *   _center_windows (BSUB_PROX_GRAPH_CENTER_BG): eta float32[nf][rows*cols] and background uint8[nf][rows*cols] as
+ *     bsub_set_center_windows takes them for frames f0 .. f0 + nf - 1.
+ *   _graphs (BSUB_PROX_GRAPH_GENERIC): graphs as bsub_set_graphs takes them (indices < rows*cols), frame_graph[nf] for frames
+ *     f0 .. f0 + nf - 1, background uint8[nf][rows*cols] or NULL. */
+int bsub_set_frame_windows(bsub_solver* s, int32_t rows, int32_t cols, int32_t f0, int32_t nf, const double* eta_host, int64_t n_eta);
+int bsub_set_frame_center_windows(bsub_solver* s, int32_t rows, int32_t cols, int32_t f0, int32_t nf, const float* eta_host,
+                                  const uint8_t* background_host);
+int bsub_set_frame_graphs(bsub_solver* s, int32_t rows, int32_t cols, int32_t f0, int32_t nf, int32_t n_graphs, const int32_t* frame_graph,
+                          const int64_t* n_groups, const int32_t* const* indptr, const int32_t* const* indices, const double* const* eta,
+                          const uint8_t* background_host);
+/* prox of the whole frames [f0, f0 + nf) -- any sub-range of the described one, else an error; nf == 0 does nothing -- held in
+ * U_frames / V_frames (row f - f0 = frame f, row pitch ld_frames >= rows*cols): the tile kernel (windows, centre windows) or the
+ * generic kernel, then the l2 shrink of each frame's background when one was given.  Whole-frame workspaces are allocated once and
+ * grow with the largest block (BSUB_GRAPH_XI_MB caps the duals); bsub_debug_graph counts the calls. */
+int bsub_step_prox_block(bsub_solver* s, const float* U_frames, float* V_frames, int64_t ld_frames, int32_t f0, int32_t nf, void* stream);
 int bsub_poll(bsub_solver* s, bsub_status* st);            /* non-blocking: host mirror written by the device       */
 int bsub_sync_status(bsub_solver* s, bsub_status* st, void* stream);   /* blocking                                 */
 
