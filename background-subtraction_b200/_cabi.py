@@ -70,7 +70,6 @@ SIGNATURES = {
     "bsub_step_shrink_b": (ctypes.c_int, [vp, vp]),
     "bsub_block_sums_buffer": (ctypes.c_int, [vp, ctypes.POINTER(vp), ctypes.POINTER(ctypes.c_int64)]),
     "bsub_step_prox_buffers": (ctypes.c_int, [vp, ctypes.POINTER(vp), ctypes.POINTER(vp), c_int64_p]),
-    "bsub_step_prox_frames": (ctypes.c_int, [vp, vp, vp, ctypes.c_int64, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, vp]),
     "bsub_set_frame_windows": (ctypes.c_int, [vp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, c_double_p, ctypes.c_int64]),
     "bsub_set_frame_center_windows": (ctypes.c_int, [vp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, c_float_p, c_uint8_p]),
     "bsub_set_frame_graphs": (ctypes.c_int, [vp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, c_int32_p,

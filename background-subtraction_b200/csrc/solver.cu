@@ -35,6 +35,31 @@ using namespace bsub;
 static const int kCommTail = 16;     // doubles after the Gram in the sum buffer
 static const int kRunAhead = 3;      // iterations the host may enqueue ahead of the device
 
+// The prox of whole rows x cols frames [f0, f0 + nf) of a clip (m pixels each; the generic kernel needs m alone), as one setter or
+// one stand-alone operator describes it.  Built by describe_windows / _centre / _graphs, run by graph_prox.
+struct GraphDesc {
+    int kind = 0;                                       // BSUB_PROX_GRAPH_LINF (windows), _CENTER_BG (centre map), _GENERIC; 0: none
+    int rows = 0, cols = 0, f0 = 0, nf = 0;
+    long long m = 0;
+    float* eta = nullptr; long long eta_stride = 0;     // tile kernel: window weights (stride 0; NULL: unit) or centre map [nf][m]
+    int* ints = nullptr; GenericGraphDev graphs = {};   // generic kernel: packed graphs, their eta in graphs.eta, frame_graph[nf]
+    unsigned char* labels = nullptr; double* bsums = nullptr;   // background (label 0) [nf][m] and its per-frame sums, or none
+    void release() {
+        for (void* p : {(void*)eta, (void*)ints, (void*)graphs.eta, (void*)labels, (void*)bsums}) if (p) cudaFree(p);
+        *this = GraphDesc();
+    }
+};
+
+// duals of the graph prox: allocated once, grown when a call needs more
+struct ProxWork {
+    float *xi = nullptr, *tot = nullptr;
+    long long xi_floats = 0, tot_floats = 0;
+    void release() {
+        for (float* p : {xi, tot}) if (p) cudaFree(p);
+        *this = ProxWork();
+    }
+};
+
 struct bsub_solver {
     bsub_config cfg;
     int device = 0, num_sms = 148;
@@ -64,18 +89,10 @@ struct bsub_solver {
     int shrink_mode = SHRINK_FLAT3;
     // generic flat groups
     int* gptr = nullptr; int* gidx = nullptr; int ngroups = 0; bool groups_set = false;
-    // overlapping graph
-    float* eta_dev = nullptr; float* xi = nullptr; long long xi_floats = 0; float* tot = nullptr;
-    float* xi2 = nullptr; float* tot2 = nullptr; int* sweeps2 = nullptr; long long xi2_floats = 0, tot2_floats = 0;   // bsub_step_prox_frames / _prox_block
-    int* sweeps_dev = nullptr; bool graph_set = false;
-    // any graphs (BSUB_PROX_GRAPH_GENERIC): packed index arrays + eta on the device, where tot lives; xi / tot / sweeps_dev above
-    int* pg_ints = nullptr; float* pg_eta = nullptr; GenericGraphDev pg_dev; GenericGraphLayout pg_layout; bool pg_bg = false;
-    // frame-range description (bsub_set_frame_*): the prox of whole rows x cols frames [fr_f0, fr_f0 + fr_nf) of the clip, run by
-    // bsub_step_prox_block on the frames a pixel-sharded driver has gathered; workspaces xi2 / tot2 above
-    bool fr_set = false; int fr_rows = 0, fr_cols = 0, fr_f0 = 0, fr_nf = 0;
-    float* fr_eta = nullptr; long long fr_eta_stride = 0;           // tile kernel: window weights (stride 0) or centre map [nf][m]
-    int* fr_ints = nullptr; float* fr_geta = nullptr; GenericGraphDev fr_graph; long long fr_max_nnz = 0;   // generic kernel
-    unsigned char* fr_labels = nullptr; double* fr_bsums = nullptr;   // background (label 0) [nf][m] and its sums, or none
+    // graph modes: the one description (whole-clip: bsub_set_graph_windows / _center_windows / _graphs, run by the SPILL pass; else
+    // a frame range: bsub_set_frame_*, run by bsub_step_prox_block on the frames a pixel-sharded driver has gathered), the duals of
+    // its prox and the counters bsub_debug_graph reads
+    GraphDesc graph; bool graph_whole = false; ProxWork work; int* sweeps_dev = nullptr;
     // l2 blocks
     unsigned char* labels_dev = nullptr; double* lam_table = nullptr; double* bsums = nullptr; int nlab = 0; bool blocks_set = false;
     unsigned char* mask_stage = nullptr;      // bsub_mask_host staging
@@ -123,6 +140,119 @@ struct DevScope {
     }
 };
 
+// ----------------------------------------------------------------------------------------------------- graph prox descriptions
+// Each builder validates every entry, then uploads *d; on failure *d holds nothing.  args_ok = false: the caller's own arguments are
+// bad, reported after the description's errors and before any device call.
+static long long window_count(int rows, int cols) { return (long long)(rows - std::min(3, rows) + 1) * (cols - std::min(3, cols) + 1); }
+
+// eta float[n_eta] (n_eta may be 0) and background uint8[nf][m] (may be NULL) -> label 0 (the complement group of the l2 kernels) /
+// 255 (keeps the graph prox result)
+static int describe_upload(GraphDesc* d, const float* eta, size_t n_eta, const uint8_t* background) {
+    const int rc = [&]() -> int {
+        if (n_eta > 0) {
+            CK(cudaMalloc((void**)&d->eta, sizeof(float) * n_eta));
+            CK(cudaMemcpy(d->eta, eta, sizeof(float) * n_eta, cudaMemcpyHostToDevice));
+        }
+        if (background == nullptr || d->nf == 0) return 0;
+        const size_t nm = (size_t)d->nf * d->m;
+        std::vector<unsigned char> lab(nm);
+        for (size_t i = 0; i < nm; ++i) lab[i] = background[i] ? 0 : 255;
+        CK(cudaMalloc((void**)&d->labels, nm));
+        CK(cudaMalloc((void**)&d->bsums, sizeof(double) * d->nf));
+        CK(cudaMemcpy(d->labels, lab.data(), nm, cudaMemcpyHostToDevice));
+        return 0;
+    }();
+    if (rc != 0) d->release();
+    return rc;
+}
+
+// the 3x3 all-window graph, eta double[n_eta] one weight per window (finite, >= 0) the same in every frame; NULL: unit weights
+static int describe_windows(GraphDesc* d, int rows, int cols, int f0, int nf, const double* eta, long long n_eta, const char* who,
+                            bool args_ok = true) {
+    const long long nw = window_count(rows, cols);
+    std::vector<float> ef;
+    if (eta != nullptr) {
+        if (n_eta != nw) { set_error("%s: eta has %lld entries, the %dx%d image has %lld windows", who, n_eta, rows, cols, nw); return -1; }
+        ef.resize((size_t)nw);
+        for (long long i = 0; i < nw; ++i) {
+            if (!(std::isfinite(eta[i]) && eta[i] >= 0.0)) { set_error("%s: eta[%lld] = %g is not finite and >= 0", who, i, eta[i]); return -1; }
+            ef[i] = (float)eta[i];
+        }
+    }
+    if (!args_ok) { set_error("%s: bad argument", who); return -1; }
+    *d = GraphDesc{BSUB_PROX_GRAPH_LINF, rows, cols, f0, nf, (long long)rows * cols};
+    return describe_upload(d, ef.data(), ef.size(), nullptr);
+}
+
+// radius-1 centre windows, eta float32[nf][rows*cols] (finite) = weight of the window centred on that pixel in that frame
+static int describe_centre(GraphDesc* d, int rows, int cols, int f0, int nf, const float* eta, const uint8_t* background, const char* who,
+                           bool args_ok = true) {
+    const size_t nm = (rows > 0 && cols > 0 && nf > 0) ? (size_t)nf * rows * cols : 0;
+    for (size_t i = 0; i < nm; ++i)
+        if (!std::isfinite(eta[i])) { set_error("%s: eta[%zu] = %g is not finite", who, i, (double)eta[i]); return -1; }
+    if (!args_ok) { set_error("%s: bad argument", who); return -1; }
+    *d = GraphDesc{BSUB_PROX_GRAPH_CENTER_BG, rows, cols, f0, nf, (long long)rows * cols};
+    d->eta_stride = d->m;
+    return describe_upload(d, eta, nm, background);
+}
+
+// any non-nested graphs (the generic kernel), frame_graph[nf] for the frames of the range
+static int describe_graphs(GraphDesc* d, int rows, int cols, long long m, int f0, int nf, int n_graphs, const int32_t* frame_graph,
+                           const int64_t* n_groups, const int32_t* const* indptr, const int32_t* const* indices, const double* const* eta,
+                           const uint8_t* background, const char* who, bool args_ok = true) {
+    GenericGraphHost H;
+    if (nf > 0) RET_IF(pack_generic_graphs(m, nf, n_graphs, frame_graph, n_groups, indptr, indices, eta, &H, who));
+    if (!args_ok) { set_error("%s: bad argument", who); return -1; }
+    *d = GraphDesc{BSUB_PROX_GRAPH_GENERIC, rows, cols, f0, nf, m};
+    if (nf > 0) {
+        float* geta = nullptr;
+        const int rc = upload_generic_graphs(H, &d->ints, &geta, &d->graphs);
+        d->graphs.eta = geta;                           // d owns it whether or not the upload finished
+        if (rc != 0) { d->release(); return rc; }
+    }
+    return describe_upload(d, nullptr, 0, background);
+}
+
+// the duals of nf frames of d at row pitch ld, grown in *w; *L: the generic kernel's layout
+static int size_work(const GraphDesc& d, long long ld, int nf, ProxWork* w, long long* xi_floats, GenericGraphLayout* L) {
+    long long tot_floats = 0;
+    if (d.kind == BSUB_PROX_GRAPH_GENERIC) {
+        *L = prox_graph_generic_layout(d.m, ld, nf, d.graphs.max_nnz);
+        *xi_floats = L->xi_floats; tot_floats = L->tot_floats;
+    } else {
+        prox_graph3_workspace(d.rows, d.cols, nf, ld, d.kind == BSUB_PROX_GRAPH_CENTER_BG ? 1 : 0, xi_floats, &tot_floats);
+    }
+    RET_IF(grow_floats(&w->xi, &w->xi_floats, *xi_floats));
+    return grow_floats(&w->tot, &w->tot_floats, tot_floats);
+}
+
+// prox of the whole frames [f0, f0 + nf) -- within d's range -- held in U / V (row f - f0 = frame f, row pitch ld): the tile or the
+// generic kernel, then the l2 shrink of each frame's background.  st != nullptr: lambda / mu and the stop flag come from the device
+// state, else lam is lambda1.  sweeps: the int[8] status block of the prox kernels.
+static int graph_prox(const GraphDesc& d, const float* U, float* V, long long ld, int f0, int nf, const DevState* st, float lam,
+                      int max_sweeps, float tol, int* sweeps, ProxWork* w, cudaStream_t stream) {
+    if (nf == 0) return 0;
+    const int lf = f0 - d.f0;
+    long long xi_floats = 0;
+    GenericGraphLayout L;
+    RET_IF(size_work(d, ld, nf, w, &xi_floats, &L));
+    if (d.kind == BSUB_PROX_GRAPH_GENERIC) {
+        GenericGraphDev g = d.graphs;
+        g.frame_graph += lf;
+        RET_IF(launch_prox_graph_generic(U, V, ld, d.m, nf, g, L, w->xi, w->tot, lam, max_sweeps, tol, sweeps, st, stream));
+    } else {
+        const float* eta = d.eta ? d.eta + (size_t)lf * d.eta_stride : nullptr;
+        RET_IF(launch_prox_graph3(U, V, w->xi, xi_floats, w->tot, eta, ld, d.rows, d.cols, nf, lam, max_sweeps, tol, sweeps, st, stream,
+                                  d.kind == BSUB_PROX_GRAPH_CENTER_BG ? 1 : 0, d.eta_stride));
+    }
+    if (d.labels) {       // background pixels: their frame's l2 shrink of G_S at non_block_lambda / mu, over the graph prox result
+        const unsigned char* lab = d.labels + (size_t)lf * d.m;
+        RET_IF(launch_block_l2_sums(U, lab, ld, d.m, nf, 1, d.bsums, st, stream));
+        RET_IF(launch_block_l2_apply(U, V, lab, ld, d.m, nf, 1, d.bsums, nullptr, st, 0.0, 0.0, stream, 1));
+    }
+    return 0;
+}
+
 static int round_half_even_005(int d) {
     // Python round(0.05 * d) -- banker's rounding on the double product (SURVEY Q5)
     return (int)nearbyint(0.05 * (double)d);
@@ -153,10 +283,11 @@ int bsub_destroy(bsub_solver* s) {
     if (s->stream_seen) cudaStreamSynchronize(s->last_stream); else cudaDeviceSynchronize();
     void* ptrs[] = {s->D, s->S, s->Y, s->T, s->L, s->U, s->st, s->log, s->comm_sum, s->comm_max, s->tasks_dev, s->gram_partial,
                     s->eb.work, s->eb.lam, s->eb.Z, s->eb.Vr, s->eb.VC, s->tpart, s->part_zz, s->part_nnz, s->part_max, s->gptr,
-                    s->gidx, s->eta_dev, s->xi, s->tot, s->sweeps_dev, s->labels_dev, s->lam_table, s->bsums, s->Wq, s->Gint,
-                    s->gi_info, s->gi_blkn, s->part_wmax, s->mask_stage, s->mask_scratch, s->stage64, s->Tt, s->xi2, s->tot2, s->sweeps2,
-                    s->pg_ints, s->pg_eta, s->fr_eta, s->fr_ints, s->fr_geta, s->fr_labels, s->fr_bsums};
+                    s->gidx, s->sweeps_dev, s->labels_dev, s->lam_table, s->bsums, s->Wq, s->Gint, s->gi_info, s->gi_blkn, s->part_wmax,
+                    s->mask_stage, s->mask_scratch, s->stage64, s->Tt};
     for (void* p : ptrs) if (p) cudaFree(p);
+    s->graph.release();
+    s->work.release();
     if (s->mirror) cudaFreeHost((void*)s->mirror);
     for (int i = 0; i <= kRunAhead; ++i) if (s->ev[i]) cudaEventDestroy(s->ev[i]);
     const int own = s->device;
@@ -203,6 +334,8 @@ int bsub_create(const bsub_config* cfg, bsub_solver** out) {
         ALLOC(s->st, sizeof(DevState)); ALLOC(s->log, sizeof(IterLog) * kMaxIterLog);
         ALLOC(s->comm_sum, sizeof(double) * ((size_t)s->npad * s->npad + kCommTail));
         ALLOC(s->comm_max, sizeof(double) * 8);
+        ALLOC(s->sweeps_dev, sizeof(int) * 8);
+        cudaMemset(s->sweeps_dev, 0, sizeof(int) * 8);
         ALLOC(s->mask_scratch, sizeof(double) * mask_stats_scratch_doubles());
         cudaMemset(s->mask_scratch, 0, sizeof(double) * mask_stats_scratch_doubles());
         cudaMemset(s->comm_sum, 0, sizeof(double) * ((size_t)s->npad * s->npad + kCommTail));
@@ -341,89 +474,55 @@ int bsub_set_flat_groups(bsub_solver* s, const int32_t* g) {
     return 0;
 }
 
-int bsub_set_graph_windows(bsub_solver* s, const double* eta, int64_t n_eta) {
-    if (!s) { set_error("bsub_set_graph_windows: null solver"); return -1; }
-    if (s->cfg.prox != BSUB_PROX_GRAPH_LINF) { set_error("bsub_set_graph_windows: solver was not created with BSUB_PROX_GRAPH_LINF"); return -1; }
-    const int rows = s->cfg.rows, cols = s->cfg.cols;
-    const long long nwi = rows - std::min(3, rows) + 1, nwj = cols - std::min(3, cols) + 1, nw = nwi * nwj;
-    if (eta != nullptr) {
-        if (n_eta != nw) { set_error("bsub_set_graph_windows: eta has %lld entries, the %dx%d image has %lld windows", (long long)n_eta, rows, cols, nw); return -1; }
-        std::vector<float> ef((size_t)nw);
-        for (long long i = 0; i < nw; ++i) ef[i] = (float)eta[i];
-        if (!s->eta_dev) CK(cudaMalloc((void**)&s->eta_dev, sizeof(float) * nw));
-        CK(cudaMemcpy(s->eta_dev, ef.data(), sizeof(float) * nw, cudaMemcpyHostToDevice));
-    }
-    // duals of the overlapping windows: whole frames up to a cap (the prox kernel walks the frames in chunks that fit)
-    if (!s->xi) {
-        long long tot_floats = 0;
-        prox_graph3_workspace(rows, cols, s->n, s->ld, 0, &s->xi_floats, &tot_floats);
-        CK(cudaMalloc((void**)&s->xi, sizeof(float) * (size_t)s->xi_floats));
-        CK(cudaMalloc((void**)&s->tot, sizeof(float) * (size_t)tot_floats));
-    }
-    if (!s->sweeps_dev) { CK(cudaMalloc((void**)&s->sweeps_dev, sizeof(int) * 8)); CK(cudaMemset(s->sweeps_dev, 0, sizeof(int) * 8)); }
-    s->graph_set = true;
+static int check_prox(bsub_solver* s, int prox, const char* prox_name, const char* who) {
+    if (!s) { set_error("%s: null solver", who); return -1; }
+    if (s->cfg.prox != prox) { set_error("%s: solver was not created with %s", who, prox_name); return -1; }
     return 0;
+}
+
+// d becomes the handle's description and the previous one is released.  A whole-clip one gets the duals of all n frames at the
+// handle's ld here, so that bsub_run allocates nothing inside its loop.
+static int set_graph(bsub_solver* s, const GraphDesc& d, bool whole) {
+    s->graph.release();
+    s->graph = d;
+    s->graph_whole = whole;
+    if (!whole) return 0;
+    long long xi_floats = 0;
+    GenericGraphLayout L;
+    return size_work(s->graph, s->ld, s->n, &s->work, &xi_floats, &L);
+}
+
+// a frame-range description only: the handle has no graph of its own pixels
+static bool frame_range_only(const bsub_solver* s) { return s->graph.kind != 0 && !s->graph_whole; }
+
+int bsub_set_graph_windows(bsub_solver* s, const double* eta, int64_t n_eta) {
+    RET_IF(check_prox(s, BSUB_PROX_GRAPH_LINF, "BSUB_PROX_GRAPH_LINF", "bsub_set_graph_windows"));
+    GraphDesc d;
+    RET_IF(describe_windows(&d, s->cfg.rows, s->cfg.cols, 0, s->n, eta, n_eta, "bsub_set_graph_windows"));
+    return set_graph(s, d, true);
 }
 
 int bsub_set_center_windows(bsub_solver* s, const float* eta, const uint8_t* background) {
     if (!s || !eta || !background) { set_error("bsub_set_center_windows: null argument"); return -1; }
-    if (s->cfg.prox != BSUB_PROX_GRAPH_CENTER_BG) { set_error("bsub_set_center_windows: solver was not created with BSUB_PROX_GRAPH_CENTER_BG"); return -1; }
-    const size_t nm = (size_t)s->n * s->m;
-    // background pixels form label 0 (the "complement" group of the l2 kernels, shrunk at non_block_lambda = 100 lambda);
-    // everything else gets a label no group uses and keeps the graph prox result
-    std::vector<unsigned char> lab(nm);
-    for (size_t i = 0; i < nm; ++i) lab[i] = background[i] ? 0 : 255;
-    if (!s->eta_dev) CK(cudaMalloc((void**)&s->eta_dev, sizeof(float) * nm));
-    if (!s->labels_dev) CK(cudaMalloc((void**)&s->labels_dev, nm));
-    if (!s->bsums) CK(cudaMalloc((void**)&s->bsums, sizeof(double) * s->n));
-    CK(cudaMemcpy(s->eta_dev, eta, sizeof(float) * nm, cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(s->labels_dev, lab.data(), nm, cudaMemcpyHostToDevice));
-    s->nlab = 1;
-    // one candidate window per pixel and frame
-    if (!s->xi) {
-        long long tot_floats = 0;
-        prox_graph3_workspace(s->cfg.rows, s->cfg.cols, s->n, s->ld, 1, &s->xi_floats, &tot_floats);
-        CK(cudaMalloc((void**)&s->xi, sizeof(float) * (size_t)s->xi_floats));
-        CK(cudaMalloc((void**)&s->tot, sizeof(float) * (size_t)tot_floats));
-    }
-    if (!s->sweeps_dev) { CK(cudaMalloc((void**)&s->sweeps_dev, sizeof(int) * 8)); CK(cudaMemset(s->sweeps_dev, 0, sizeof(int) * 8)); }
-    s->graph_set = true;
-    return 0;
+    RET_IF(check_prox(s, BSUB_PROX_GRAPH_CENTER_BG, "BSUB_PROX_GRAPH_CENTER_BG", "bsub_set_center_windows"));
+    GraphDesc d;
+    RET_IF(describe_centre(&d, s->cfg.rows, s->cfg.cols, 0, s->n, eta, background, "bsub_set_center_windows"));
+    return set_graph(s, d, true);
 }
 
 int bsub_set_graphs(bsub_solver* s, int32_t n_graphs, const int32_t* frame_graph, const int64_t* n_groups, const int32_t* const* indptr,
                     const int32_t* const* indices, const double* const* eta, const uint8_t* background) {
-    if (!s) { set_error("bsub_set_graphs: null solver"); return -1; }
-    if (s->cfg.prox != BSUB_PROX_GRAPH_GENERIC) { set_error("bsub_set_graphs: solver was not created with BSUB_PROX_GRAPH_GENERIC"); return -1; }
-    GenericGraphHost H;
-    RET_IF(pack_generic_graphs(s->m, s->n, n_graphs, frame_graph, n_groups, indptr, indices, eta, &H, "bsub_set_graphs"));
-    RET_IF(upload_generic_graphs(H, &s->pg_ints, &s->pg_eta, &s->pg_dev));
-    s->pg_layout = prox_graph_generic_layout(s->m, s->ld, s->n, H.max_nnz);
-    if (s->xi) { cudaFree(s->xi); s->xi = nullptr; }
-    if (s->tot) { cudaFree(s->tot); s->tot = nullptr; }
-    CK(cudaMalloc((void**)&s->xi, sizeof(float) * (size_t)s->pg_layout.xi_floats));
-    if (s->pg_layout.tot_floats > 0) CK(cudaMalloc((void**)&s->tot, sizeof(float) * (size_t)s->pg_layout.tot_floats));
-    s->xi_floats = s->pg_layout.xi_floats;
-    s->pg_bg = background != nullptr;
-    if (s->pg_bg) {           // label 0 = background (the complement group of the l2 kernels), 255 = keeps the graph prox result
-        const size_t nm = (size_t)s->n * s->m;
-        std::vector<unsigned char> lab(nm);
-        for (size_t i = 0; i < nm; ++i) lab[i] = background[i] ? 0 : 255;
-        if (!s->labels_dev) CK(cudaMalloc((void**)&s->labels_dev, nm));
-        if (!s->bsums) CK(cudaMalloc((void**)&s->bsums, sizeof(double) * s->n));
-        CK(cudaMemcpy(s->labels_dev, lab.data(), nm, cudaMemcpyHostToDevice));
-        s->nlab = 1;
-    }
-    if (!s->sweeps_dev) { CK(cudaMalloc((void**)&s->sweeps_dev, sizeof(int) * 8)); CK(cudaMemset(s->sweeps_dev, 0, sizeof(int) * 8)); }
-    s->graph_set = true;
-    return 0;
+    RET_IF(check_prox(s, BSUB_PROX_GRAPH_GENERIC, "BSUB_PROX_GRAPH_GENERIC", "bsub_set_graphs"));
+    GraphDesc d;                  // the handle's m: the generic kernel needs no image geometry
+    RET_IF(describe_graphs(&d, s->cfg.rows, s->cfg.cols, s->m, 0, s->n, n_graphs, frame_graph, n_groups, indptr, indices, eta, background,
+                           "bsub_set_graphs"));
+    return set_graph(s, d, true);
 }
 
 // ---------------------------------------------------------------------------- frame-range descriptions (bsub_step_prox_block)
 static int frame_range_check(bsub_solver* s, int prox, const char* prox_name, int32_t rows, int32_t cols, int32_t f0, int32_t nf,
                              const char* who) {
-    if (!s) { set_error("%s: null solver", who); return -1; }
-    if (s->cfg.prox != prox) { set_error("%s: solver was not created with %s", who, prox_name); return -1; }
+    RET_IF(check_prox(s, prox, prox_name, who));
     if (rows <= 0 || cols <= 0 || (long long)rows * cols > (1LL << 30)) { set_error("%s: bad frame geometry %d x %d", who, rows, cols); return -1; }
     if (f0 < 0 || nf < 0 || (long long)f0 + nf > s->n) {
         set_error("%s: frames [%d, %lld) are not a range of the %d frames of the clip", who, f0, (long long)f0 + nf, s->n); return -1;
@@ -431,76 +530,29 @@ static int frame_range_check(bsub_solver* s, int prox, const char* prox_name, in
     return 0;
 }
 
-// drops the previous description; the new one takes effect once everything has been uploaded
-static void frame_range_clear(bsub_solver* s) {
-    for (void* p : {(void*)s->fr_eta, (void*)s->fr_ints, (void*)s->fr_geta, (void*)s->fr_labels, (void*)s->fr_bsums}) if (p) cudaFree(p);
-    s->fr_eta = nullptr; s->fr_ints = nullptr; s->fr_geta = nullptr; s->fr_labels = nullptr; s->fr_bsums = nullptr;
-    s->fr_set = false; s->fr_eta_stride = 0; s->fr_max_nnz = 0;
-}
-
-// background uint8[nf][m] (may be NULL) -> label 0 (the complement group of the l2 kernels) / 255 (keeps the graph prox result)
-static int frame_range_finish(bsub_solver* s, int32_t rows, int32_t cols, int32_t f0, int32_t nf, const uint8_t* background) {
-    const size_t nm = (size_t)nf * rows * cols;
-    if (background != nullptr && nf > 0) {
-        std::vector<unsigned char> lab(nm);
-        for (size_t i = 0; i < nm; ++i) lab[i] = background[i] ? 0 : 255;
-        CK(cudaMalloc((void**)&s->fr_labels, nm));
-        CK(cudaMalloc((void**)&s->fr_bsums, sizeof(double) * nf));
-        CK(cudaMemcpy(s->fr_labels, lab.data(), nm, cudaMemcpyHostToDevice));
-    }
-    if (!s->sweeps_dev) { CK(cudaMalloc((void**)&s->sweeps_dev, sizeof(int) * 8)); CK(cudaMemset(s->sweeps_dev, 0, sizeof(int) * 8)); }
-    s->fr_rows = rows; s->fr_cols = cols; s->fr_f0 = f0; s->fr_nf = nf;
-    s->fr_set = true;
-    return 0;
-}
-
 int bsub_set_frame_windows(bsub_solver* s, int32_t rows, int32_t cols, int32_t f0, int32_t nf, const double* eta, int64_t n_eta) {
     RET_IF(frame_range_check(s, BSUB_PROX_GRAPH_LINF, "BSUB_PROX_GRAPH_LINF", rows, cols, f0, nf, "bsub_set_frame_windows"));
-    const long long nw = (long long)(rows - std::min(3, rows) + 1) * (cols - std::min(3, cols) + 1);
-    std::vector<float> ef;
-    if (eta != nullptr) {
-        if (n_eta != nw) { set_error("bsub_set_frame_windows: eta has %lld entries, the %dx%d image has %lld windows", (long long)n_eta, rows, cols, nw); return -1; }
-        ef.resize((size_t)nw);
-        for (long long i = 0; i < nw; ++i) {
-            if (!(std::isfinite(eta[i]) && eta[i] >= 0.0)) { set_error("bsub_set_frame_windows: eta[%lld] = %g is not finite and >= 0", i, eta[i]); return -1; }
-            ef[i] = (float)eta[i];
-        }
-    }
-    frame_range_clear(s);
-    if (eta != nullptr) {                  // the same weights in every frame
-        CK(cudaMalloc((void**)&s->fr_eta, sizeof(float) * nw));
-        CK(cudaMemcpy(s->fr_eta, ef.data(), sizeof(float) * nw, cudaMemcpyHostToDevice));
-    }
-    return frame_range_finish(s, rows, cols, f0, nf, nullptr);
+    GraphDesc d;
+    RET_IF(describe_windows(&d, rows, cols, f0, nf, eta, n_eta, "bsub_set_frame_windows"));
+    return set_graph(s, d, false);
 }
 
 int bsub_set_frame_center_windows(bsub_solver* s, int32_t rows, int32_t cols, int32_t f0, int32_t nf, const float* eta, const uint8_t* background) {
     RET_IF(frame_range_check(s, BSUB_PROX_GRAPH_CENTER_BG, "BSUB_PROX_GRAPH_CENTER_BG", rows, cols, f0, nf, "bsub_set_frame_center_windows"));
-    const size_t nm = (size_t)nf * rows * cols;
     if (nf > 0 && (!eta || !background)) { set_error("bsub_set_frame_center_windows: null argument"); return -1; }
-    for (size_t i = 0; i < nm; ++i)
-        if (!std::isfinite(eta[i])) { set_error("bsub_set_frame_center_windows: eta[%zu] = %g is not finite", i, (double)eta[i]); return -1; }
-    frame_range_clear(s);
-    if (nf > 0) {
-        CK(cudaMalloc((void**)&s->fr_eta, sizeof(float) * nm));
-        CK(cudaMemcpy(s->fr_eta, eta, sizeof(float) * nm, cudaMemcpyHostToDevice));
-    }
-    s->fr_eta_stride = (long long)rows * cols;
-    return frame_range_finish(s, rows, cols, f0, nf, background);
+    GraphDesc d;
+    RET_IF(describe_centre(&d, rows, cols, f0, nf, eta, background, "bsub_set_frame_center_windows"));
+    return set_graph(s, d, false);
 }
 
 int bsub_set_frame_graphs(bsub_solver* s, int32_t rows, int32_t cols, int32_t f0, int32_t nf, int32_t n_graphs, const int32_t* frame_graph,
                           const int64_t* n_groups, const int32_t* const* indptr, const int32_t* const* indices, const double* const* eta,
                           const uint8_t* background) {
     RET_IF(frame_range_check(s, BSUB_PROX_GRAPH_GENERIC, "BSUB_PROX_GRAPH_GENERIC", rows, cols, f0, nf, "bsub_set_frame_graphs"));
-    GenericGraphHost H;
-    if (nf > 0) RET_IF(pack_generic_graphs((long long)rows * cols, nf, n_graphs, frame_graph, n_groups, indptr, indices, eta, &H, "bsub_set_frame_graphs"));
-    frame_range_clear(s);
-    if (nf > 0) {
-        RET_IF(upload_generic_graphs(H, &s->fr_ints, &s->fr_geta, &s->fr_graph));
-        s->fr_max_nnz = H.max_nnz;
-    }
-    return frame_range_finish(s, rows, cols, f0, nf, background);
+    GraphDesc d;
+    RET_IF(describe_graphs(&d, rows, cols, (long long)rows * cols, f0, nf, n_graphs, frame_graph, n_groups, indptr, indices, eta, background,
+                           "bsub_set_frame_graphs"));
+    return set_graph(s, d, false);
 }
 
 int bsub_set_blocks(bsub_solver* s, const uint8_t* labels, const int32_t* lam_ptr, const double* lam) {
@@ -642,7 +694,7 @@ static int check_ready(bsub_solver* s) {
     if (!s->loaded) { set_error("no data loaded (call bsub_load_* first)"); return -1; }
     if (s->cfg.prox == BSUB_PROX_FLAT_LINF && !s->groups_set) { set_error("one of graphs or groups must not be None"); return -1; }
     if ((s->cfg.prox == BSUB_PROX_GRAPH_LINF || s->cfg.prox == BSUB_PROX_GRAPH_CENTER_BG || s->cfg.prox == BSUB_PROX_GRAPH_GENERIC) &&
-        !s->graph_set && !s->fr_set) { set_error("one of graphs or groups must not be None"); return -1; }
+        s->graph.kind == 0) { set_error("one of graphs or groups must not be None"); return -1; }
     if (s->cfg.prox == BSUB_PROX_BLOCK_L2 && !s->blocks_set) { set_error("blocks_by_frame / lambdas_by_frame not set"); return -1; }
     return 0;
 }
@@ -715,11 +767,11 @@ static int step_shrink_impl(bsub_solver* s, void* stream, int part) {
     if (!s || !s->initialised) { set_error("bsub_step_shrink: solver not initialised"); return -1; }
     cudaStream_t st = use_stream(s, stream);
     // the overlapping-window mode splits too: between the halves the driver re-shards G_S by FRAMES (the prox of a frame needs the
-    // whole image) and brings S back
-    // (bsub_step_prox_frames), and so does every graph mode once the handle has a frame-range description (bsub_step_prox_block)
-    const bool split = s->shrink_mode == SHRINK_SPILL && (s->cfg.prox == BSUB_PROX_BLOCK_L2 || s->cfg.prox == BSUB_PROX_GRAPH_LINF || s->fr_set);
+    // whole image), runs bsub_step_prox_block and brings S back; so does every graph mode with a frame-range description
+    const bool split = s->shrink_mode == SHRINK_SPILL &&
+                       (s->cfg.prox == BSUB_PROX_BLOCK_L2 || s->cfg.prox == BSUB_PROX_GRAPH_LINF || frame_range_only(s));
     if (part == 2 && !split) return 0;
-    if (part == 0 && s->fr_set && !s->graph_set) {
+    if (part == 0 && frame_range_only(s)) {
         set_error("bsub_step_shrink: the handle holds only a frame-range description; use _shrink_a, bsub_step_prox_block, _shrink_b");
         return -1;
     }
@@ -780,30 +832,15 @@ static int step_shrink_impl(bsub_solver* s, void* stream, int part) {
         // two-phase: U = G_S -> prox -> S_new (written over S) -> dual update
         if (s->cfg.prox == BSUB_PROX_FLAT_LINF) {
             RET_IF(launch_prox_groups_csr(s->U, s->S, s->ld, s->m, s->n, s->gptr, s->gidx, s->ngroups, 0.f, s->st, st));
-        } else if (s->cfg.prox == BSUB_PROX_GRAPH_LINF) {
-            if (part == 1) return 0;                       // the driver runs the prox on frame shards, then calls part 2
-            RET_IF(launch_prox_graph3(s->U, s->S, s->xi, s->xi_floats, s->tot, s->eta_dev, s->ld, s->cfg.rows, s->cfg.cols, s->n, 0.f,
-                                      s->cfg.graph_max_sweeps, (float)s->cfg.graph_tol, s->sweeps_dev, s->st, st));
-        } else if (part == 1 && s->fr_set) {
-            return 0;                                      // the driver runs the prox on frame shards (bsub_step_prox_block)
-        } else if (s->cfg.prox == BSUB_PROX_GRAPH_CENTER_BG) {
-            // S = prox_by_frame(G_S) then the background pixels of every frame are overwritten by their l2 shrink of G_S
-            RET_IF(launch_prox_graph3(s->U, s->S, s->xi, s->xi_floats, s->tot, s->eta_dev, s->ld, s->cfg.rows, s->cfg.cols, s->n, 0.f,
-                                      s->cfg.graph_max_sweeps, (float)s->cfg.graph_tol, s->sweeps_dev, s->st, st, 1, s->m));
-            RET_IF(launch_block_l2_sums(s->U, s->labels_dev, s->ld, s->m, s->n, 1, s->bsums, s->st, st));
-            RET_IF(launch_block_l2_apply(s->U, s->S, s->labels_dev, s->ld, s->m, s->n, 1, s->bsums, nullptr, s->st, 0.0, 0.0, st, 1));
-        } else if (s->cfg.prox == BSUB_PROX_GRAPH_GENERIC) {
-            RET_IF(launch_prox_graph_generic(s->U, s->S, s->ld, s->m, s->n, s->pg_dev, s->pg_layout, s->xi, s->tot, 0.f, s->cfg.graph_max_sweeps,
-                                             (float)s->cfg.graph_tol, s->sweeps_dev, s->st, st));
-            if (s->pg_bg) {
-                RET_IF(launch_block_l2_sums(s->U, s->labels_dev, s->ld, s->m, s->n, 1, s->bsums, s->st, st));
-                RET_IF(launch_block_l2_apply(s->U, s->S, s->labels_dev, s->ld, s->m, s->n, 1, s->bsums, nullptr, s->st, 0.0, 0.0, st, 1));
-            }
-        } else {   // BSUB_PROX_BLOCK_L2
+        } else if (s->cfg.prox == BSUB_PROX_BLOCK_L2) {
             RET_IF(launch_block_l2_sums(s->U, s->labels_dev, s->ld, s->m, s->n, s->nlab, s->bsums, s->st, st));
             if (part == 1) return 0;                       // the driver all-reduces bsums, then calls part 2
             RET_IF(launch_block_l2_apply(s->U, s->S, s->labels_dev, s->ld, s->m, s->n, s->nlab, s->bsums, s->lam_table, s->st, 0.0,
                                          0.0, st));
+        } else {   // graph modes
+            if (part == 1 && split) return 0;              // the driver runs the prox on frame shards, then calls part 2
+            RET_IF(graph_prox(s->graph, s->U, s->S, s->ld, 0, s->n, s->st, 0.f, s->cfg.graph_max_sweeps, (float)s->cfg.graph_tol,
+                              s->sweeps_dev, &s->work, st));
         }
         nparts = s->num_sms * 8;
         RET_IF(launch_dual_update(s->D, s->S, s->S, s->Y, s->T, s->eb.VC, s->eb.vstride, s->st, s->L, s->ld, s->n, s->part_zz,
@@ -827,60 +864,19 @@ int bsub_step_prox_buffers(bsub_solver* s, float** G_S, float** S, int64_t* ld) 
     return 0;
 }
 
-int bsub_step_prox_frames(bsub_solver* s, const float* Uf, float* Vf, int64_t ldf, int32_t rows, int32_t cols, int32_t nf, void* stream) {
-    if (!s || !s->initialised) { set_error("bsub_step_prox_frames: solver not initialised"); return -1; }
-    if (s->cfg.prox != BSUB_PROX_GRAPH_LINF) { set_error("bsub_step_prox_frames: solver was not created with BSUB_PROX_GRAPH_LINF"); return -1; }
-    if (nf <= 0) return 0;
-    if (!Uf || !Vf || (long long)rows * cols > ldf) { set_error("bsub_step_prox_frames: bad argument"); return -1; }
-    cudaStream_t st = use_stream(s, stream);
-    long long xf = 0, tf = 0;
-    prox_graph3_workspace(rows, cols, nf, ldf, 0, &xf, &tf);
-    RET_IF(grow_floats(&s->xi2, &s->xi2_floats, xf));
-    RET_IF(grow_floats(&s->tot2, &s->tot2_floats, tf));
-    if (!s->sweeps2) { CK(cudaMalloc((void**)&s->sweeps2, sizeof(int) * 8)); CK(cudaMemset(s->sweeps2, 0, sizeof(int) * 8)); }
-    // lambda / mu and the stop flag come from the device state, exactly as in the unsharded pass
-    return launch_prox_graph3(Uf, Vf, s->xi2, xf, s->tot2, nullptr, ldf, rows, cols, nf, 0.f, s->cfg.graph_max_sweeps, (float)s->cfg.graph_tol,
-                              s->sweeps2, s->st, st);
-}
-
 int bsub_step_prox_block(bsub_solver* s, const float* Uf, float* Vf, int64_t ldf, int32_t f0, int32_t nf, void* stream) {
     if (!s || !s->initialised) { set_error("bsub_step_prox_block: solver not initialised"); return -1; }
-    if (!s->fr_set) { set_error("bsub_step_prox_block: the handle has no frame-range description (bsub_set_frame_*)"); return -1; }
-    if (nf < 0 || f0 < s->fr_f0 || (long long)f0 + nf > (long long)s->fr_f0 + s->fr_nf) {
-        set_error("bsub_step_prox_block: frames [%d, %lld) are outside the described range [%d, %d)", f0, (long long)f0 + nf, s->fr_f0,
-                  s->fr_f0 + s->fr_nf);
+    if (!frame_range_only(s)) { set_error("bsub_step_prox_block: the handle has no frame-range description (bsub_set_frame_*)"); return -1; }
+    const GraphDesc& d = s->graph;
+    if (nf < 0 || f0 < d.f0 || (long long)f0 + nf > (long long)d.f0 + d.nf) {
+        set_error("bsub_step_prox_block: frames [%d, %lld) are outside the described range [%d, %d)", f0, (long long)f0 + nf, d.f0, d.f0 + d.nf);
         return -1;
     }
     if (nf == 0) return 0;
-    const int rows = s->fr_rows, cols = s->fr_cols, lf = f0 - s->fr_f0;
-    const long long m = (long long)rows * cols;
-    if (!Uf || !Vf || ldf < m) { set_error("bsub_step_prox_block: bad argument"); return -1; }
-    cudaStream_t st = use_stream(s, stream);
+    if (!Uf || !Vf || ldf < d.m) { set_error("bsub_step_prox_block: bad argument"); return -1; }
     // lambda / mu and the stop flag come from the device state, exactly as in the unsharded pass
-    if (s->cfg.prox == BSUB_PROX_GRAPH_GENERIC) {
-        const GenericGraphLayout L = prox_graph_generic_layout(m, ldf, nf, s->fr_max_nnz);
-        RET_IF(grow_floats(&s->xi2, &s->xi2_floats, L.xi_floats));
-        RET_IF(grow_floats(&s->tot2, &s->tot2_floats, L.tot_floats));
-        GenericGraphDev g = s->fr_graph;
-        g.frame_graph += lf;
-        RET_IF(launch_prox_graph_generic(Uf, Vf, ldf, m, nf, g, L, s->xi2, s->tot2, 0.f, s->cfg.graph_max_sweeps, (float)s->cfg.graph_tol,
-                                         s->sweeps_dev, s->st, st));
-    } else {
-        const int center = s->cfg.prox == BSUB_PROX_GRAPH_CENTER_BG ? 1 : 0;
-        long long xf = 0, tf = 0;
-        prox_graph3_workspace(rows, cols, nf, ldf, center, &xf, &tf);
-        RET_IF(grow_floats(&s->xi2, &s->xi2_floats, xf));
-        RET_IF(grow_floats(&s->tot2, &s->tot2_floats, tf));
-        const float* eta = s->fr_eta ? s->fr_eta + (size_t)lf * s->fr_eta_stride : nullptr;
-        RET_IF(launch_prox_graph3(Uf, Vf, s->xi2, xf, s->tot2, eta, ldf, rows, cols, nf, 0.f, s->cfg.graph_max_sweeps, (float)s->cfg.graph_tol,
-                                  s->sweeps_dev, s->st, st, center, s->fr_eta_stride));
-    }
-    if (s->fr_labels) {       // background pixels: their frame's l2 shrink of G_S at non_block_lambda / mu, over the graph prox result
-        const unsigned char* lab = s->fr_labels + (size_t)lf * m;
-        RET_IF(launch_block_l2_sums(Uf, lab, ldf, m, nf, 1, s->fr_bsums, s->st, st));
-        RET_IF(launch_block_l2_apply(Uf, Vf, lab, ldf, m, nf, 1, s->fr_bsums, nullptr, s->st, 0.0, 0.0, st, 1));
-    }
-    return 0;
+    return graph_prox(d, Uf, Vf, ldf, f0, nf, s->st, 0.f, s->cfg.graph_max_sweeps, (float)s->cfg.graph_tol, s->sweeps_dev, &s->work,
+                      use_stream(s, stream));
 }
 
 int bsub_block_sums_buffer(bsub_solver* s, double** sums, int64_t* count) {
@@ -928,7 +924,7 @@ int bsub_sync_status(bsub_solver* s, bsub_status* out, void* stream) {
 }
 
 int bsub_run(bsub_solver* s, void* stream) {
-    if (s && s->fr_set && !s->graph_set) {
+    if (s && frame_range_only(s)) {
         set_error("bsub_run: the handle holds only a frame-range description (bsub_set_frame_*), not the graphs of its own pixels");
         return -1;
     }
@@ -1056,8 +1052,8 @@ int bsub_debug_counters(bsub_solver* s, int64_t* out8) {
 
 int bsub_debug_graph(bsub_solver* s, int64_t* out4) {
     if (!s || !out4) { set_error("bsub_debug_graph: null argument"); return -1; }
-    int h[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    if (s->sweeps_dev) CK(cudaMemcpy(h, s->sweeps_dev, sizeof(h), cudaMemcpyDeviceToHost));
+    int h[8];
+    CK(cudaMemcpy(h, s->sweeps_dev, sizeof(h), cudaMemcpyDeviceToHost));
     out4[0] = h[0]; out4[1] = h[4]; out4[2] = h[5]; out4[3] = h[6];
     return 0;
 }
@@ -1170,84 +1166,51 @@ int bsub_prox_flat_groups_dev(const float* U, float* V, int64_t ld, int64_t m, i
     return 0;
 }
 
+// the prox of the operators: all n frames of d at lambda1, the sweep count of the call; synchronises the stream and releases d
+static int prox_once(GraphDesc* d, const float* U, float* V, long long ld, int n, double lambda1, int max_sweeps, double tol,
+                     int32_t* sweeps_used, void* stream) {
+    cudaStream_t st = as_stream(stream);
+    ProxWork w;
+    DevScope mem;
+    int* sw = nullptr;
+    int sw_h = 0;
+    const int rc = [&]() -> int {
+        RET_IF(mem.alloc(&sw, sizeof(int) * 8));
+        CK(cudaMemsetAsync(sw, 0, sizeof(int) * 8, st));
+        RET_IF(graph_prox(*d, U, V, ld, 0, n, nullptr, (float)lambda1, max_sweeps > 0 ? max_sweeps : 4000, (float)tol, sw, &w, st));
+        CK(cudaMemcpyAsync(&sw_h, sw, sizeof(int), cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        return 0;
+    }();
+    w.release();
+    d->release();
+    if (rc == 0 && sweeps_used) *sweeps_used = sw_h;
+    return rc;
+}
+
 int bsub_prox_graph3_dev(const float* U, float* V, int64_t ld, int32_t rows, int32_t cols, int32_t n, double lambda1,
                          const double* eta_host, int32_t max_sweeps, double tol, int32_t* sweeps_used, void* stream) {
-    if (!U || !V || (long long)rows * cols > ld) { set_error("bsub_prox_graph3_dev: bad argument"); return -1; }
-    cudaStream_t st = as_stream(stream);
-    const long long nwi = rows - std::min(3, rows) + 1, nwj = cols - std::min(3, cols) + 1, nw = nwi * nwj;
-    DevScope mem;
-    float *xi = nullptr, *tot = nullptr, *eta = nullptr; int* sw = nullptr;
-    long long xi_floats = 0, tot_floats = 0;
-    prox_graph3_workspace(rows, cols, n, ld, 0, &xi_floats, &tot_floats);
-    RET_IF(mem.alloc(&xi, sizeof(float) * (size_t)xi_floats));
-    RET_IF(mem.alloc(&tot, sizeof(float) * (size_t)tot_floats));
-    RET_IF(mem.alloc(&sw, sizeof(int) * 8));
-    CK(cudaMemset(sw, 0, sizeof(int) * 8));
-    if (eta_host) {
-        std::vector<float> ef((size_t)nw);
-        for (long long i = 0; i < nw; ++i) ef[i] = (float)eta_host[i];
-        RET_IF(mem.alloc(&eta, sizeof(float) * nw));
-        CK(cudaMemcpy(eta, ef.data(), sizeof(float) * nw, cudaMemcpyHostToDevice));
-    }
-    RET_IF(launch_prox_graph3(U, V, xi, xi_floats, tot, eta, ld, rows, cols, n, (float)lambda1, max_sweeps > 0 ? max_sweeps : 4000, (float)tol, sw,
-                              nullptr, st));
-    int sw_h = 0;
-    CK(cudaMemcpyAsync(&sw_h, sw, sizeof(int), cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    if (sweeps_used) *sweeps_used = sw_h;
-    return 0;
+    GraphDesc d;
+    RET_IF(describe_windows(&d, rows, cols, 0, n, eta_host, window_count(rows, cols), "bsub_prox_graph3_dev",
+                            U && V && (long long)rows * cols <= ld));
+    return prox_once(&d, U, V, ld, n, lambda1, max_sweeps, tol, sweeps_used, stream);
 }
 
 int bsub_prox_center3_dev(const float* U, float* V, int64_t ld, int32_t rows, int32_t cols, int32_t n, double lambda1,
                           const float* eta_host, int32_t max_sweeps, double tol, int32_t* sweeps_used, void* stream) {
-    if (!U || !V || !eta_host || (long long)rows * cols > ld) { set_error("bsub_prox_center3_dev: bad argument"); return -1; }
-    cudaStream_t st = as_stream(stream);
-    const long long m = (long long)rows * cols;
-    DevScope mem;
-    float *xi = nullptr, *tot = nullptr, *eta = nullptr; int* sw = nullptr;
-    long long xi_floats = 0, tot_floats = 0;                                      // one candidate window per pixel and frame
-    prox_graph3_workspace(rows, cols, n, ld, 1, &xi_floats, &tot_floats);
-    RET_IF(mem.alloc(&xi, sizeof(float) * (size_t)xi_floats));
-    RET_IF(mem.alloc(&tot, sizeof(float) * (size_t)tot_floats));
-    RET_IF(mem.alloc(&eta, sizeof(float) * (size_t)n * m));
-    RET_IF(mem.alloc(&sw, sizeof(int) * 8));
-    CK(cudaMemset(sw, 0, sizeof(int) * 8));
-    CK(cudaMemcpy(eta, eta_host, sizeof(float) * (size_t)n * m, cudaMemcpyHostToDevice));
-    RET_IF(launch_prox_graph3(U, V, xi, xi_floats, tot, eta, ld, rows, cols, n, (float)lambda1, max_sweeps > 0 ? max_sweeps : 4000, (float)tol, sw,
-                              nullptr, st, 1, m));
-    int sw_h = 0;
-    CK(cudaMemcpyAsync(&sw_h, sw, sizeof(int), cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    if (sweeps_used) *sweeps_used = sw_h;
-    return 0;
+    if (!eta_host) { set_error("bsub_prox_center3_dev: bad argument"); return -1; }
+    GraphDesc d;
+    RET_IF(describe_centre(&d, rows, cols, 0, n, eta_host, nullptr, "bsub_prox_center3_dev", U && V && (long long)rows * cols <= ld));
+    return prox_once(&d, U, V, ld, n, lambda1, max_sweeps, tol, sweeps_used, stream);
 }
 
 int bsub_prox_graph_dev(const float* U, float* V, int64_t ld, int64_t m, int32_t n, double lambda1, int32_t n_graphs, const int32_t* frame_graph,
                         const int64_t* n_groups, const int32_t* const* indptr, const int32_t* const* indices, const double* const* eta,
                         int32_t max_sweeps, double tol, int32_t* sweeps_used, void* stream) {
-    GenericGraphHost H;                                   // validation first: bad input never reaches the device
-    RET_IF(pack_generic_graphs(m, n, n_graphs, frame_graph, n_groups, indptr, indices, eta, &H, "bsub_prox_graph_dev"));
-    if (!U || !V || ld < m) { set_error("bsub_prox_graph_dev: bad argument"); return -1; }
-    cudaStream_t st = as_stream(stream);
-    DevScope mem;
-    int* ints = nullptr; float* eta_d = nullptr;
-    GenericGraphDev gd;
-    const int rc = upload_generic_graphs(H, &ints, &eta_d, &gd);
-    mem.ptrs.push_back(ints); mem.ptrs.push_back(eta_d);
-    if (rc != 0) return rc;
-    const GenericGraphLayout L = prox_graph_generic_layout(m, ld, n, H.max_nnz);
-    float *xi = nullptr, *tot = nullptr; int* sw = nullptr;
-    RET_IF(mem.alloc(&xi, sizeof(float) * (size_t)L.xi_floats));
-    if (L.tot_floats > 0) RET_IF(mem.alloc(&tot, sizeof(float) * (size_t)L.tot_floats));
-    RET_IF(mem.alloc(&sw, sizeof(int) * 8));
-    CK(cudaMemsetAsync(sw, 0, sizeof(int) * 8, st));
-    RET_IF(launch_prox_graph_generic(U, V, ld, m, n, gd, L, xi, tot, (float)lambda1, max_sweeps > 0 ? max_sweeps : 4000, (float)tol, sw,
-                                     nullptr, st));
-    int sw_h = 0;
-    CK(cudaMemcpyAsync(&sw_h, sw, sizeof(int), cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    if (sweeps_used) *sweeps_used = sw_h;
-    return 0;
+    GraphDesc d;
+    RET_IF(describe_graphs(&d, 0, 0, m, 0, n, n_graphs, frame_graph, n_groups, indptr, indices, eta, nullptr, "bsub_prox_graph_dev",
+                           U && V && ld >= m));
+    return prox_once(&d, U, V, ld, n, lambda1, max_sweeps, tol, sweeps_used, stream);
 }
 
 int bsub_block_shrink_dev(const float* G, float* R, int64_t ld, int64_t m, int32_t n, const uint8_t* labels, const int32_t* lam_ptr,

@@ -114,13 +114,16 @@ class CudaStepSolver:
             if graph_cols is None:
                 raise Exception("CudaStepSolver: graphs needs graph_cols, the number of columns of the whole frame")
             route = api.route_graphs(graphs, rows * graph_cols, n, (rows, graph_cols), background_masks=background_masks)
-        if route is not None:
-            graph_cols = route.cols
         self.frame_range = None
         if route is not None:
+            graph_cols = route.cols
             self.frame_range = (0, n) if frames is None else (int(frames[0]), int(frames[1]))
         elif frames is not None:
             raise Exception("CudaStepSolver: frames applies to the graph modes given by graphs or weight_mask")
+        elif graph_cols is not None and not l1:
+            if blocks is not None:
+                raise Exception("CudaStepSolver: blocks and graph_cols are mutually exclusive")
+            route = api.GraphRoute(C.PROX_GRAPH_LINF, rows, graph_cols)      # unit weights: frame_range stays None
         if delta is None:
             delta = 1.0 if l1 else 10
         self.rows, self.cols_local, self.graph_cols = rows, cols_local, graph_cols
@@ -134,21 +137,13 @@ class CudaStepSolver:
                                   max_iter=max_iter)
             self.lazy_S = False
             self.dec = api.Decomposition(cfg)
-            self.dec.set_frame_route(route, *self.frame_range)
+            self.dec.set_frame_route(route, *(self.frame_range or (0, n)))
         elif l1:
             cfg = api.make_config(self.m, n, C.PROX_L1, 0, 0, delta=delta, mu_scale=1.25, rho=1.2, use_sv_prediction=False,
                                   m_global=m_global, d_global=min(m_global, n), max_iter=max_iter, tile_rows=tile_rows,
                                   cluster_frames=cluster_frames, flags=0 if store_S_lazily else C.FLAG_ALWAYS_STORE_S)
             self.lazy_S = bool(store_S_lazily)
             self.dec = api.Decomposition(cfg)
-        elif graph_cols is not None:
-            if blocks is not None:
-                raise Exception("CudaStepSolver: blocks and graph_cols are mutually exclusive")
-            cfg = api.make_config(self.m, n, C.PROX_GRAPH_LINF, rows, cols_local, delta=delta, m_global=m_global,
-                                  d_global=min(m_global, n), max_iter=max_iter)
-            self.lazy_S = False
-            self.dec = api.Decomposition(cfg)
-            self.dec.set_graph_windows(None)
         elif blocks is None:
             cfg = api.make_config(self.m, n, C.PROX_FLAT_LINF, rows, cols_local, delta=delta, m_global=m_global,
                                   d_global=min(m_global, n), max_iter=max_iter, tile_rows=tile_rows,
@@ -226,11 +221,8 @@ class CudaStepSolver:
 
     def prox_frames(self, Uf, Vf, rows, cols, nf):
         """Prox of this rank's nf whole frames (rows of Uf / Vf, row stride Uf.stride(0)) at this handle's lambda / mu."""
-        if self.frame_range is not None:
-            self.prox_block(Uf, Vf, self.frame_range[0], nf)
-        elif nf > 0:
-            C.check(self.lib.bsub_step_prox_frames(self.h, ctypes.c_void_p(Uf.data_ptr()), ctypes.c_void_p(Vf.data_ptr()),
-                                                   int(Uf.stride(0)), rows, cols, nf, self._s()))
+        # the unit-weight window description (frame_range None) holds no per-frame data: frames [0, nf) of it prox any nf frames
+        self.prox_block(Uf, Vf, self.frame_range[0] if self.frame_range is not None else 0, nf)
 
     def prox_block(self, Uf, Vf, f0, nf):
         """Prox of the whole frames [f0, f0 + nf) of the clip, held in the rows of Uf / Vf: any block of this solver's frame range."""

@@ -105,13 +105,14 @@ int bsub_destroy(bsub_solver* s);
  * flat: int32[m] 1-based ids from get_proximal_flat_groups_nonoverlap (lsd_improvement.py:14-34); a regular 3x3
  *       tiling of the rows x cols image is recognised and fused, anything else takes the generic two-phase path. */
 int bsub_set_flat_groups(bsub_solver* s, const int32_t* groups_host);
-/* graph: overlapping windows of getGraphSPAMS_all_groups (inexact_alm_lsd.py:13-46); eta_host may be NULL (all 1) */
+/* graph: overlapping windows of getGraphSPAMS_all_groups (inexact_alm_lsd.py:13-46); eta_host double[n_eta] one weight per window
+ * (finite, >= 0), or NULL (all 1) */
 int bsub_set_graph_windows(bsub_solver* s, const double* eta_host, int64_t n_eta);
 /* blocks: blocks_by_frame / lambdas_by_frame of group_sparse_RPCA.py:45 as a label map uint8[n][m] (0 = complement,
  *       b = block b of that frame) plus the CSR (lam_ptr[n+1], lam) of the per-frame lambda lists. */
 int bsub_set_blocks(bsub_solver* s, const uint8_t* labels_host, const int32_t* lam_ptr, const double* lam);
 /* per-frame centre windows + background (BSUB_PROX_GRAPH_CENTER_BG): eta_host float32[n][m] = weight of the 3x3 window
- * centred on that pixel in that frame (<= 0: no window; get_proximal_graph_group_centers, lsd_improvement.py:74-120),
+ * centred on that pixel in that frame (finite; <= 0: no window; get_proximal_graph_group_centers, lsd_improvement.py:74-120),
  * background_host uint8[n][m] != 0 where the pixel belongs to the frame's background mask (lsd_improvement.py:434). */
 int bsub_set_center_windows(bsub_solver* s, const float* eta_host, const uint8_t* background_host);
 /* any graphs (BSUB_PROX_GRAPH_GENERIC): n_graphs SPAMS-style CSC groups_var matrices as the reference builds them -- graph k has
@@ -156,21 +157,18 @@ int bsub_step_shrink_b(bsub_solver* s, void* stream);
 int bsub_block_sums_buffer(bsub_solver* s, double** sums, int64_t* count);
 /* Graph modes on pixel shards: the prox of a frame needs the whole image but no other frame, so between the two halves of the pass
  * the driver re-shards G_S by FRAMES (all-to-all), runs the prox of its frames and brings S back:
- *   _shrink_a (G_S of this pixel shard into the buffer _prox_buffers returns) -> exchange -> prox of nf whole frames of rows x cols
- *   pixels (device pointers, lambda/mu and the stop flag from this handle's device state) -> exchange (result into the S pointer of
+ *   _shrink_a (G_S of this pixel shard into the buffer _prox_buffers returns) -> exchange -> bsub_step_prox_block on whole frames
+ *   (device pointers, lambda/mu and the stop flag from this handle's device state) -> exchange (result into the S pointer of
  *   _prox_buffers) -> _shrink_b.
- * bsub_step_prox_frames: all-window graphs with unit weights, on a handle set up with bsub_set_graph_windows (whose _shrink_a always
- * stops before the prox).
- * bsub_step_prox_block: every graph mode, on a handle that holds a frame-range description (bsub_set_frame_*, below); once it has
- * one, _shrink_a stops before the prox and _shrink_b finishes the pass in BSUB_PROX_GRAPH_CENTER_BG / _GENERIC too.  The l1 mode
- * (BSUB_PROX_L1) is elementwise and shards with bsub_step_shrink alone. */
+ * The handle holds a frame-range description (bsub_set_frame_*, below).  _shrink_a then stops before the prox in every graph mode, as
+ * it always does in BSUB_PROX_GRAPH_LINF, and _shrink_b finishes the pass.  The l1 mode (BSUB_PROX_L1) is elementwise and shards
+ * with bsub_step_shrink alone. */
 int bsub_step_prox_buffers(bsub_solver* s, float** G_S, float** S, int64_t* ld);
-int bsub_step_prox_frames(bsub_solver* s, const float* U_frames, float* V_frames, int64_t ld_frames, int32_t rows, int32_t cols,
-                          int32_t n_frames, void* stream);
 /* Frame-range descriptions: the prox of whole rows x cols frames [f0, f0 + nf) of the clip (the frames this rank owns after the
- * exchange; nf may be 0).  Only those frames' data is copied, every entry is validated before anything reaches the device, and a new
- * description replaces the previous one.  A handle that holds only such a description has no graph for its own pixels: bsub_run and
- * bsub_step_shrink refuse it.
+ * exchange; nf may be 0).  Only those frames' data is copied, and every entry is validated before anything reaches the device.  A
+ * handle holds one graph description: each bsub_set_frame_* or whole-clip setter (bsub_set_graph_windows / _center_windows /
+ * _graphs, which describe frames [0, n) of the handle's own pixels) replaces the previous one.  A handle whose description is a
+ * frame range has no graph for its own pixels: bsub_run and bsub_step_shrink refuse it.
  *   _windows (BSUB_PROX_GRAPH_LINF): the 3x3 all-window graph, eta double[n_eta] one weight per window as bsub_set_graph_windows
  *     takes it (finite, >= 0), the same in every frame; NULL: unit weights.
  *   _center_windows (BSUB_PROX_GRAPH_CENTER_BG): eta float32[nf][rows*cols] and background uint8[nf][rows*cols] as
@@ -209,7 +207,8 @@ int bsub_debug_info(bsub_solver* s, int32_t* out16);   /* ..., [12] plane projec
  * [4] Gram mode of the next iteration (0 fp64 DMMA, 1 int8 tcgen05), [5] last digit pass saturated, [6] the solve has switched
  * to the fp64 Gram for accuracy, [7] 1e6 * bound of the int8 Gram's truncation error relative to (1/mu)^2 */
 int bsub_debug_counters(bsub_solver* s, int64_t* out8);
-/* overlapping-window / generic graph prox of this handle: out4 = {outer iterations of the last call, their total over all calls, calls, calls that hit graph_max_sweeps} */
+/* graph prox of this handle (SPILL pass or bsub_step_prox_block): out4 = {outer iterations of the last call, their total over all calls,
+ * calls, calls that hit graph_max_sweeps} */
 int bsub_debug_graph(bsub_solver* s, int64_t* out4);
 /* foreground_mask(D, L, S, sigmas) of utils.py:139-149 on the solver's own D, L, S; mask uint8[n][m] on the host */
 int bsub_mask_stats_local(bsub_solver* s, int phase /*0: max|S|, 1: count/sum/sumsq*/, void* stream);
@@ -225,12 +224,13 @@ int bsub_prox_flat3_dev(const float* U, float* V, int64_t ld, int32_t rows, int3
 /* prox_flat for an arbitrary groups vector (host int32[m]) */
 int bsub_prox_flat_groups_dev(const float* U, float* V, int64_t ld, int64_t m, int32_t n, const int32_t* groups_host,
                               double lambda1, void* stream);
-/* prox(G_S, lambda1, graph) on the overlapping 3x3 windows   inexact_alm_lsd.py:49-57 */
+/* prox(G_S, lambda1, graph) on the overlapping 3x3 windows   inexact_alm_lsd.py:49-57; eta_host as for bsub_set_graph_windows.
+ * The three graph operators validate their graphs and eta before anything else, as the setters do, and synchronise the stream. */
 int bsub_prox_graph3_dev(const float* U, float* V, int64_t ld, int32_t rows, int32_t cols, int32_t n, double lambda1,
                          const double* eta_host, int32_t max_sweeps, double tol, int32_t* sweeps_used, void* stream);
 /* prox_by_frame(G_S, lambda1, graphs) with the per-frame centre-window graphs of get_proximal_graph_group_centers
  * (inexact_alm_lsd.py:60-68, lsd_improvement.py:74-120): eta_host float32[n][rows*cols] = weight of the 3x3 window centred on
- * that pixel of that frame (<= 0: no window) */
+ * that pixel of that frame (finite; <= 0: no window) */
 int bsub_prox_center3_dev(const float* U, float* V, int64_t ld, int32_t rows, int32_t cols, int32_t n, double lambda1,
                           const float* eta_host, int32_t max_sweeps, double tol, int32_t* sweeps_used, void* stream);
 /* prox / prox_by_frame (inexact_alm_lsd.py:49-68) for any non-nested graphs, all frames in one launch: graphs and frame_graph as for

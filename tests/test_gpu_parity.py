@@ -262,7 +262,8 @@ def test_group_sparse_through_sharded_driver(B, highway_fixture, summary):
 
 def test_graph_mode_through_sharded_driver(B, watersurface_u8):
     """The overlapping-window LSD through dist.ShardedLSD (world size 1: the split shrink pass, bsub_step_prox_buffers /
-    bsub_step_prox_frames -- the pieces the multi-GPU driver puts an all-to-all between): same result as bsub_run."""
+    bsub_step_prox_block on a unit-weight frame-range description -- the pieces the multi-GPU driver puts an all-to-all between):
+    same result as bsub_run."""
     import torch
     from background_subtraction_b200 import dist as bdist
     from oracle import alm_oracle as O

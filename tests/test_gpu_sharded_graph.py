@@ -91,6 +91,8 @@ def _whole_clip(B, D, mode):
     if mode == "windows_eta":
         g = _window_graph(B)
         return B.lsd_decomposition(D, graphs=g), dict(graphs=g, graph_cols=W)
+    if mode == "windows":                                        # the reference's default LSD(): unit weights, graph_cols alone
+        return B.lsd_decomposition(D, graphs=B.getGraphSPAMS_all_groups((H, W), (3, 3))), dict(graph_cols=W)
     cfg = B.make_config(H * W, T, C.PROX_L1, 0, 0, delta=1.0, mu_scale=1.25, rho=1.2, use_sv_prediction=False)   # inexact_alm_rpca
     dec = B.Decomposition(cfg)
     dec.load(D)
@@ -110,7 +112,8 @@ def _sharded(D, kw, cls=None):
     return s
 
 
-@pytest.mark.parametrize("mode,prox", [("generic", 5), ("generic_bg", 5), ("centre_bg", 4), ("windows_eta", 1), ("l1", 3)])
+@pytest.mark.parametrize("mode,prox", [("generic", 5), ("generic_bg", 5), ("centre_bg", 4), ("windows_eta", 1), ("windows", 1),
+                                       ("l1", 3)])
 def test_mode_through_sharded_driver_matches_bsub_run(B, D, mode, prox):
     dec, kw = _whole_clip(B, D, mode)
     assert dec.cfg.prox == prox

@@ -120,6 +120,27 @@ def test_graph_lsd_golden(B, golden_cases, watersurface_u8):
     assert rel_fro(L, golden_cases["graph_a_L"]) <= TOL_F and rel_fro(S, golden_cases["graph_a_S"]) <= TOL_F
 
 
+def test_redescribed_graph_windows_replace_the_weights(B, watersurface_u8):
+    """A whole-clip window handle given per-window weights and then re-described with unit weights (NULL) solves as a fresh
+    unit-weight handle does: each description replaces the previous one."""
+    from background_subtraction_b200 import _cabi as C
+    from oracle import alm_oracle as O
+    h, w, t = 48, 60, 12
+    D, _x, _mean = O.normalize_and_center(watersurface_u8[:h, :w, :t])
+
+    def solve(*etas):
+        dec = B.Decomposition(B.make_config(h * w, t, C.PROX_GRAPH_LINF, h, w))
+        for eta in etas:
+            dec.set_graph_windows(eta)
+        dec.load(D)
+        dec.run()
+        return dec.status(), [l['svp'] for l in dec.log()], dec.download('S')
+    st0, svp0, S0 = solve(None)
+    st1, svp1, S1 = solve(np.random.default_rng(7).uniform(0.2, 3.0, (h - 2) * (w - 2)), None)
+    assert st1.iter == st0.iter and svp1 == svp0
+    assert rel_fro(S1, S0) <= 1e-6
+
+
 def test_with_background_golden(B, watersurface_u8):
     """inexact_alm_lsd_with_background (SURVEY 8f row 1) against what the reference's own loop produced: per-frame
     centre-window graphs (built here and handed over as SPAMS dicts) + background l2 shrink."""

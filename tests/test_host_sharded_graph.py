@@ -1,7 +1,8 @@
 """-m "not gpu": host side of the sharded graph modes -- the frame-range entry points resolve, their host code adds no device code
 (they launch the existing prox kernels, so no kernel's registers or spills can change), the kernel choice the public solvers and
-dist.CudaStepSolver share (api.route_graphs / route_weight_mask), and the argument checks CudaStepSolver makes before any device
-work."""
+dist.CudaStepSolver share (api.route_graphs / route_weight_mask), and the argument checks CudaStepSolver and the window operators
+make before any device work."""
+import ctypes
 import os
 import re
 import subprocess
@@ -67,3 +68,33 @@ def test_route_picks_the_kernels_of_the_public_solvers():
 def test_step_solver_checks_its_arguments(kw, msg):
     with pytest.raises(Exception, match=msg):
         dist.CudaStepSolver(3, 3, 4, 18, **kw)
+
+
+def test_step_prox_frames_is_gone():
+    """bsub_step_prox_block serves every graph mode on frame shards, unit-weight windows included: the older entry point is gone."""
+    lib = C.load()
+    hdr = open(os.path.join(ROOT, "include", "bsub_b200.h")).read()
+    assert not hasattr(lib, "bsub_step_prox_frames")
+    assert "bsub_step_prox_frames" not in C.SIGNATURES and "bsub_step_prox_frames" not in hdr
+
+
+@pytest.mark.parametrize("fn,eta,msg", [
+    ("bsub_prox_graph3_dev", [1.0, float("nan")], r"bsub_prox_graph3_dev: eta\[1\] = nan is not finite and >= 0"),
+    ("bsub_prox_graph3_dev", [-0.5, 1.0], r"eta\[0\] = -0.5 is not finite and >= 0"),
+    ("bsub_prox_graph3_dev", [1.0, 2.0], "bsub_prox_graph3_dev: bad argument"),
+    ("bsub_prox_center3_dev", [0.5, float("nan")], r"bsub_prox_center3_dev: eta\[1\] = nan is not finite"),
+    ("bsub_prox_center3_dev", [-1.0, 2.0], "bsub_prox_center3_dev: bad argument"),
+])
+def test_window_operators_check_eta_first(fn, eta, msg):
+    """NULL matrices: the weights are checked first, so bad ones are reported and good ones fail only on the NULL pointers --
+    nothing reaches the device either way.  A 3 x 4 image has two 3 x 3 windows; the centre map of one 1 x 2 frame, two entries."""
+    lib = C.load()
+    sw = ctypes.c_int32(0)
+    if fn == "bsub_prox_graph3_dev":
+        e = np.asarray(eta, dtype=np.float64)
+        rc = lib.bsub_prox_graph3_dev(None, None, 12, 3, 4, 1, 0.1, e.ctypes.data_as(C.c_double_p), 10, 1e-6, ctypes.byref(sw), None)
+    else:
+        e = np.asarray(eta, dtype=np.float32)
+        rc = lib.bsub_prox_center3_dev(None, None, 2, 1, 2, 1, 0.1, e.ctypes.data_as(C.c_float_p), 10, 1e-6, ctypes.byref(sw), None)
+    assert rc != 0
+    assert re.search(msg, lib.bsub_last_error().decode())
