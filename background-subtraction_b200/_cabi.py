@@ -72,6 +72,8 @@ SIGNATURES = {
     "bsub_step_prox_buffers": (ctypes.c_int, [vp, ctypes.POINTER(vp), ctypes.POINTER(vp), c_int64_p]),
     "bsub_set_frame_windows": (ctypes.c_int, [vp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, c_double_p, ctypes.c_int64]),
     "bsub_set_frame_center_windows": (ctypes.c_int, [vp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, c_float_p, c_uint8_p]),
+    "bsub_set_frame_weight_map_dev": (ctypes.c_int, [vp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, vp, ctypes.c_int64,
+                                                     vp]),
     "bsub_set_frame_graphs": (ctypes.c_int, [vp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, c_int32_p,
                                              c_int64_p, ctypes.POINTER(c_int32_p), ctypes.POINTER(c_int32_p), ctypes.POINTER(c_double_p),
                                              c_uint8_p]),

@@ -505,6 +505,17 @@ class Decomposition:
             C.check(self.lib.bsub_set_frame_graphs(self.h, rows, cols, f0, nf, len(csc), fg.ctypes.data_as(C.c_int32_p),
                                                    ng.ctypes.data_as(C.c_int64_p), ip, ix, et, bgp))
 
+    def set_frame_weight_map(self, weight, rows, cols, f0):
+        """Device variant of set_frame_route for LSD_improved's weight map: weight = CUDA tensor float32 [nf][rows * cols] (row pitch
+        weight.stride(0)) of frames [f0, f0 + nf); > 0 centre-window weight, < 0 background (bsub_set_frame_weight_map_dev)."""
+        import torch
+        if not (_is_torch(weight) and weight.is_cuda and weight.dtype == torch.float32 and weight.dim() == 2 and
+                weight.shape[1] == rows * cols and (weight.shape[0] == 0 or weight.stride(1) == 1)):
+            raise Exception("weight map must be a CUDA float32 tensor [frames][%d] with unit pixel stride" % (rows * cols))
+        nf = int(weight.shape[0])
+        C.check(self.lib.bsub_set_frame_weight_map_dev(self.h, rows, cols, f0, nf, ctypes.c_void_p(weight.data_ptr()) if nf else None,
+                                                       int(weight.stride(0)) if nf else rows * cols, self.stream()))
+
     def set_blocks(self, labels, lam_ptr, lam):
         labels = np.ascontiguousarray(labels, dtype=np.uint8)
         lam_ptr = np.ascontiguousarray(lam_ptr, dtype=np.int32)

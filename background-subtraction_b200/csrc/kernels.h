@@ -167,6 +167,10 @@ int launch_mask_stats(const float* D, const float* L, const float* S, long long 
                       const double* absmax, double* stats /*[3]: count, sum, sumsq*/, double* scratch, cudaStream_t s);
 int launch_mask_write(const float* S, long long ld, long long m, int n, const double* stats, double sigmas,
                       unsigned char* mask, long long mask_ld, cudaStream_t s);
+// weight map float [nf][ld] -> eta [nf][m] (positive entries, else 0) and labels [nf][m] (0: negative entry, else 255); the flat
+// index f * m + p of the first non-finite entry is atomicMin'ed into *first_bad (nf >= 1)
+int launch_weight_map_describe(const float* w, long long ld, long long m, int nf, float* eta, unsigned char* labels,
+                               unsigned long long* first_bad, cudaStream_t s);
 
 // ---------------------------------------------------------------- prox.cu (operator-level + generic modes)
 int launch_prox_flat3(const float* U, float* V, long long ld, int rows, int cols, int n, float lam, cudaStream_t s);

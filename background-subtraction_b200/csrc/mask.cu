@@ -144,4 +144,29 @@ int launch_mask_write(const float* S, long long ld, long long m, int n, const do
     return 0;
 }
 
+// LSD_improved's weight map -> centre-window description: eta = the positive entries (0 elsewhere), label 0 where the entry is
+// negative (background) and 255 elsewhere; the flat index f * m + p of the first non-finite entry goes to *first_bad (atomicMin)
+__global__ void weight_map_describe_kernel(const float* __restrict__ w, long long ld, long long m, int nf, float* __restrict__ eta,
+                                           unsigned char* __restrict__ labels, unsigned long long* first_bad) {
+    for (int f = blockIdx.y; f < nf; f += gridDim.y)
+        for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < m; p += (long long)gridDim.x * blockDim.x) {
+            const float v = w[(size_t)f * ld + p];
+            const size_t i = (size_t)f * m + p;
+            if (!isfinite(v)) atomicMin(first_bad, (unsigned long long)i);
+            eta[i] = v > 0.f ? v : 0.f;
+            labels[i] = v < 0.f ? 0 : 255;
+        }
+}
+
+int launch_weight_map_describe(const float* w, long long ld, long long m, int nf, float* eta, unsigned char* labels,
+                               unsigned long long* first_bad, cudaStream_t s) {
+    long long gx = (m + MK_THREADS - 1) / MK_THREADS;
+    if (gx < 1) gx = 1;
+    if (gx > 1024) gx = 1024;
+    dim3 g((unsigned)gx, nf < 512 ? nf : 512);
+    weight_map_describe_kernel<<<g, MK_THREADS, 0, s>>>(w, ld, m, nf, eta, labels, first_bad);
+    BSUB_CUDA_CHECK(cudaGetLastError());
+    return 0;
+}
+
 }  // namespace bsub

@@ -545,6 +545,44 @@ int bsub_set_frame_center_windows(bsub_solver* s, int32_t rows, int32_t cols, in
     return set_graph(s, d, false);
 }
 
+int bsub_set_frame_weight_map_dev(bsub_solver* s, int32_t rows, int32_t cols, int32_t f0, int32_t nf, const float* weight, int64_t ld,
+                                  void* stream) {
+    const char* who = "bsub_set_frame_weight_map_dev";
+    RET_IF(frame_range_check(s, BSUB_PROX_GRAPH_CENTER_BG, "BSUB_PROX_GRAPH_CENTER_BG", rows, cols, f0, nf, who));
+    const long long m = (long long)rows * cols;
+    if (nf > 0 && !weight) { set_error("%s: null argument", who); return -1; }
+    if (nf > 0 && ld < m) { set_error("%s: ld = %lld is less than rows*cols = %lld", who, (long long)ld, m); return -1; }
+    GraphDesc d{BSUB_PROX_GRAPH_CENTER_BG, rows, cols, f0, nf, m};
+    d.eta_stride = m;
+    if (nf > 0) {
+        cudaStream_t st = use_stream(s, stream);
+        DevScope scope;
+        unsigned long long* bad_dev = nullptr;
+        unsigned long long bad = 0;
+        const size_t nm = (size_t)nf * m;
+        // the same buffers describe_upload makes from a host map with a background array: eta, labels and their per-frame sums
+        const int rc = [&]() -> int {
+            RET_IF(scope.alloc(&bad_dev, sizeof(unsigned long long)));
+            CK(cudaMalloc((void**)&d.eta, sizeof(float) * nm));
+            CK(cudaMalloc((void**)&d.labels, nm));
+            CK(cudaMalloc((void**)&d.bsums, sizeof(double) * nf));
+            CK(cudaMemsetAsync(bad_dev, 0xff, sizeof(unsigned long long), st));
+            RET_IF(launch_weight_map_describe(weight, ld, m, nf, d.eta, d.labels, bad_dev, st));
+            CK(cudaMemcpyAsync(&bad, bad_dev, sizeof(bad), cudaMemcpyDeviceToHost, st));
+            CK(cudaStreamSynchronize(st));
+            if (bad == ~0ULL) return 0;
+            const long long f = (long long)(bad / (unsigned long long)m), p = (long long)(bad % (unsigned long long)m);
+            float v = 0.f;
+            CK(cudaMemcpyAsync(&v, weight + (size_t)f * ld + p, sizeof(float), cudaMemcpyDeviceToHost, st));
+            CK(cudaStreamSynchronize(st));
+            set_error("%s: weight[%lld][%lld] (frame %lld, pixel %lld) = %g is not finite", who, f, p, f0 + f, p, (double)v);
+            return -1;
+        }();
+        if (rc != 0) { d.release(); return rc; }       // the handle keeps its previous description
+    }
+    return set_graph(s, d, false);
+}
+
 int bsub_set_frame_graphs(bsub_solver* s, int32_t rows, int32_t cols, int32_t f0, int32_t nf, int32_t n_graphs, const int32_t* frame_graph,
                           const int64_t* n_groups, const int32_t* const* indptr, const int32_t* const* indices, const double* const* eta,
                           const uint8_t* background) {

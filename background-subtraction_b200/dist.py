@@ -42,6 +42,36 @@ def shard_frames(n, world, rank):
     return f0, f0 + base + (1 if rank < extra else 0)
 
 
+def columns_to_frames(comm, src, dst, rows, cols):
+    """all-to-all from the column sharding to the frame sharding: src [n][rows * cols_local] holds this rank's pixel columns
+    (shard_columns) of every frame; rows [0, nf) of dst [>= nf][>= rows * cols] receive the whole frames shard_frames gives this rank."""
+    W = comm.world
+    n = src.shape[0]
+    cr = [shard_columns(cols, W, q) for q in range(W)]
+    fr = [shard_frames(n, W, q) for q in range(W)]
+    nf = fr[comm.rank][1] - fr[comm.rank][0]
+    send = [src[a:b, :].contiguous() for a, b in fr]
+    recv = [src.new_empty((nf, (c1 - c0) * rows)) for c0, c1 in cr]
+    comm.exchange(recv, send)
+    for (c0, c1), t in zip(cr, recv):
+        dst[:nf, c0 * rows:c1 * rows] = t
+
+
+def frames_to_columns(comm, src, dst, rows, cols):
+    """The way back: rows [0, nf) of src hold this rank's whole frames (shard_frames); dst [n][rows * cols_local] receives this rank's
+    pixel columns of every frame."""
+    W = comm.world
+    n = dst.shape[0]
+    cr = [shard_columns(cols, W, q) for q in range(W)]
+    fr = [shard_frames(n, W, q) for q in range(W)]
+    nf = fr[comm.rank][1] - fr[comm.rank][0]
+    send = [src[:nf, c0 * rows:c1 * rows].contiguous() for c0, c1 in cr]
+    recv = [dst.new_empty((b - a, dst.shape[1])) for a, b in fr]
+    comm.exchange(recv, send)
+    for (a, b), t in zip(fr, recv):
+        dst[a:b, :] = t
+
+
 class TorchComm:
     """all-reduce (and the all-to-all of the overlapping-window mode) on torch tensors over torch.distributed (NCCL on GPUs, gloo
     on CPU)."""
@@ -97,7 +127,9 @@ class CudaStepSolver:
         frame (rows x graph_cols pixels), and api.route_graphs / api.route_weight_mask pick the kernel as those solvers do:
           graphs = SPAMS graph dict or per-frame list, with graph_cols: inexact_alm_lsd(graphs=...);
           graphs + background_masks (list of n boolean masks of the whole frame): inexact_alm_lsd_with_background;
-          weight_mask = [h, w, t] map of build_improved_LSD_graphs: center_window_decomposition (LSD_improved's second pass).
+          weight_mask = [h, w, t] map of build_improved_LSD_graphs: center_window_decomposition (LSD_improved's second pass);
+          or, with graph_cols, a CUDA float32 tensor [f1 - f0][rows * graph_cols] holding only the map of `frames`, already on the
+          device (bsub_set_frame_weight_map_dev; what ShardedLSDImproved builds).
         l1=True: inexact_alm_rpca (elementwise soft threshold, /root/reference/lsd_improvement.py:123-196: delta 1.0, mu0 =
         1.25 / ||D||_2, rho 1.2, no sv prediction), which shards without any exchange.  Default: flat 3x3 l_inf groups (LSD)."""
         if sum(x is not None for x in (blocks, graphs, weight_mask)) + bool(l1) > 1:
@@ -105,7 +137,12 @@ class CudaStepSolver:
         if background_masks is not None and graphs is None:
             raise Exception("CudaStepSolver: background_masks needs graphs")
         route = None
-        if weight_mask is not None:
+        frame_map = api._is_torch(weight_mask)
+        if frame_map:
+            if graph_cols is None:
+                raise Exception("CudaStepSolver: a device weight_mask of the rank's frames needs graph_cols")
+            route = api.GraphRoute(C.PROX_GRAPH_CENTER_BG, rows, graph_cols)
+        elif weight_mask is not None:
             gc = int(np.shape(weight_mask)[1])
             if graph_cols is not None and graph_cols != gc:
                 raise Exception("CudaStepSolver: weight_mask has %d columns, graph_cols = %d" % (gc, graph_cols))
@@ -137,7 +174,14 @@ class CudaStepSolver:
                                   max_iter=max_iter)
             self.lazy_S = False
             self.dec = api.Decomposition(cfg)
-            self.dec.set_frame_route(route, *(self.frame_range or (0, n)))
+            if frame_map:
+                f0, f1 = self.frame_range
+                if int(weight_mask.shape[0]) != f1 - f0:
+                    raise Exception("CudaStepSolver: the device weight_mask has %d frames, frames = [%d, %d)"
+                                    % (int(weight_mask.shape[0]), f0, f1))
+                self.dec.set_frame_weight_map(weight_mask, rows, graph_cols, f0)
+            else:
+                self.dec.set_frame_route(route, *(self.frame_range or (0, n)))
         elif l1:
             cfg = api.make_config(self.m, n, C.PROX_L1, 0, 0, delta=delta, mu_scale=1.25, rho=1.2, use_sv_prediction=False,
                                   m_global=m_global, d_global=min(m_global, n), max_iter=max_iter, tile_rows=tile_rows,
@@ -373,25 +417,15 @@ class ShardedLSD:
         if W == 1:
             s.prox_frames(U, S, rows, cols, nf)
             return
-        cr = [shard_columns(cols, W, q) for q in range(W)]
-        fr = [shard_frames(n, W, q) for q in range(W)]
         m_full = rows * cols
         ldf = (m_full + 31) // 32 * 32
         Uf, Vf = s.frames_like(nf, ldf), s.frames_like(nf, ldf)
         # S travels too: once the solve has stopped (the host runs a few iterations ahead of the device-side flag) the prox kernel
         # returns at its first line, and what comes back must then be the S that is already there
-        for src, dst in ((U, Uf), (S, Vf)):
-            send = [src[a:b, :].contiguous() for a, b in fr]
-            recv = [U.new_empty((nf, (c1 - c0) * rows)) for c0, c1 in cr]
-            comm.exchange(recv, send)
-            for (c0, c1), t in zip(cr, recv):
-                dst[:nf, c0 * rows:c1 * rows] = t
+        columns_to_frames(comm, U, Uf, rows, cols)
+        columns_to_frames(comm, S, Vf, rows, cols)
         s.prox_frames(Uf, Vf, rows, cols, nf)
-        send = [Vf[:nf, c0 * rows:c1 * rows].contiguous() for c0, c1 in cr]
-        recv = [U.new_empty((b - a, U.shape[1])) for a, b in fr]
-        comm.exchange(recv, send)
-        for (a, b), t in zip(fr, recv):
-            S[a:b, :] = t
+        frames_to_columns(comm, Vf, S, rows, cols)
 
     def finish(self, sigmas=2.0, want_mask=True):
         s, comm = self.s, self.comm
@@ -403,6 +437,164 @@ class ShardedLSD:
         s.mask_stats(1)
         comm.all_reduce_sum(s.mask_tail_view())
         return s.mask_device(sigmas)
+
+
+class CudaImprovedOps:
+    """What ShardedLSDImproved computes with on this GPU: the step solvers of the two passes, the per-frame morphology and merge,
+    and the results.  The gloo tests substitute NumPy stand-ins (same methods) so that the driver's own code runs on CPU ranks."""
+
+    device = "cuda"
+
+    def matrix(self, D):
+        """D shard, [n][m_local] frame-major (NumPy float64 or torch) -> the float32 device copy both passes load."""
+        import torch
+        if api._is_torch(D):
+            return D.to(device="cuda", dtype=torch.float32).contiguous()
+        # rounded to float32 on the host (round to nearest, as the device conversion of bsub_load_D_f64_host): half the bytes to copy
+        return torch.from_numpy(np.ascontiguousarray(D, dtype=np.float32)).to("cuda")
+
+    def pass1(self, D, rows, cols_local, n, m_global, alg_ver):
+        """improved_LSD_weight_mask's first solve: inexact_alm_lsd on the flat 3x3 groups at delta 1.0 (alg_ver 2) or
+        inexact_alm_rpca at delta 10.0 (alg_ver 1)."""
+        s = CudaStepSolver(rows, cols_local, n, m_global, delta=10.0 if alg_ver == 1 else 1.0, l1=alg_ver == 1)
+        s.load(D)
+        return s
+
+    def pass2(self, D, rows, cols_local, n, m_global, cols, frames, weight):
+        """center_window_decomposition (delta 10) of the frame range `frames` described by weight [nf][rows * cols]."""
+        s = CudaStepSolver(rows, cols_local, n, m_global, graph_cols=cols, weight_mask=weight, frames=frames)
+        s.load(D)
+        return s
+
+    def summary(self, s):
+        """(iterations, converged, rank of L per iteration) of a finished solve."""
+        st = s.status()
+        return int(st.iter), bool(st.converged), [l['svp'] for l in s.dec.log()]
+
+    def close(self, s):
+        s.dec.close()
+
+    def weight_map(self, mask, rows, cols, disk_ratio, weights):
+        """merge_masks((S_mask, apply_morph_ops(S_mask, disk_ratio)), weights) on the frames of mask (uint8 [nf][rows * cols], on the
+        device) -> (float32 [nf][rows * cols] map, -1 = background; number of its positive entries)."""
+        import torch
+        from . import flow
+        nf = int(mask.shape[0])
+        if nf == 0:
+            return torch.empty((0, rows * cols), dtype=torch.float32, device="cuda"), 0
+        morph = flow.morph_frames_dev(mask, rows, cols, flow.disk_radius('disk', disk_ratio * rows))
+        out = torch.where(mask != 0, float(weights[0]), torch.where(morph != 0, float(weights[1]), -1.0)).to(torch.float32)
+        return out, int((out > 0).sum())
+
+    def outputs(self, s, mask, rows, cols_local, n, like):
+        """(S [rows * cols_local, n], S_mask [rows, cols_local, n] bool, L [rows, cols_local, n]) as LSD_improved returns them:
+        torch CUDA tensors for a torch input, else NumPy (float64 L / S)."""
+        shape = (rows, cols_local, n)
+        S_mask = mask.view(n, cols_local, rows).permute(2, 1, 0) != 0
+        if api._is_torch(like):
+            L = s.dec.device_tensor('L').clone().t()
+            S = s.dec.device_tensor('S').clone().t()
+            return S, S_mask, L.reshape(cols_local, rows, n).permute(1, 0, 2)
+        return s.dec.download('S'), np.ascontiguousarray(S_mask.cpu().numpy()), s.dec.download('L').reshape(shape, order='F')
+
+
+class ShardedLSDImproved:
+    """flow.LSD_improved (/root/reference/lsd_improvement.py:441-487) over `comm.world` GPUs, one call of run() per rank on the rank's
+    image columns shard_columns(w, world, rank) of the [h, w, t] clip:
+      pre-processing   normalizeImage and the mean from three all-reduces (MAX of -min, MAX of the shifted max, SUM);
+      pass 1           ShardedLSD on the column shard (flat 3x3 at delta 1.0, or l1 at delta 10.0) and its foreground mask;
+      columns->frames  one all-to-all of the uint8 mask: this rank gets whole frames shard_frames(t, world, rank);
+      back-off         morphology, merge and the mask-percentage back-off (flow.mask_backoff) on those frames, with one all-reduce
+                       of the positive count per step: every rank takes the same steps;
+      pass 2           the centre-window solve of ShardedLSD, its prox described by exactly the weight map of those frames (device
+                       tensor, no host round trip), and its mask.
+    The disk morphology couples neighbouring columns but not frames, so the frame sharding is exact: no halo, no approximation.  A
+    rank with no frame (t < world) takes part in every collective.  `ops` supplies the solvers and the per-frame work
+    (CudaImprovedOps); the choreography does not know whether it drives CUDA or NumPy.  After run(): weight_frames = this rank's
+    frames of the weight map (float32 [nf][h * w]), frames = (f0, f1), pass1_log / pass2_log = (iterations, converged, ranks)."""
+
+    def __init__(self, comm, ops=None, run_ahead=3):
+        self.comm, self.ops, self.run_ahead = comm, ops if ops is not None else CudaImprovedOps(), run_ahead
+        self.weight_frames = self.frames = self.pass1_log = self.pass2_log = None
+
+    def _all_reduce(self, value, op, dtype):
+        import torch
+        buf = torch.tensor([value], dtype=dtype, device=self.ops.device)
+        op(buf)
+        return buf.item()
+
+    def run(self, cube, shape, alg_ver=2, downsample_ratio=1, hooks=None):
+        """cube: this rank's columns [h, cols_local, t] (NumPy, normalised in place like the reference does, or a torch tensor);
+        shape: (h, w, t) of the whole clip.  hooks(name, 'begin' | 'end') around 'pre', 'pass1', 'mask', 'backoff', 'pass2',
+        'final_mask'.  Returns (S, S_mask, L_recon, ImData1, ImMean, shape, iterations, converged, graph_iter, graph_converged) of
+        LSD_improved, restricted to this rank's columns (ImMean and shape are the whole clip's)."""
+        import torch
+        from . import flow
+        comm, ops = self.comm, self.ops
+        hk = hooks or (lambda name, phase: None)
+        if downsample_ratio != 1:
+            raise Exception("ShardedLSDImproved: downsample_ratio must be 1 (resizing couples columns: resize the clip first)")
+        if alg_ver not in (1, 2):
+            raise Exception("LSD_improved wrong alg ver")
+        h, w, t = (int(v) for v in shape)
+        c0, c1 = shard_columns(w, comm.world, comm.rank)
+        cl = c1 - c0
+        if tuple(int(v) for v in cube.shape) != (h, cl, t):
+            raise Exception("ShardedLSDImproved: rank %d of %d owns columns [%d, %d) of the %d, so its cube must be [%d, %d, %d], not %s"
+                            % (comm.rank, comm.world, c0, c1, w, h, cl, t, tuple(cube.shape)))
+        on_torch = api._is_torch(cube)
+        hk('pre', 'begin')
+        x = cube.to(torch.float64) if on_torch else np.asarray(cube, dtype=np.float64)
+        lo = -self._all_reduce(-float(x.min()), comm.all_reduce_max, torch.float64)
+        x -= lo
+        hi = self._all_reduce(float(x.max()), comm.all_reduce_max, torch.float64)
+        x *= 1.0 / hi
+        mean = self._all_reduce(float(x.sum()), comm.all_reduce_sum, torch.float64) / (h * w * t)
+        x2 = x - mean
+        D = ops.matrix(x2.permute(2, 1, 0).reshape(t, cl * h) if on_torch else np.ascontiguousarray(x2.transpose(2, 1, 0)).reshape(t, cl * h))
+        del x2
+        hk('pre', 'end')
+
+        hk('pass1', 'begin')
+        s1 = ops.pass1(D, h, cl, t, h * w, alg_ver)
+        drv = ShardedLSD(s1, comm, run_ahead=self.run_ahead)
+        drv.solve()
+        hk('pass1', 'end')
+        hk('mask', 'begin')
+        mask = drv.finish(2.0)                                  # [t][h * cl] uint8
+        self.pass1_log = ops.summary(s1)
+        ops.close(s1)
+        del s1, drv
+        f0, f1 = self.frames = shard_frames(t, comm.world, comm.rank)
+        if comm.world == 1:
+            mask_f = mask
+        else:
+            mask_f = mask.new_zeros((max(f1 - f0, 1), h * w))
+            columns_to_frames(comm, mask, mask_f, h, w)
+            mask_f = mask_f[:f1 - f0]
+        hk('mask', 'end')
+
+        hk('backoff', 'begin')
+
+        def weight_for(disk_ratio):
+            wf, count = ops.weight_map(mask_f, h, w, disk_ratio, (1, 1.5))
+            return wf, int(self._all_reduce(int(count), comm.all_reduce_sum, torch.int64))
+        self.weight_frames = flow.mask_backoff(weight_for, h, h * w * t)
+        hk('backoff', 'end')
+
+        hk('pass2', 'begin')
+        s2 = ops.pass2(D, h, cl, t, h * w, w, (f0, f1), self.weight_frames)
+        drv = ShardedLSD(s2, comm, run_ahead=self.run_ahead)
+        drv.solve()
+        hk('pass2', 'end')
+        hk('final_mask', 'begin')
+        mask2 = drv.finish(2.0)
+        self.pass2_log = ops.summary(s2)
+        S, S_mask, L_recon = ops.outputs(s2, mask2, h, cl, t, cube)
+        hk('final_mask', 'end')
+        it, conv, _ = self.pass2_log
+        git, gconv, _ = self.pass1_log
+        return S, S_mask, L_recon, x, mean, (h, w, t), it, conv, git, gconv
 
 
 def cuda_fence(_it):

@@ -327,16 +327,23 @@ def disk_radius(footprint_name, size):
 def apply_morph_ops(input, footprint_name='disk', percetage=0.05):
     """/root/reference/lsd_improvement.py:323-335 on a [h, w, t] boolean cube: dilation, then closing (dilation + erosion), by
     disk(ceil(percetage * h) // 2), frame by frame (the footprint has extent 1 along time)."""
-    torch = _torch()
     r = disk_radius(footprint_name, percetage * input.shape[0])
     dev, (h, w, t) = _mask_to_device(input)
+    return _mask_from_device(morph_frames_dev(dev, h, w, r), (h, w, t), input)
+
+
+def morph_frames_dev(mask_dev, rows, cols, radius):
+    """The morphology of apply_morph_ops on a uint8 [nf][rows * cols] CUDA tensor (pixel p = j*rows + i, non-zero = set, nf >= 1):
+    dilation, then closing (dilation + erosion), by disk(radius), frame by frame.  Returns a new uint8 [nf][rows * cols] tensor."""
+    torch = _torch()
+    nf, m = int(mask_dev.shape[0]), rows * cols
     lib = C.load()
     st = A._stream_ptr()
-    b1, b2 = torch.empty_like(dev), torch.empty_like(dev)
-    scratch = torch.empty(t * h * w + 2 * r + 1, dtype=torch.uint8, device="cuda")
-    for src, dst, erode in ((dev, b1, 0), (b1, b2, 0), (b2, b1, 1)):      # dilation; closing = dilation, erosion
-        C.check(lib.bsub_morph_disk_dev(_vp(src), h * w, _vp(dst), h * w, h, w, t, r, erode, _vp(scratch), st))
-    return _mask_from_device(b1, (h, w, t), input)
+    b1, b2 = (torch.empty((nf, m), dtype=torch.uint8, device="cuda") for _ in range(2))
+    scratch = torch.empty(nf * m + 2 * radius + 1, dtype=torch.uint8, device="cuda")
+    for src, dst, erode in ((mask_dev, b1, 0), (b1, b2, 0), (b2, b1, 1)):      # dilation; closing = dilation, erosion
+        C.check(lib.bsub_morph_disk_dev(_vp(src), src.stride(0), _vp(dst), m, rows, cols, nf, radius, erode, _vp(scratch), st))
+    return b1
 
 
 def merge_masks(masks, weights, background_marker=-1):
@@ -365,22 +372,32 @@ def improved_LSD_weight_mask(D, original_shape, weights, delta=1.0, proximal_obj
     else:
         raise Exception("Unknown improved LSD mode")
     S_mask = A.foreground_mask(D, L, S, sigmas_from_mean=2).reshape(original_shape, order='F')
+
+    def weight_for(disk_ratio):
+        weight_mask = merge_masks((S_mask, apply_morph_ops(S_mask, percetage=disk_ratio)), weights)
+        return weight_mask, int(np.sum(weight_mask > 0))
+    return mask_backoff(weight_for, original_shape[0], S_mask.size), iter_count, convergence
+
+
+def mask_backoff(weight_for, rows, total):
+    """The mask-percentage back-off of build_improved_LSD_graphs (/root/reference/lsd_improvement.py:385-404): weight_for(disk_ratio)
+    -> (weight map, number of its positive entries), total = number of entries of the whole map (rows = image height).  Shrinks the
+    disk ratio by 0.01 from 0.05 while more than 20 % of the map is positive; returns the last weight map.  The decision rests on the
+    count alone, so a sharded caller whose callable returns the all-reduced count takes the same steps on every rank."""
     disk_ratio, step = 0.05, 0.01
     total_allowed_iterations, current_iteration, max_mask_percent = 5, 1, 20
-    S_mask_morph = apply_morph_ops(S_mask, percetage=disk_ratio)
-    weight_mask = merge_masks((S_mask, S_mask_morph), weights)
-    mask_percent = calc_mask_percent(weight_mask) * 100
+    weight_mask, count = weight_for(disk_ratio)
+    mask_percent = count / total * 100
     # the reference's loop raises its own iteration allowance every pass (lsd_improvement.py:396-398), so it only ends when the
     # mask shrinks below the cap; a disk of radius 0 cannot shrink further, which bounds it here
     while mask_percent > max_mask_percent and current_iteration < total_allowed_iterations:
         disk_ratio -= step
         total_allowed_iterations += 1
-        if disk_ratio * original_shape[0] <= 0:
+        if disk_ratio * rows <= 0:
             break
-        S_mask_morph = apply_morph_ops(S_mask, percetage=disk_ratio)
-        weight_mask = merge_masks((S_mask, S_mask_morph), weights)
-        mask_percent = calc_mask_percent(weight_mask) * 100
-    return weight_mask, iter_count, convergence
+        weight_mask, count = weight_for(disk_ratio)
+        mask_percent = count / total * 100
+    return weight_mask
 
 
 def build_improved_LSD_graphs(D, original_shape, weights, delta=1.0, proximal_object=None, mode=None):

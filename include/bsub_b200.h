@@ -178,6 +178,14 @@ int bsub_step_prox_buffers(bsub_solver* s, float** G_S, float** S, int64_t* ld);
 int bsub_set_frame_windows(bsub_solver* s, int32_t rows, int32_t cols, int32_t f0, int32_t nf, const double* eta_host, int64_t n_eta);
 int bsub_set_frame_center_windows(bsub_solver* s, int32_t rows, int32_t cols, int32_t f0, int32_t nf, const float* eta_host,
                                   const uint8_t* background_host);
+/* _center_windows from a weight map already on the device (BSUB_PROX_GRAPH_CENTER_BG): weight float32 [nf][ld] (device memory, row
+ * pitch ld >= rows*cols), row f = frame f0 + f, pixel p = j*rows + i -- LSD_improved's merged map of those frames.  An entry > 0 is
+ * the weight of the centre window at that pixel, < 0 marks a background pixel, 0 is neither: the same description
+ * bsub_set_frame_center_windows builds from eta = max(weight, 0) and background = (weight < 0).  A kernel on `stream` writes it into
+ * new device buffers; the call then waits for the stream and, if an entry is not finite, reports the first one (its row, pixel and
+ * clip frame) and keeps the handle's previous description.  nf == 0 is accepted (weight may then be NULL). */
+int bsub_set_frame_weight_map_dev(bsub_solver* s, int32_t rows, int32_t cols, int32_t f0, int32_t nf, const float* weight, int64_t ld,
+                                  void* stream);
 int bsub_set_frame_graphs(bsub_solver* s, int32_t rows, int32_t cols, int32_t f0, int32_t nf, int32_t n_graphs, const int32_t* frame_graph,
                           const int64_t* n_groups, const int32_t* const* indptr, const int32_t* const* indices, const double* const* eta,
                           const uint8_t* background_host);
