@@ -1188,8 +1188,7 @@ EigPlan make_eig_plan(int n, int npad) {
     EigPlan p;
     p.n = n; p.npad = npad;
     int C = 1;
-    int rows_target = 40;
-    if (const char* e = getenv("BSUB_EIG_ROWS")) rows_target = std::max(1, std::min(atoi(e), 3 * EIG_WARPS));   // <= 3 rows per warp
+    const int rows_target = 40;
     while (C < 16 && (n + C - 1) / C > rows_target) C *= 2;
     const size_t cap = 225 * 1024;
     auto bytes_for = [&](int Cc, bool in_smem) {

@@ -266,13 +266,6 @@ int make_tensor_map_u64(CUtensorMap* map, const void* base, int rank, const uint
     return make_tensor_map_any(map, base, CU_TENSOR_MAP_DATA_TYPE_UINT64, rank, dims, strides_bytes, box, CU_TENSOR_MAP_SWIZZLE_NONE);
 }
 
-int make_tensor_map_u64_swz(CUtensorMap* map, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
-                            const uint32_t* box, int swizzle_bytes) {
-    const CUtensorMapSwizzle swz = swizzle_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : swizzle_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B :
-                                   swizzle_bytes == 32 ? CU_TENSOR_MAP_SWIZZLE_32B : CU_TENSOR_MAP_SWIZZLE_NONE;
-    return make_tensor_map_any(map, base, CU_TENSOR_MAP_DATA_TYPE_UINT64, rank, dims, strides_bytes, box, swz);
-}
-
 int make_tensor_map_u8(CUtensorMap* map, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
                        const uint32_t* box, int swizzle_bytes) {
     const CUtensorMapSwizzle swz = swizzle_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : swizzle_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B :

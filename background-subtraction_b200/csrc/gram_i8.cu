@@ -17,7 +17,6 @@
 //   warp 2     TMEM allocator (512 columns = 4 classes x 128)
 //   warps 4-7  epilogue: tcgen05.ld of the four class accumulators, recombination into int64, atomicAdd to global
 #include <cooperative_groups.h>
-#include <stdio.h>
 #include <math.h>
 #include <algorithm>
 #include <vector>
@@ -657,7 +656,6 @@ int launch_gram_i8(const GramI8Plan& p, const CUtensorMap& map, const CUtensorMa
                 if (cudaOccupancyMaxActiveClusters(&ncl, gram_i8_c3_kernel, &cfg) == cudaSuccess && ncl >= 2) c3_clusters = std::min(ncl, p.grid / 3);
             }
             (void)cudaGetLastError();
-            if (getenv("BSUB_DEBUG")) fprintf(stderr, "gram_i8: %d multicast clusters of 3 CTAs\n", c3_clusters);
         }
         if (c3_clusters >= 2) {
             GramI8C3Args c;

@@ -89,7 +89,7 @@ int launch_shrink(const ShrinkPlan& p, ShrinkBuffers b, const DevState* st, int 
 
 // ---------------------------------------------------------------- shrink_tma.cu (fast path, rows % 4 == 0)
 struct ShrinkTmaPlan {
-    int n, rows, cols, R, P, Cf, nf, KR, grid_clusters, nparts, ntile_r, ntile_c, bufstride, NT, occ;
+    int n, rows, cols, R, P, Cf, nf, KR, grid_clusters, nparts, ntile_r, ntile_c, bufstride;
     long long ld, ntiles;
     size_t smem_bytes, tpart_floats;
 };
@@ -101,7 +101,7 @@ int launch_shrink_tma(const ShrinkTmaPlan& p, const ShrinkTmaMaps& maps, ShrinkB
 
 // ---------------------------------------------------------------- shrink_stream.cu (fastest path: rank <= 16, rows % 4 == 0)
 struct ShrinkStreamPlan {
-    int n, rows, cols, R, P, FC, NS, NCW, nchunkf, grid, nparts, ntile_r, ntile_c, bufstride;
+    int n, rows, cols, R, P, FC, NS, nchunkf, grid, nparts, ntile_r, ntile_c, bufstride;
     int kcap;                  // largest rank the streamed kernel takes (16)
     long long ld, ntiles;
     size_t smem_bytes;
@@ -117,8 +117,7 @@ int launch_shrink_stream(const ShrinkStreamPlan& p, const ShrinkTmaMaps& maps, S
 
 // ---------------------------------------------------------------- shrink_flat.cu (single-pass streamed shrink, rank <= 8, T from project.cu)
 struct ShrinkFlatPlan { int n, rows, cols, FC, NS, nchunkf, ntile_r, grid; long long ld, ntiles; size_t smem_bytes; };
-struct ShrinkFlatMaps { CUtensorMap D, S, Y, Q, VC;
-                        CUtensorMap Qs; };   // digit planes, 8 frames x 9 units per box, 128-byte swizzle (register-transposed stores)
+struct ShrinkFlatMaps { CUtensorMap D, S, Y, Q, VC; };
 bool make_shrink_flat_plan(int n, int rows, int cols, long long ld, int num_sms, const ShrinkStreamPlan& sp, ShrinkFlatPlan* out);
 int make_shrink_flat_maps(const ShrinkFlatPlan& p, const float* D, float* S, float* Y, signed char* Wq, long long ldq, const float* VC, int vstride,
                           ShrinkFlatMaps* m);
@@ -184,8 +183,8 @@ int launch_block_l2_apply(const float* U, float* V, const unsigned char* labels,
                           double mu_override, double non_block_lambda, cudaStream_t s, int keep_other = 0);
 int launch_prox_l1(const float* U, float* V, long long ld, long long m, int n, float lam, cudaStream_t s);
 struct GraphProxPlan { int rows, cols, n; long long ld; size_t xi_floats; int max_sweeps; float tol; };
-// workspace: xi = duals of whole frames (capped: the kernel walks the frames in chunks that fit), tot = per-pixel dual sums of
-// the frames held (ld floats each); BSUB_GRAPH_GLOBAL selects the HBM-resident sweep kernel (all frames at once)
+// workspace: xi = duals of whole frames (BSUB_GRAPH_XI_MB cap, default 8 GB: the kernel walks the frames in chunks that fit),
+// tot = per-pixel dual sums of the frames held (ld floats each)
 void prox_graph3_workspace(int rows, int cols, int n, long long ld, int center, long long* xi_floats, long long* tot_floats);
 int launch_prox_graph3(const float* U, float* V, float* xi, long long xi_floats, float* tot, const float* eta, long long ld, int rows,
                        int cols, int n, float lam, int max_sweeps, float tol, int* sweeps_out, const DevState* st,

@@ -13,7 +13,6 @@
 // r x 4 partial sums in registers and reduce over the 8 frame lanes with shuffles.  Output: T in pixel order ([k][ld], for
 // the final materialisation of L) and regrouped per tile and 3x3 group ([tile][k][group][12]) for the shrink kernel.
 // HBM traffic: 4 B per matrix element read (+ r/n of that written).
-#include <stdlib.h>
 #include <algorithm>
 #include "common.cuh"
 #include "kernels.h"
@@ -191,7 +190,6 @@ bool make_project_plan(int n, int R, long long ldq, int num_sms, ProjectPlan* ou
     // warps with a prefetch slot; two slots per warp only when shared memory holds them for a full set of warps
     if (nslots >= 2 * PJ_MAXW) { p.DEPTH = 2; p.NW = PJ_MAXW; }
     else { p.DEPTH = 1; p.NW = std::min(PJ_MAXW, nslots); }
-    if (const char* e = getenv("BSUB_PROJ_WARPS")) { const int w = atoi(e); if (w >= 1 && w <= PJ_MAXW && w * p.DEPTH <= nslots) p.NW = w; }
     p.smem_bytes = vs + (size_t)p.NW * p.DEPTH * p.slot_bytes;
     const long long nunits = ldq / 16;
     p.grid = (int)std::max<long long>(1, std::min<long long>(num_sms, (nunits + p.NW - 1) / p.NW));

@@ -246,156 +246,28 @@ int launch_prox_l1(const float* U, float* V, long long ld, long long m, int n, f
 // colour are disjoint, so one colour step is one fully parallel pass.  Window geometry reproduces
 // get_vars_idx_top_left (/root/reference/utils.py:249-257): top-lefts i in [0, rows-3], j in [0, cols-3],
 // extent min(3, rows-1-i) x min(3, cols-1-j)  => last image row / column uncovered (SURVEY Q8).
-// Per frame f: xi[f][w][9] dual variables, tot[f][p] = sum of duals on pixel p.  A persistent cooperative grid
-// sweeps until the largest dual change of a sweep is <= tol (checked every sweep through a device flag pair).
-struct GraphArgs {
-    const float* U; float* V; float* xi; float* tot; const float* eta;
-    long long ld; int rows, cols, n; float lam; int max_sweeps; float tol;
-    int* sweeps_out; unsigned int* change_bits;   // [2] ping-pong max-change (as float bits)
-    const DevState* st;
-    // centre mode (get_proximal_graph_group_centers, /root/reference/lsd_improvement.py:74-120): one candidate window per
-    // pixel, centred on it and clipped to the image (utils.py:234-246); eta[f][pixel] > 0 selects and weights it
-    int center; long long eta_stride;
-};
-
-__global__ void __launch_bounds__(PX_THREADS) prox_graph3_kernel(GraphArgs a) {
-    cg::grid_group grid = cg::this_grid();
-    if (a.st != nullptr) {
-        if (a.st->done) return;                                  // uniform over the grid
-        a.lam = (float)(a.st->lambda / a.st->mu);
-        a.tol = a.tol * a.lam;                                   // relative tolerance in solver mode
-    }
-    const int rows = a.rows, cols = a.cols;
-    const bool ctr = a.center != 0;
-    const int nwi = ctr ? rows : rows - min(3, rows) + 1, nwj = ctr ? cols : cols - min(3, cols) + 1;   // numX, numY of the reference
-    const long long nw = (long long)nwi * nwj;
-    const long long gsz = (long long)gridDim.x * blockDim.x, gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    // init
-    for (long long i = gid; i < (long long)a.n * a.ld; i += gsz) a.tot[i] = 0.f;
-    for (long long i = gid; i < (long long)a.n * nw * 9; i += gsz) a.xi[i] = 0.f;
-    if (gid == 0) { a.change_bits[0] = 0u; a.change_bits[1] = 0u; }
-    grid.sync();
-    int sw = 0;
-    for (; sw < a.max_sweeps; ++sw) {
-        float mych = 0.f;
-        for (int col = 0; col < 9; ++col) {
-            const int ci = col % 3, cj = col / 3;
-            const int ni = (nwi - ci + 2) / 3, nj = (nwj - cj + 2) / 3;       // windows of this colour per axis
-            const long long nwc = (ni > 0 && nj > 0) ? (long long)ni * nj : 0;
-            for (long long t = gid; t < nwc * a.n; t += gsz) {
-                const int f = (int)(t / nwc);
-                const long long wq = t - (long long)f * nwc;
-                const int wj = (int)(wq / ni) * 3 + cj, wi = (int)(wq % ni) * 3 + ci;
-                const int i0 = ctr ? max(wi - 1, 0) : wi, j0 = ctr ? max(wj - 1, 0) : wj;
-                const int hh = ctr ? min(wi + 1, rows - 1) - i0 + 1 : min(3, rows - 1 - wi);
-                const int ww = ctr ? min(wj + 1, cols - 1) - j0 + 1 : min(3, cols - 1 - wj);
-                if (hh <= 0 || ww <= 0) continue;
-                const long long widx = (long long)wj * nwi + wi;
-                const float eta_w = ctr ? a.eta[(size_t)f * a.eta_stride + widx] : (a.eta != nullptr ? a.eta[widx] : 1.f);
-                if (ctr && !(eta_w > 0.f)) continue;                      // no group centred on this pixel in this frame
-                const float* u = a.U + (size_t)f * a.ld;
-                float* tot = a.tot + (size_t)f * a.ld;
-                float* xi = a.xi + ((size_t)f * nw + widx) * 9;
-                const float radius = a.lam * eta_w;
-                float r[9], ar[9], xo[9];
-                float sabs = 0.f;
-#pragma unroll
-                for (int c = 0; c < 3; ++c)
-#pragma unroll
-                    for (int dr = 0; dr < 3; ++dr) {
-                        const int e = c * 3 + dr;
-                        const bool ok = (dr < hh) && (c < ww);
-                        float val = 0.f, x0 = 0.f;
-                        if (ok) {
-                            const long long p = (long long)(j0 + c) * rows + i0 + dr;
-                            x0 = xi[e];
-                            val = u[p] - tot[p] + x0;
-                        }
-                        r[e] = val; ar[e] = fabsf(val); xo[e] = x0; sabs += fabsf(val);
-                    }
-                float theta = 0.f;
-                if (sabs > radius) theta = px_clip_level9(ar, radius);
-#pragma unroll
-                for (int c = 0; c < 3; ++c)
-#pragma unroll
-                    for (int dr = 0; dr < 3; ++dr) {
-                        const int e = c * 3 + dr;
-                        if ((dr < hh) && (c < ww)) {
-                            const long long p = (long long)(j0 + c) * rows + i0 + dr;
-                            const float xn = copysignf(fmaxf(ar[e] - theta, 0.f), r[e]);   // projection on the l1 ball
-                            const float dlt = xn - xo[e];
-                            xi[e] = xn;
-                            tot[p] += dlt;
-                            mych = fmaxf(mych, fabsf(dlt));
-                        }
-                    }
-            }
-            grid.sync();
-        }
-        mych = warp_max(mych);
-        if ((threadIdx.x & 31) == 0 && mych > 0.f) atomicMax(a.change_bits + (sw & 1), __float_as_uint(mych));
-        grid.sync();
-        const float ch = __uint_as_float(*((volatile unsigned int*)(a.change_bits + (sw & 1))));
-        if (gid == 0) a.change_bits[(sw + 1) & 1] = 0u;
-        if (ch <= a.tol) { ++sw; break; }
-    }
-    grid.sync();
-    for (long long i = gid; i < (long long)a.n * a.ld; i += gsz) a.V[i] = a.U[i] - a.tot[i];
-    if (gid == 0 && a.sweeps_out != nullptr) *a.sweeps_out = sw;
-}
-
-static int launch_prox_graph3_global(const float* U, float* V, float* xi, float* tot, const float* eta, long long ld, int rows, int cols, int n,
-                                     float lam, int max_sweeps, float tol, int* sweeps_out, const DevState* st, cudaStream_t s, int center,
-                                     long long eta_stride) {
-    static int blocks_per_sm = 0, num_sms = 0;
-    static unsigned int* change_bits = nullptr;
-    if (blocks_per_sm == 0) {
-        int dev = 0;
-        BSUB_CUDA_CHECK(cudaGetDevice(&dev));
-        BSUB_CUDA_CHECK(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev));
-        BSUB_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, prox_graph3_kernel, PX_THREADS, 0));
-        if (blocks_per_sm < 1) { set_error("prox_graph3: kernel does not fit"); return -1; }
-        BSUB_CUDA_CHECK(cudaMalloc(&change_bits, 2 * sizeof(unsigned int)));
-    }
-    GraphArgs a;
-    a.U = U; a.V = V; a.xi = xi; a.tot = tot; a.eta = eta; a.ld = ld; a.rows = rows; a.cols = cols; a.n = n; a.lam = lam;
-    // sweeps_out, when given, is an int[4] owned by the caller: [0] sweeps used, [1..2] the ping-pong change flags (per solver
-    // handle, so that handles running concurrently on different streams do not share them)
-    a.max_sweeps = max_sweeps; a.tol = tol; a.sweeps_out = sweeps_out; a.st = st;
-    a.change_bits = (sweeps_out != nullptr) ? reinterpret_cast<unsigned int*>(sweeps_out + 1) : change_bits;
-    a.center = center; a.eta_stride = eta_stride;
-    if (center && eta == nullptr) { set_error("prox_graph3: centre mode needs the per-frame eta map"); return -1; }
-    const long long nw9 = ((long long)rows * cols / 9 + 1) * n;
-    long long want = (nw9 + PX_THREADS - 1) / PX_THREADS;
-    long long maxb = (long long)blocks_per_sm * num_sms;
-    if (want > maxb) want = maxb;
-    if (want < 1) want = 1;
-    void* args[] = {&a};
-    BSUB_CUDA_CHECK(cudaLaunchCooperativeKernel((void*)prox_graph3_kernel, dim3((unsigned)want), dim3(PX_THREADS), args, 0, s));
-    return 0;
-}
-
-// ---------------------------------------------------------------------------------------- overlapping windows, tile-local
-// The same dual block-coordinate descent, reordered so that the sweeps run in shared memory instead of HBM.  The early ALM
-// iterations need thousands of sweeps (lambda/mu is large and the dual mass spreads like a diffusion: measured with the oracle,
-// WaterSurface iteration 1 = 4292 sweeps, a 540 x 960 frame ~1900); the kernel above moves ~180 B per matrix element and
-// sweep through HBM and pays ten grid-wide barriers per sweep.  Here a CTA takes a GT_T x GT_T pixel tile of one frame, loads
-// u, the per-pixel dual sums `tot` and the duals of the windows that lie ENTIRELY inside the tile (84 B per element), runs up
-// to GT_INNER nine-colour sweeps on them in shared memory (block barriers only) and writes them back.  Windows that straddle
+// Per frame f: xi[f][w][9] dual variables, tot[f][p] = sum of duals on pixel p.
+//
+// The sweeps run in shared memory, not in HBM.  The early ALM iterations need thousands of sweeps (lambda/mu is large and the
+// dual mass spreads like a diffusion: measured with the oracle, WaterSurface iteration 1 = 4292 sweeps, a 540 x 960 frame
+// ~1900), and a grid-wide sweep over HBM moves ~180 B per matrix element and sweep and pays ten grid-wide barriers per sweep
+// (one per colour, plus the stop test).  Here a CTA takes a GT_T x GT_T pixel tile of one frame, loads u, the per-pixel dual
+// sums `tot` and the duals of the windows that lie ENTIRELY inside the tile (84 B per element), runs up to GT_INNER nine-colour sweeps on them in shared memory (block barriers only) and writes them back.  Windows that straddle
 // a tile border stay frozen during that visit; the tiling is shifted diagonally by a third of a tile in each of three phases
 // ((0,0), (11,11), (22,22)): a window straddles a row border in at most one phase and a column border in at most one phase,
 // so it is interior -- and updated -- in at least one of the three.  Every update is still an exact block minimisation of
 // the same dual objective and simultaneously updated windows never overlap, so the iteration converges to the same (unique)
 // primal solution as the sequential sweep of the oracle; stop test: the largest dual change of a whole outer iteration
 // (3 phases x inner sweeps) <= tol.  One grid-wide barrier per phase instead of per colour.
-// The state is (xi, tot) with r = u - tot + xi and tot += xi' - xi exactly as in the kernel above: a window whose projection
-// reproduces its dual bit for bit changes nothing, so the iteration reaches a true fixed point in fp32 (carrying x = u - tot
-// instead re-rounds x at every visit: it never settles below ~1 ulp of u and drifts -- seen in round 2).
+// The state is (xi, tot) with r = u - tot + xi and tot += xi' - xi: a window whose projection reproduces its dual bit for bit
+// changes nothing, so the iteration reaches a true fixed point in fp32 (carrying x = u - tot instead re-rounds x at every
+// visit: it never settles below ~1 ulp of u and drifts -- seen in round 2).
 // Duals are not kept between calls (cold start, like the oracle), so frames are processed in chunks whose duals fit the
 // caller's buffer (prox_graph3_workspace: capped, default 8 GB) -- 4K x 600 needs ~18 GB per 60-frame chunk instead of 179 GB.
 constexpr int GT_T = 32, GT_PITCH = 33, GT_THREADS = 128, GT_INNER = 48, GT_SHIFT = 11;
 constexpr int GT_TILE = GT_T * GT_PITCH;
 constexpr size_t GT_SMEM = sizeof(float) * (size_t)GT_TILE * (3 + 9);
+constexpr float GT_COUNT_FACTOR = 8.f;      // dead bands a dual change must exceed to count towards the stop test (see the kernel)
 
 struct GraphTileArgs {
     const float* U; float* V; float* xi; float* tot; const float* eta;
@@ -405,6 +277,8 @@ struct GraphTileArgs {
     float count_factor;                           // a change counts towards the stop test when it exceeds count_factor x the dead band
     int* stats;                                   // [3] running totals over the calls of a handle: outer iterations, calls, calls that hit the cap
     const DevState* st;
+    // centre mode (get_proximal_graph_group_centers, /root/reference/lsd_improvement.py:74-120): one candidate window per
+    // pixel, centred on it and clipped to the image (utils.py:234-246); eta[f][pixel] > 0 selects and weights it
     int center; long long eta_stride;
     int nwi, nwj, chunk;
 };
@@ -614,21 +488,13 @@ __global__ void __launch_bounds__(GT_THREADS) prox_graph3_tile_kernel(GraphTileA
     }
 }
 
-static bool graph3_use_global() {
-    static const bool g = getenv("BSUB_GRAPH_GLOBAL") != nullptr;
-    return g;
-}
-
 // workspace of launch_prox_graph3: duals xi (whole frames, capped) and per-pixel dual sums tot (one row of ld floats per frame held)
 void prox_graph3_workspace(int rows, int cols, int n, long long ld, int center, long long* xi_floats, long long* tot_floats) {
     const long long nw = center ? (long long)rows * cols : (long long)(rows - std::min(3, rows) + 1) * (cols - std::min(3, cols) + 1);
-    long long frames = n;
-    if (!graph3_use_global()) {
-        long long cap_mb = 8192;
-        if (const char* e = getenv("BSUB_GRAPH_XI_MB")) cap_mb = std::max(1LL, atoll(e));
-        const long long cap = cap_mb * (1LL << 20) / 4;
-        frames = std::max(1LL, std::min<long long>(n, cap / std::max(1LL, nw * 9)));
-    }
+    long long cap_mb = 8192;
+    if (const char* e = getenv("BSUB_GRAPH_XI_MB")) cap_mb = std::max(1LL, atoll(e));
+    const long long cap = cap_mb * (1LL << 20) / 4;
+    const long long frames = std::max(1LL, std::min<long long>(n, cap / std::max(1LL, nw * 9)));
     *xi_floats = frames * nw * 9 + 16;            // + the three work counters of the tile kernel
     *tot_floats = frames * ld;
 }
@@ -637,8 +503,6 @@ int launch_prox_graph3(const float* U, float* V, float* xi, long long xi_floats,
                        int n, float lam, int max_sweeps, float tol, int* sweeps_out, const DevState* st, cudaStream_t s, int center,
                        long long eta_stride) {
     if (xi == nullptr || tot == nullptr) { set_error("prox_graph3: missing workspace"); return -1; }
-    if (graph3_use_global())
-        return launch_prox_graph3_global(U, V, xi, tot, eta, ld, rows, cols, n, lam, max_sweeps, tol, sweeps_out, st, s, center, eta_stride);
     if (sweeps_out == nullptr) { set_error("prox_graph3: the caller's int[8] status block is required"); return -1; }
     static int blocks_per_sm = 0, num_sms = 0;
     static unsigned long long attr_devs = 0;
@@ -659,8 +523,7 @@ int launch_prox_graph3(const float* U, float* V, float* xi, long long xi_floats,
     // solver handle, so that handles running concurrently on different streams do not share them), [4..6] running totals
     a.change_bits = reinterpret_cast<unsigned int*>(sweeps_out + 1);
     a.stats = sweeps_out + 4;                                              // the caller's int[8]: [4..6] running totals
-    static const float count_factor = getenv("BSUB_GRAPH_COUNT_FACTOR") ? (float)atof(getenv("BSUB_GRAPH_COUNT_FACTOR")) : 8.f;
-    a.count_factor = count_factor;
+    a.count_factor = GT_COUNT_FACTOR;
     a.center = center; a.eta_stride = eta_stride;
     a.nwi = center ? rows : rows - std::min(3, rows) + 1;
     a.nwj = center ? cols : cols - std::min(3, cols) + 1;

@@ -21,7 +21,7 @@
 // (sum_active - z) / |active| of the final set, exact to fp32 rounding for every group size).  Groups of <= PG_SMALL pixels take
 // one thread each (no local arrays: the operands are re-read from shared memory on each pass), larger ones one warp.
 // fp32 hazards handled as in the tile kernel: the state is (xi, tot), not x = u - tot; a projection that moved by <= ~2 ulp of its
-// operands keeps its dual, and a change counts towards the stop test only above count_factor of those dead bands.
+// operands keeps its dual, and a change counts towards the stop test only above PG_COUNT_FACTOR of those dead bands.
 #include <cooperative_groups.h>
 #include <math.h>
 #include <stdlib.h>
@@ -38,6 +38,7 @@ constexpr int PG_THREADS = 256;
 constexpr int PG_SMALL = 32;                       // groups up to this size: one thread; larger: one warp
 constexpr int PG_MAX_SHIFT = 15;                   // <= 32768 pixels (128 KB of tot) per CTA
 constexpr float PG_BAND = 2.4e-7f;                 // ~2 ulp
+constexpr float PG_COUNT_FACTOR = 8.f;             // dead bands a dual change must exceed to count towards the stop test
 
 struct PgArgs {
     const float* U; float* V; long long ld; int m, n;
@@ -406,8 +407,7 @@ int launch_prox_graph_generic(const float* U, float* V, long long ld, long long 
                                              (int)(sizeof(float) << PG_MAX_SHIFT)));
     PgArgs a;
     a.U = U; a.V = V; a.ld = ld; a.m = (int)m; a.n = n; a.lam = lam; a.tol = tol; a.max_sweeps = max_sweeps;
-    static const float count_factor = getenv("BSUB_GRAPH_COUNT_FACTOR") ? (float)atof(getenv("BSUB_GRAPH_COUNT_FACTOR")) : 8.f;
-    a.count_factor = count_factor;
+    a.count_factor = PG_COUNT_FACTOR;
     a.g = g; a.xi = xi; a.totg = L.tot_global ? totg : nullptr; a.shift = L.shift; a.status = status; a.st = st;
     cudaLaunchConfig_t cfg = {};
     cudaLaunchAttribute attr[1];

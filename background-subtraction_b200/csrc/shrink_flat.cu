@@ -25,7 +25,6 @@
 // for 2 + 2.  T of the whole group (6 x r x 768 B) sits in shared memory.
 // Rank > 8, the first iteration (no planes of W yet), the spill modes and image heights that are not a multiple of 4
 // stay on shrink_stream.cu / shrink_tma.cu / shrink.cu; the choice is made on the device from DevState.
-#include <stdlib.h>
 #include <algorithm>
 #include "common.cuh"
 #include "kernels.h"
@@ -47,8 +46,6 @@ struct ShrinkFlatArgs {
     int force_S;                           // always store S (pixel-sharded drivers, restart after a saturated digit pass)
     double* part_zz; unsigned long long* part_nnz; float* part_max; float* part_wmax;
     int mode;
-    int probe;                             // BSUB_FLAT_PROBE (measurement only, results are wrong): 1 = data movement without compute
-    int policy;                            // L2 evict_first hint on the D / Y loads (bit 0) and on the S / Y stores (bit 1); BSUB_FLAT_POLICY
 };
 
 __device__ __forceinline__ void sf_mbar_arrive(uint64_t* bar) {
@@ -144,25 +141,18 @@ __device__ __forceinline__ void sf_item(float* dsp, float* ysp, const float (&T)
 }
 
 // consumer side of one group of gt tiles: for every frame chunk, for every tile of the group: one stage of FC frames.
-// XP = 0: the 9 words of a (group, frame) go to a warp-private staging area, and the warp transposes 4 pixels x 4 digits with byte
-//         permutes from there (dense plane boxes [4][9][FC][16 B] in the stage).
-// XP = 1: the 4 x 4 byte transpose runs in registers over the four lanes that hold four neighbouring groups (2 shuffles + 2 byte
-//         permutes per word), and every lane stores ONE 32-bit word per entry: plane (g & 3), unit e, frame f, word (g >> 2).  The
-//         stage holds the planes as 4 x FC/8 boxes of [9 units][8 frames][16 B] = 9 rows of 128 B under TMA's 128-byte swizzle
-//         (16-byte chunk index ^= 128-byte row index & 7, both taken from the shared-memory address): the four planes of an entry
-//         lie 18 rows apart (FC = 16), i.e. in rows of residues r, r+2, r+4, r+6 mod 8, and the warp's two frames f, f+1 (f even)
-//         are chunks c, c^1 before the XOR -> the 32 stores of one entry hit 8 different chunks x 4 words = 32 distinct banks
-//         (the dense layout puts the 16 lanes of a frame on 4 banks).
-template <int KR, int MODE, int XP>
+// The 9 words of a (group, frame) go to a warp-private staging area, and the warp transposes 4 pixels x 4 digits with byte
+// permutes from there (dense plane boxes [4][9][FC][16 B] in the stage).  Kept over a transpose in registers across lanes
+// (1080p x 300, ms per solve: 94.4 staged, 100.5 in registers with 128-byte-swizzled 8-frame boxes, 94.7 in registers with the
+// dense boxes; profiles/r2r_shrink_variants.log): the bank conflicts of the staged stores do not bound the kernel.
+template <int KR, int MODE>
 __device__ __forceinline__ void sf_group(const ShrinkFlatArgs& a, const float* Tg, int gt, unsigned char* ring, size_t stage_bytes, const float* Vst_all,
                                          unsigned int* ustage, uint64_t* full, uint64_t* done, int& q, int lane, int cw, const SfScal& sc, const bool ws,
                                          float& zl_acc, unsigned int& nnz_acc, float& max_acc, float& wmax_acc) {
     const int g = lane & 15, flh = lane >> 4;
     const int FC = a.FC, NS = a.NS;
-    unsigned int* ust = ustage + flh * SF_P + g;              // XP = 0: this thread's words of the warp's staging area: [frame half][entry][group]
+    unsigned int* ust = ustage + flh * SF_P + g;              // this thread's words of the warp's staging area: [frame half][entry][group]
     const size_t slot = (size_t)FC * SF_P * sizeof(float);
-    const int l4 = g & 3;
-    const unsigned int sel1 = (l4 & 2) ? 0x3276u : 0x5410u, sel2 = (l4 & 1) ? 0x3715u : 0x6240u;
     for (int c = 0; c < a.nchunkf; ++c)
         for (int t = 0; t < gt; ++t, ++q) {
             float T[KR > 0 ? KR : 1][9];                      // the 3x3 group's T of this tile
@@ -180,56 +170,34 @@ __device__ __forceinline__ void sf_group(const ShrinkFlatArgs& a, const float* T
             unsigned char* b = ring + (size_t)s * stage_bytes;
             float* bD = reinterpret_cast<float*>(b);
             float* bY = reinterpret_cast<float*>(b + slot);
-            unsigned char* bP = b + 2 * slot;                     // XP = 0: [4 planes][9 k16 blocks][FC frames][16 B]
-            const uint32_t bPa = smem_u32(bP);
+            unsigned char* bP = b + 2 * slot;                     // [4 planes][9 k16 blocks][FC frames][16 B]
             const float* Vst = Vst_all + (size_t)s * FC * SF_KMAX;
-            for (int f0 = 0; f0 < FC && a.probe != 1; f0 += SF_FL) {
+            for (int f0 = 0; f0 < FC; f0 += SF_FL) {
                 unsigned int uw[9];
-                if (XP) {
-                    const int f = f0 + 2 * cw + flh;              // the warp's two frames of this round (even, odd): loads stay conflict-free
-                    sf_item<KR, MODE>(bD + (size_t)f * SF_P + 3 * g, bY + (size_t)f * SF_P + 3 * g, T, Vst + f * SF_KMAX, sc, ws, uw, zl_acc, nnz_acc,
-                                      max_acc, wmax_acc);
-                    // XP = 1: box (plane l4, frames 8*(f>>3) .. +7): 9 rows of 128 B, swizzled
-                    // XP = 2: the dense boxes of XP = 0 ([plane][unit][FC frames][16 B]): 256-byte runs in HBM, 4-way bank conflicts
-                    const uint32_t box = (XP == 1) ? bPa + (uint32_t)((l4 * (FC >> 3) + (f >> 3)) * (9 * 128)) + 4u * (uint32_t)(g >> 2)
-                                                   : bPa + (uint32_t)(l4 * 9 * FC * 16 + f * 16) + 4u * (uint32_t)(g >> 2);
-                    const uint32_t rstride = (XP == 1) ? 128u : (uint32_t)(FC * 16);
+                const int fw = f0 + 2 * cw, f = fw + flh;     // the warp's two frames of this round, and mine
+                sf_item<KR, MODE>(bD + (size_t)f * SF_P + 3 * g, bY + (size_t)f * SF_P + 3 * g, T, Vst + f * SF_KMAX, sc, ws, uw, zl_acc, nnz_acc,
+                                  max_acc, wmax_acc);
 #pragma unroll
-                    for (int e = 0; e < 9; ++e) {
-                        const unsigned int r1 = __shfl_xor_sync(0xffffffffu, uw[e], 2);
-                        const unsigned int v = __byte_perm(uw[e], r1, sel1);
-                        const unsigned int r2 = __shfl_xor_sync(0xffffffffu, v, 1);
-                        const unsigned int o = __byte_perm(v, r2, sel2);
-                        const uint32_t row = box + rstride * e;
-                        const uint32_t addr = (XP == 1) ? row + ((((row >> 7) ^ (uint32_t)f) & 7u) << 4) : row;
-                        asm volatile("st.shared.u32 [%0], %1;" ::"r"(addr), "r"(o) : "memory");
+                for (int e = 0; e < 9; ++e) ust[e * SF_NG] = uw[e];
+                __syncwarp();
+                // 2 frames x 36 position quads: 4 pixels x 4 digits -> one 32-bit word per plane
+#pragma unroll
+                for (int tt = 0; tt < 3; ++tt) {
+                    const int qi = lane + 32 * tt;
+                    if (qi < 72) {
+                        const int fh = qi / 36, pq = qi - 36 * fh;
+                        const uint4 w = *reinterpret_cast<const uint4*>(ustage + fh * SF_P + 4 * pq);
+                        const unsigned int t0 = __byte_perm(w.x, w.y, 0x5140), t1 = __byte_perm(w.z, w.w, 0x5140);
+                        const unsigned int t2 = __byte_perm(w.x, w.y, 0x7362), t3 = __byte_perm(w.z, w.w, 0x7362);
+                        unsigned char* dst = bP + ((size_t)(pq >> 2) * FC + (fw + fh)) * 16 + 4 * (pq & 3);
+                        const size_t pstride = (size_t)9 * FC * 16;
+                        *reinterpret_cast<unsigned int*>(dst) = __byte_perm(t0, t1, 0x5410);
+                        *reinterpret_cast<unsigned int*>(dst + pstride) = __byte_perm(t0, t1, 0x7632);
+                        *reinterpret_cast<unsigned int*>(dst + 2 * pstride) = __byte_perm(t2, t3, 0x5410);
+                        *reinterpret_cast<unsigned int*>(dst + 3 * pstride) = __byte_perm(t2, t3, 0x7632);
                     }
-                } else {
-                    const int fw = f0 + 2 * cw, f = fw + flh;     // the warp's two frames of this round, and mine
-                    sf_item<KR, MODE>(bD + (size_t)f * SF_P + 3 * g, bY + (size_t)f * SF_P + 3 * g, T, Vst + f * SF_KMAX, sc, ws, uw, zl_acc, nnz_acc,
-                                      max_acc, wmax_acc);
-#pragma unroll
-                    for (int e = 0; e < 9; ++e) ust[e * SF_NG] = uw[e];
-                    __syncwarp();
-                    // 2 frames x 36 position quads: 4 pixels x 4 digits -> one 32-bit word per plane
-#pragma unroll
-                    for (int tt = 0; tt < 3; ++tt) {
-                        const int qi = lane + 32 * tt;
-                        if (qi < 72) {
-                            const int fh = qi / 36, pq = qi - 36 * fh;
-                            const uint4 w = *reinterpret_cast<const uint4*>(ustage + fh * SF_P + 4 * pq);
-                            const unsigned int t0 = __byte_perm(w.x, w.y, 0x5140), t1 = __byte_perm(w.z, w.w, 0x5140);
-                            const unsigned int t2 = __byte_perm(w.x, w.y, 0x7362), t3 = __byte_perm(w.z, w.w, 0x7362);
-                            unsigned char* dst = bP + ((size_t)(pq >> 2) * FC + (fw + fh)) * 16 + 4 * (pq & 3);
-                            const size_t pstride = (size_t)9 * FC * 16;
-                            *reinterpret_cast<unsigned int*>(dst) = __byte_perm(t0, t1, 0x5410);
-                            *reinterpret_cast<unsigned int*>(dst + pstride) = __byte_perm(t0, t1, 0x7632);
-                            *reinterpret_cast<unsigned int*>(dst + 2 * pstride) = __byte_perm(t2, t3, 0x5410);
-                            *reinterpret_cast<unsigned int*>(dst + 3 * pstride) = __byte_perm(t2, t3, 0x7632);
-                        }
-                    }
-                    __syncwarp();
                 }
+                __syncwarp();
             }
             fence_proxy_async_smem();                             // my writes -> visible to the storer's TMA stores
             __syncwarp();
@@ -237,7 +205,7 @@ __device__ __forceinline__ void sf_group(const ShrinkFlatArgs& a, const float* T
         }
 }
 
-template <int MODE, int XP>
+template <int MODE>
 __global__ void __launch_bounds__(32 * (SF_NCW + 2), 1)
 shrink_flat_kernel(const __grid_constant__ CUtensorMap mapD, const __grid_constant__ CUtensorMap mapS, const __grid_constant__ CUtensorMap mapY,
                    const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensorMap mapVC, ShrinkFlatArgs a) {
@@ -296,7 +264,6 @@ shrink_flat_kernel(const __grid_constant__ CUtensorMap mapD, const __grid_consta
     if (warp == 0) {
         // ===================== loader =====================
         if (lane == 0) {
-            const uint64_t pol = l2_policy_evict_first();          // everything is touched once
             int q = 0;
             for (long long g0 = tile0; g0 < tile1; g0 += SF_TG) {
                 const int gt = (int)min((long long)SF_TG, tile1 - g0);
@@ -310,13 +277,10 @@ shrink_flat_kernel(const __grid_constant__ CUtensorMap mapD, const __grid_consta
                         unsigned char* b = ring + (size_t)s * stage_bytes;
                         mbar_expect_tx(&full[s], (uint32_t)(2 * slot) + (uint32_t)(FC * SF_KMAX * sizeof(float)));
                         tma_load_2d(Vst + (size_t)s * FC * SF_KMAX, &mapVC, &full[s], 0, c * FC);
-                        if (a.policy & 1) {
-                            tma_load_3d_hint(b, &mapD, &full[s], i0, j0, c * FC, pol);
-                            tma_load_3d_hint(b + slot, &mapY, &full[s], i0, j0, c * FC, pol);
-                        } else {
-                            tma_load_3d(b, &mapD, &full[s], i0, j0, c * FC);
-                            tma_load_3d(b + slot, &mapY, &full[s], i0, j0, c * FC);
-                        }
+                        // no L2 evict_first hint: on these loads it cost 2 % per solve, on the stores nothing (94.4 ms without,
+                        // 96.4 on the loads, 94.4 on the stores; 1080p x 300, profiles/r2r_shrink_variants.log)
+                        tma_load_3d(b, &mapD, &full[s], i0, j0, c * FC);
+                        tma_load_3d(b + slot, &mapY, &full[s], i0, j0, c * FC);
                     }
             }
         }
@@ -324,7 +288,6 @@ shrink_flat_kernel(const __grid_constant__ CUtensorMap mapD, const __grid_consta
     } else if (warp == 1) {
         // ===================== storer =====================
         if (lane == 0) {
-            const uint64_t pol = l2_policy_evict_first();
             int q = 0;
             for (long long g0 = tile0; g0 < tile1; g0 += SF_TG) {
                 const int gt = (int)min((long long)SF_TG, tile1 - g0);
@@ -335,22 +298,10 @@ shrink_flat_kernel(const __grid_constant__ CUtensorMap mapD, const __grid_consta
                         const int s = q % NS;
                         mbar_wait(&done[s], (uint32_t)((q / NS) & 1));
                         unsigned char* b = ring + (size_t)s * stage_bytes;
-                        if (a.policy & 2) {
-                            if (write_S) tma_store_3d_hint(&mapS, b, i0, j0, c * FC, pol);
-                            tma_store_3d_hint(&mapY, b + slot, i0, j0, c * FC, pol);
-                        } else {
-                            if (write_S) tma_store_3d(&mapS, b, i0, j0, c * FC);
-                            tma_store_3d(&mapY, b + slot, i0, j0, c * FC);
-                        }
-                        if (XP == 1) {
-                            const int nh = FC >> 3;                     // boxes of 8 frames (128-byte rows, swizzled)
-                            for (int sl = 0; sl < 4; ++sl)
-                                for (int hf = 0; hf < nh; ++hf)
-                                    tma_store_3d(&mapQ, b + 2 * slot + (size_t)(sl * nh + hf) * (9 * 128), 2 * (c * FC + 8 * hf), (int)((g0 + t) * 9), sl);
-                        } else {
-                            for (int sl = 0; sl < 4; ++sl)
-                                tma_store_3d(&mapQ, b + 2 * slot + (size_t)sl * 9 * FC * 16, 2 * c * FC, (int)((g0 + t) * 9), sl);
-                        }
+                        if (write_S) tma_store_3d(&mapS, b, i0, j0, c * FC);
+                        tma_store_3d(&mapY, b + slot, i0, j0, c * FC);
+                        for (int sl = 0; sl < 4; ++sl)
+                            tma_store_3d(&mapQ, b + 2 * slot + (size_t)sl * 9 * FC * 16, 2 * c * FC, (int)((g0 + t) * 9), sl);
                         tma_store_commit();
                         tma_store_wait_read<0>();
                         sf_mbar_arrive(&freeb[s]);
@@ -374,7 +325,7 @@ shrink_flat_kernel(const __grid_constant__ CUtensorMap mapD, const __grid_consta
             }
             sf_cp_async_wait_all();
             sf_bar_sync(1, SF_NTC);
-#define SF_CALL(KR_) sf_group<KR_, MODE, XP>(a, Tb, gt, ring, stage_bytes, Vst, ustage, full, done, q, lane, cw, sc, write_S, zl_acc, nnz_acc, max_acc, wmax_acc)
+#define SF_CALL(KR_) sf_group<KR_, MODE>(a, Tb, gt, ring, stage_bytes, Vst, ustage, full, done, q, lane, cw, sc, write_S, zl_acc, nnz_acc, max_acc, wmax_acc)
             switch (r) {
                 case 0: SF_CALL(0); break;
                 case 1: SF_CALL(1); break;
@@ -415,11 +366,8 @@ bool make_shrink_flat_plan(int n, int rows, int cols, long long ld, int num_sms,
     if (sp.R != SF_R || rows % 4 != 0) return false;
     ShrinkFlatPlan p;
     p.n = n; p.rows = rows; p.cols = cols; p.ld = ld;
-    const char* env_fc = getenv("BSUB_FLAT_FC");
-    const char* env_ns = getenv("BSUB_FLAT_STAGES");
-    p.FC = env_fc ? atoi(env_fc) : 16;
-    if (p.FC != 32) p.FC = 16;
-    p.NS = env_ns ? atoi(env_ns) : 8;
+    p.FC = 16;
+    p.NS = 8;
     while (p.NS >= 3 && sf_smem_bytes(p.FC, p.NS) > SF_SMEM_CAP) --p.NS;
     if (p.NS < 3) return false;
     p.nchunkf = (n + p.FC - 1) / p.FC;
@@ -443,8 +391,6 @@ int make_shrink_flat_maps(const ShrinkFlatPlan& p, const float* D, float* S, flo
     const uint64_t qstrides[2] = {(uint64_t)16 * p.n, (uint64_t)ldq * (uint64_t)p.n};
     const uint32_t qbox[3] = {(uint32_t)(2 * p.FC), 9u, 1u};
     if (make_tensor_map_u64(&m->Q, Wq, 3, qdims, qstrides, qbox) != 0) return -1;
-    const uint32_t qsbox[3] = {16u, 9u, 1u};                                   // 8 frames x 16 B = one 128-byte swizzle row per unit
-    if (make_tensor_map_u64_swz(&m->Qs, Wq, 3, qdims, qstrides, qsbox, 128) != 0) return -1;
     if (vstride < SF_KMAX) { set_error("shrink_flat: VC row stride %d < %d", vstride, SF_KMAX); return -1; }
     const uint64_t vdims[2] = {(uint64_t)vstride, (uint64_t)p.n};
     const uint64_t vstrides[1] = {(uint64_t)vstride * sizeof(float)};
@@ -498,12 +444,12 @@ int launch_rebuild_S(const ShrinkFlatPlan& p, const float* D, const float* Y, fl
     return 0;
 }
 
-template <int MODE, int XP>
+template <int MODE>
 static int launch_sf(const ShrinkFlatPlan& p, const ShrinkFlatMaps& maps, const ShrinkFlatArgs& a, cudaStream_t stream) {
     static unsigned long long attr_devs = 0;
     if (first_call_on_device(&attr_devs))
-        BSUB_CUDA_CHECK(cudaFuncSetAttribute(shrink_flat_kernel<MODE, XP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SF_SMEM_CAP));
-    shrink_flat_kernel<MODE, XP><<<p.grid, 32 * (SF_NCW + 2), p.smem_bytes, stream>>>(maps.D, maps.S, maps.Y, XP == 1 ? maps.Qs : maps.Q, maps.VC, a);
+        BSUB_CUDA_CHECK(cudaFuncSetAttribute(shrink_flat_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SF_SMEM_CAP));
+    shrink_flat_kernel<MODE><<<p.grid, 32 * (SF_NCW + 2), p.smem_bytes, stream>>>(maps.D, maps.S, maps.Y, maps.Q, maps.VC, a);
     BSUB_CUDA_CHECK(cudaGetLastError());
     return 0;
 }
@@ -511,22 +457,11 @@ static int launch_sf(const ShrinkFlatPlan& p, const ShrinkFlatMaps& maps, const 
 int launch_shrink_flat(const ShrinkFlatPlan& p, const ShrinkFlatMaps& maps, const float* Tt, DevState* st, int mode, int force_S, double* part_zz,
                        unsigned long long* part_nnz, float* part_max, float* part_wmax, cudaStream_t stream) {
     ShrinkFlatArgs a;
-    a.s_stale_next = &st->s_stale_next; a.force_S = (force_S || getenv("BSUB_FLAT_ALWAYS_S") != nullptr) ? 1 : 0;
+    a.s_stale_next = &st->s_stale_next; a.force_S = force_S ? 1 : 0;
     a.Tt = Tt; a.n = p.n; a.rows = p.rows; a.cols = p.cols; a.FC = p.FC; a.NS = p.NS; a.nchunkf = p.nchunkf; a.ntile_r = p.ntile_r;
     a.ntiles = p.ntiles; a.st = st; a.part_zz = part_zz; a.part_nnz = part_nnz; a.part_max = part_max; a.part_wmax = part_wmax; a.mode = mode;
-    { const char* e = getenv("BSUB_FLAT_PROBE"); a.probe = e ? atoi(e) : 0; }
-    // measured (scripts/r2_variants.py, 1080p x 300, ms per solve): policy 3: 96.7, 1: 96.4, 2: 94.4, 0: 94.4 -- the evict_first hint on the
-    // loads costs 2 %, on the stores nothing
-    { const char* e = getenv("BSUB_FLAT_POLICY"); a.policy = e ? atoi(e) : 0; }
-    // BSUB_FLAT_XPOSE: 0 = transposition staged through shared memory (default), 1 = in registers with swizzled 8-frame plane boxes
-    // (conflict-free, but 128-byte runs in HBM), 2 = in registers with the dense 16-frame boxes (256-byte runs, 4-way conflicts on 9
-    // stores).  Measured (same script, policy 0): 94.4 / 100.5 / 94.7 ms per solve -- the 171 M bank-conflict wavefronts of variant 0
-    // (ncu r2p) are not what bounds the kernel, and the shorter HBM runs of variant 1 cost 13 % of the kernel.
-    const int xp = []() { const char* e = getenv("BSUB_FLAT_XPOSE"); const int v = e ? atoi(e) : 0; return (v < 0 || v > 2) ? 0 : v; }();
-#define SF_LAUNCH(MODE_) (xp == 0 ? launch_sf<MODE_, 0>(p, maps, a, stream) : xp == 1 ? launch_sf<MODE_, 1>(p, maps, a, stream) : launch_sf<MODE_, 2>(p, maps, a, stream))
-    if (mode == SHRINK_L1) return SF_LAUNCH(SHRINK_L1);
-    if (mode == SHRINK_FLAT3) return SF_LAUNCH(SHRINK_FLAT3);
-#undef SF_LAUNCH
+    if (mode == SHRINK_L1) return launch_sf<SHRINK_L1>(p, maps, a, stream);
+    if (mode == SHRINK_FLAT3) return launch_sf<SHRINK_FLAT3>(p, maps, a, stream);
     set_error("shrink_flat: mode %d is not handled by this kernel", mode);
     return -1;
 }

@@ -19,7 +19,6 @@
 // named barriers of the per-tile T reduction.  No thread-block clusters, no cross-CTA exchange.
 // HBM traffic: read D,S,Y + write S,Y = 20 B per matrix element, + 4 B for the digit planes (+ the part of the 8 B
 // phase-B re-read that misses L2).
-#include <stdlib.h>
 #include <algorithm>
 #include "common.cuh"
 #include "kernels.h"
@@ -31,6 +30,7 @@ namespace bsub {
 constexpr int SS_KC = 16;                 // largest rank handled by this kernel (a plan may cap it at 8 to fit Vr, VC of long clips)
 constexpr int SS_KRED = 8;                // singular vectors per round of the per-tile T reduction
 constexpr size_t SS_SMEM_CAP = 227 * 1024 - 256;
+constexpr int SS_NCW = 8;                 // consumer warps (block = 32 * (SS_NCW + 2))
 
 struct ShrinkStreamArgs {
     float* T; const float* Vr; const float* VC; int vstride;
@@ -254,16 +254,15 @@ __device__ __forceinline__ void ss_phase_b(const ShrinkStreamArgs& a, float* rin
     }
 }
 
-// NCW: consumer warps (block = 32 * (NCW + 2)).  RT / FCT: tile rows and frames per stage as compile-time constants
-// (0 = take them from the arguments): with the default plan (48 rows, 28 frames) every index computation of the inner
-// loops folds into immediates and shifts.
-template <int NCW, int RT, int FCT>
-__global__ void __launch_bounds__(32 * (NCW + 2), 1)
+// RT / FCT: tile rows and frames per stage as compile-time constants (0 = take them from the arguments): with the default
+// plan (48 rows, 28 frames) every index computation of the inner loops folds into immediates and shifts.
+template <int RT, int FCT>
+__global__ void __launch_bounds__(32 * (SS_NCW + 2), 1)
 shrink_stream_kernel(const __grid_constant__ CUtensorMap mapD, const __grid_constant__ CUtensorMap mapS,
                      const __grid_constant__ CUtensorMap mapY, const __grid_constant__ CUtensorMap mapOut,
                      const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensorMap mapVr,
                      const __grid_constant__ CUtensorMap mapVC, ShrinkStreamArgs a) {
-    constexpr int NTC = 32 * NCW;
+    constexpr int NTC = 32 * SS_NCW;
     const DevState* st = a.st;
     if (st->done) return;
     const int r = st->svp;
@@ -276,7 +275,7 @@ shrink_stream_kernel(const __grid_constant__ CUtensorMap mapD, const __grid_cons
         return;
     }
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int R = RT ? RT : a.R, P = 3 * R, NQ = P / 4, NFL = (32 * NCW) / NQ, FC = FCT ? FCT : a.FC, NS = a.NS;
+    const int R = RT ? RT : a.R, P = 3 * R, NQ = P / 4, NFL = (32 * SS_NCW) / NQ, FC = FCT ? FCT : a.FC, NS = a.NS;
     const int BS = (RT && FCT) ? ((FCT * 3 * RT + 127) / 128 * 128) : a.BS, QS = (RT && FCT) ? ((FCT * 3 * RT + 127) / 128 * 128) : a.QS;
     const double mu_d = st->mu;
     const float inv_mu = (float)(1.0 / mu_d), mu_f = (float)mu_d;
@@ -305,7 +304,7 @@ shrink_stream_kernel(const __grid_constant__ CUtensorMap mapD, const __grid_cons
     __shared__ double redd[32];
 
     if (threadIdx.x == 0) {
-        for (int s = 0; s < NS; ++s) { mbar_init(&full[s], 1); mbar_init(&done[s], NCW); mbar_init(&freeb[s], 1); }
+        for (int s = 0; s < NS; ++s) { mbar_init(&full[s], 1); mbar_init(&done[s], SS_NCW); mbar_init(&freeb[s], 1); }
         mbar_fence_init();
         tma_prefetch_desc(&mapD); tma_prefetch_desc(&mapS); tma_prefetch_desc(&mapY); tma_prefetch_desc(&mapOut);
         tma_prefetch_desc(&mapVr); tma_prefetch_desc(&mapVC);
@@ -474,9 +473,9 @@ shrink_stream_kernel(const __grid_constant__ CUtensorMap mapD, const __grid_cons
 }
 
 // -------------------------------------------------------------------------------------------------------------
-static size_t ss_smem_bytes(int n, int R, int FC, int NS, int NTC) {
+static size_t ss_smem_bytes(int n, int R, int FC, int NS) {
     (void)n;
-    const int P = 3 * R, NQ = P / 4, NFL = NTC / NQ;
+    const int P = 3 * R, NQ = P / 4, NFL = 32 * SS_NCW / NQ;
     const size_t bs = ((size_t)FC * P + 127) / 128 * 128;
     size_t fl = (size_t)NS * 3 * bs + (size_t)NFL * SS_KRED * P + (size_t)SS_KC * 4 * R + (size_t)NS * ((FC * SS_KC + 31) / 32 * 32) + 32;
     return fl * sizeof(float) + (size_t)3 * NS * sizeof(uint64_t) + 64;
@@ -486,12 +485,7 @@ bool make_shrink_stream_plan(int n, int rows, int cols, long long ld, int num_sm
     if (rows % 4 != 0 || rows < 12) return false;
     ShrinkStreamPlan p;
     p.n = n; p.rows = rows; p.cols = cols; p.ld = ld;
-    const char* env_w = getenv("BSUB_STREAM_WARPS");
-    const char* env_ns = getenv("BSUB_STREAM_STAGES");
-    const char* env_fc = getenv("BSUB_STREAM_FC");
-    int NCW = env_w ? atoi(env_w) : 8;
-    if (NCW != 16) NCW = 8;
-    const int NTC = 32 * NCW;
+    const int NTC = 32 * SS_NCW;
     int R = R_hint > 0 ? ((R_hint + 11) / 12) * 12 : 48;
     const int rows12 = ((rows + 11) / 12) * 12;
     R = std::min(std::min(R, rows12), 252);
@@ -499,14 +493,13 @@ bool make_shrink_stream_plan(int n, int rows, int cols, long long ld, int num_sm
         const int NQ = 3 * R / 4;
         if (NQ > NTC) continue;
         const int NFL = NTC / NQ;
-        int FC = env_fc ? atoi(env_fc) : 4 * NFL;
-        FC = std::max(1, std::min(FC, std::min(n, 256)));
-        int NS = env_ns ? atoi(env_ns) : 6;
-        while (NS >= 3 && ss_smem_bytes(n, R, FC, NS, NTC) > SS_SMEM_CAP) --NS;
+        const int FC = std::max(1, std::min(4 * NFL, std::min(n, 256)));
+        int NS = 6;
+        while (NS >= 3 && ss_smem_bytes(n, R, FC, NS) > SS_SMEM_CAP) --NS;
         if (NS < 3) continue;
-        p.R = R; p.P = 3 * R; p.FC = FC; p.NS = NS; p.NCW = NCW; p.kcap = SS_KC;
+        p.R = R; p.P = 3 * R; p.FC = FC; p.NS = NS; p.kcap = SS_KC;
         p.bufstride = (int)(((size_t)FC * p.P + 127) / 128 * 128);
-        p.smem_bytes = ss_smem_bytes(n, R, FC, NS, NTC);
+        p.smem_bytes = ss_smem_bytes(n, R, FC, NS);
         p.nchunkf = (n + FC - 1) / FC;
         p.ntile_r = (rows + R - 1) / R;
         p.ntile_c = (cols + 2) / 3;
@@ -560,15 +553,15 @@ int make_shrink_stream_qmap(const ShrinkStreamPlan& p, signed char* Wq, ShrinkTm
     return 0;
 }
 
-template <int NCW, int RT, int FCT>
+template <int RT, int FCT>
 static int launch_ss(const ShrinkStreamPlan& p, const ShrinkTmaMaps& maps, const ShrinkStreamArgs& a, int mode, cudaStream_t stream) {
     static unsigned long long attr_devs = 0;      // one bit per device: the attribute is per (function, device)
     if (first_call_on_device(&attr_devs)) {
-        BSUB_CUDA_CHECK(cudaFuncSetAttribute(shrink_stream_kernel<NCW, RT, FCT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SS_SMEM_CAP));
+        BSUB_CUDA_CHECK(cudaFuncSetAttribute(shrink_stream_kernel<RT, FCT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SS_SMEM_CAP));
     }
     const CUtensorMap& outmap = (mode == SHRINK_SPILL) ? maps.U : maps.S;
-    shrink_stream_kernel<NCW, RT, FCT><<<p.grid, 32 * (NCW + 2), p.smem_bytes, stream>>>(maps.D, maps.S, maps.Y, outmap, maps.Q, maps.Vr,
-                                                                                        maps.VC, a);
+    shrink_stream_kernel<RT, FCT><<<p.grid, 32 * (SS_NCW + 2), p.smem_bytes, stream>>>(maps.D, maps.S, maps.Y, outmap, maps.Q, maps.Vr,
+                                                                                      maps.VC, a);
     BSUB_CUDA_CHECK(cudaGetLastError());
     return 0;
 }
@@ -578,17 +571,15 @@ int launch_shrink_stream(const ShrinkStreamPlan& p, const ShrinkTmaMaps& maps, S
     if (mode == SHRINK_SPILL && !maps.has_U) { set_error("shrink_stream: spill buffer map missing"); return -1; }
     ShrinkStreamArgs a;
     a.T = b.T; a.Vr = b.Vr; a.VC = b.VC; a.vstride = b.vstride; a.ld = p.ld; a.n = p.n; a.rows = p.rows; a.cols = p.cols;
-    a.R = p.R; a.P = p.P; a.NQ = p.P / 4; a.NFL = (32 * p.NCW) / a.NQ; a.FC = p.FC; a.NS = p.NS; a.BS = p.bufstride;
+    a.R = p.R; a.P = p.P; a.NQ = p.P / 4; a.NFL = (32 * SS_NCW) / a.NQ; a.FC = p.FC; a.NS = p.NS; a.BS = p.bufstride;
     a.nchunkf = p.nchunkf; a.ntile_r = p.ntile_r; a.ntiles = p.ntiles; a.st = st; a.part_zz = b.part_zz; a.part_nnz = b.part_nnz;
     a.part_max = b.part_max; a.part_wmax = b.part_wmax; a.mode = mode;
     a.wq = (maps.has_Q && b.part_wmax != nullptr) ? 1 : 0; a.Pq = p.P; a.implied_first = b.implied_first; a.kcap = p.kcap;
     a.Tt = (mode != SHRINK_SPILL) ? b.Tt : nullptr;
     a.have_flat = (mode != SHRINK_SPILL) ? b.have_flat : 0;
     a.QS = (int)(((size_t)p.FC * p.P + 127) / 128 * 128);
-    if (p.NCW == 16) return launch_ss<16, 0, 0>(p, maps, a, mode, stream);
-    if (p.R == 48 && p.FC == 28) return launch_ss<8, 48, 28>(p, maps, a, mode, stream);
-    if (p.R == 48 && p.FC == 32) return launch_ss<8, 48, 32>(p, maps, a, mode, stream);
-    return launch_ss<8, 0, 0>(p, maps, a, mode, stream);
+    if (p.R == 48 && p.FC == 28) return launch_ss<48, 28>(p, maps, a, mode, stream);
+    return launch_ss<0, 0>(p, maps, a, mode, stream);
 }
 
 }  // namespace bsub

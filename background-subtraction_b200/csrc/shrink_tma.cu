@@ -13,10 +13,10 @@
 //     exchanged through L2 around ONE hardware cluster barrier;
 //   * sweep 2 builds a = D - L in place, runs the prox + dual update per 3x3 group in shared memory, and the
 //     results leave through two TMA box stores (S and Y; out-of-image elements are clipped by the hardware).
-// Two or three CTAs share an SM so that the barrier / exchange bubbles of one tile are filled by another CTA.
+// Two CTAs share an SM (one when no tile fits half of shared memory) so that the barrier / exchange bubbles of one tile
+// are filled by another CTA.
 // HBM traffic is exactly read D,S,Y + write S,Y = 20 B per matrix element.
 #include <cooperative_groups.h>
-#include <stdlib.h>
 #include <algorithm>
 #include "common.cuh"
 #include "kernels.h"
@@ -28,6 +28,7 @@ namespace bsub {
 
 constexpr int ST_KC = 8;          // singular vectors per register chunk
 constexpr size_t ST_SMEM_CAP = 227 * 1024 - 256;
+constexpr int ST_NT = 256;         // threads per CTA
 
 struct ShrinkTmaArgs {
     float* T; float* tpart; const float* Vr; const float* VC; int vstride;
@@ -123,8 +124,7 @@ __device__ __forceinline__ void sweep2a_sub(float* bD, const float* Tp, const fl
         default: { constexpr int K_ = 8; CALL; } break; \
     }
 
-template <int NT, int MINB>
-__global__ void __launch_bounds__(NT, MINB)
+__global__ void __launch_bounds__(ST_NT, 2)
 shrink_tma_kernel(const __grid_constant__ CUtensorMap mapD, const __grid_constant__ CUtensorMap mapS,
                   const __grid_constant__ CUtensorMap mapY, const __grid_constant__ CUtensorMap mapOut, ShrinkTmaArgs a) {
     const DevState* st = a.st;
@@ -167,7 +167,7 @@ shrink_tma_kernel(const __grid_constant__ CUtensorMap mapD, const __grid_constan
     }
     auto load_V = [&](int kc) {                           // Vr / VC rows of my frames for singular vectors [8kc, 8kc+8)
         const int k0 = kc * ST_KC;
-        for (int idx = tid; idx < nfr * ST_KC; idx += NT) {
+        for (int idx = tid; idx < nfr * ST_KC; idx += ST_NT) {
             const int f = idx / ST_KC, k = idx - f * ST_KC;
             const bool ok = (k0 + k) < r;
             Vr_s[idx] = ok ? a.Vr[(size_t)(f0 + f) * a.vstride + k0 + k] : 0.f;
@@ -237,7 +237,7 @@ shrink_tma_kernel(const __grid_constant__ CUtensorMap mapD, const __grid_constan
                 }
                 __syncthreads();
                 const int kend = min(KR, kcnt - kr0);
-                for (int idx = tid; idx < kend * NQ; idx += NT) {
+                for (int idx = tid; idx < kend * NQ; idx += ST_NT) {
                     const int k = idx / NQ, q = idx - k * NQ;
                     float4 sum = make_float4(0.f, 0.f, 0.f, 0.f);
                     for (int l = 0; l < NFL; ++l) {
@@ -249,7 +249,7 @@ shrink_tma_kernel(const __grid_constant__ CUtensorMap mapD, const __grid_constan
             }
             // all partials of the cluster are in place (this is also the CTA barrier after the reduction)
             cluster.sync();
-            for (int idx = tid; idx < kcnt * NQ; idx += NT) {
+            for (int idx = tid; idx < kcnt * NQ; idx += ST_NT) {
                 const int k = idx / NQ, q = idx - k * NQ;
                 float4 sum = make_float4(0.f, 0.f, 0.f, 0.f);
                 for (int rk = 0; rk < a.Cf; ++rk) {                 // fixed order: every CTA gets bit-identical T
@@ -275,7 +275,7 @@ shrink_tma_kernel(const __grid_constant__ CUtensorMap mapD, const __grid_constan
             if (nchunk > 1) {
                 __syncthreads();
                 load_V(kc);
-                for (int idx = tid; idx < kcnt * NQ; idx += NT) {
+                for (int idx = tid; idx < kcnt * NQ; idx += ST_NT) {
                     const int k = idx / NQ, q = idx - k * NQ;
                     *reinterpret_cast<float4*>(Tp + (size_t)k * P + 4 * q) =
                         *reinterpret_cast<const float4*>(myscratch + (size_t)(k0 + k) * P + 4 * q);
@@ -289,7 +289,7 @@ shrink_tma_kernel(const __grid_constant__ CUtensorMap mapD, const __grid_constan
         // ---------------- sweep 2b: prox + dual update in shared memory (S_new -> bS, Y_new -> bY) ----------------
         if (a.mode == SHRINK_FLAT3) {
             const int NG = R / 3;
-            for (int itx = tid; itx < nfr * NG; itx += NT) {
+            for (int itx = tid; itx < nfr * NG; itx += ST_NT) {
                 const int f = itx / NG, g = itx - f * NG;
                 const float* dsp = bD + (size_t)f * P + 3 * g;
                 float* ssp = bS + (size_t)f * P + 3 * g;
@@ -338,7 +338,7 @@ shrink_tma_kernel(const __grid_constant__ CUtensorMap mapD, const __grid_constan
                 zz_acc += (double)zl;
             }
         } else if (a.mode == SHRINK_L1) {
-            for (int itx = tid; itx < nfr * P; itx += NT) {
+            for (int itx = tid; itx < nfr * P; itx += ST_NT) {
                 const float av = bD[itx], yv = bY[itx];
                 const float x = av + yv * inv_mu;
                 const float sv = copysignf(fmaxf(fabsf(x) - lamq, 0.f), x);
@@ -349,7 +349,7 @@ shrink_tma_kernel(const __grid_constant__ CUtensorMap mapD, const __grid_constan
                 max_acc = fmaxf(max_acc, fabsf(sv));
             }
         } else {   // SHRINK_SPILL: G_S goes out through mapOut (= U); the dual update happens in lowrank_kernel<true>
-            for (int itx = tid; itx < nfr * P; itx += NT) bS[itx] = bD[itx] + bY[itx] * inv_mu;
+            for (int itx = tid; itx < nfr * P; itx += ST_NT) bS[itx] = bD[itx] + bY[itx] * inv_mu;
         }
         fence_proxy_async_smem();          // my generic writes -> visible to the TMA store
         __syncthreads();
@@ -378,8 +378,8 @@ shrink_tma_kernel(const __grid_constant__ CUtensorMap mapD, const __grid_constan
 }
 
 // -------------------------------------------------------------------------------------------------------------
-static size_t st_smem_bytes(int n, int R, int Cf, int KR, int NT) {
-    const int P = 3 * R, NQ = P / 4, NFL = NT / NQ;
+static size_t st_smem_bytes(int n, int R, int Cf, int KR) {
+    const int P = 3 * R, NQ = P / 4, NFL = ST_NT / NQ;
     const int nf = (n + Cf - 1) / Cf;
     const size_t bs = ((size_t)nf * P + 31) / 32 * 32;
     size_t fl = (size_t)6 * bs + (size_t)NFL * KR * P + (size_t)3 * ST_KC * P + (size_t)2 * nf * ST_KC;
@@ -390,18 +390,11 @@ bool make_shrink_tma_plan(int n, int rows, int cols, long long ld, int num_sms, 
     if (rows % 4 != 0 || rows < 12) return false;               // TMA global strides must be multiples of 16 B
     ShrinkTmaPlan p;
     p.n = n; p.rows = rows; p.cols = cols; p.ld = ld;
-    const char* env_nt = getenv("BSUB_SHRINK_THREADS");
-    const char* env_occ = getenv("BSUB_SHRINK_OCC");
-    int NT = env_nt ? atoi(env_nt) : 256;
-    if (NT != 512) NT = 256;
-    int occ = env_occ ? atoi(env_occ) : 2;                      // CTAs per SM the shared-memory budget is sized for
-    if (NT == 512) occ = 1;
-    if (occ < 1) occ = 1;
-    if (occ > 3) occ = 3;
+    int occ = 2;                                                // CTAs per SM the shared-memory budget is sized for
     const int rows12 = ((rows + 11) / 12) * 12;
     auto cap_for = [&](int o) { return (size_t)((228 * 1024) / o - 1024 - 512); };
     auto fits = [&](int Rr, int Cc, int Kr, int o) {
-        return (n + Cc - 1) / Cc <= 256 && 3 * Rr / 4 <= NT && st_smem_bytes(n, Rr, Cc, Kr, NT) <= std::min(cap_for(o), ST_SMEM_CAP);
+        return (n + Cc - 1) / Cc <= 256 && 3 * Rr / 4 <= ST_NT && st_smem_bytes(n, Rr, Cc, Kr) <= std::min(cap_for(o), ST_SMEM_CAP);
     };
     int R = 0, Cf = 0, KR = 0;
     for (; occ >= 1 && R == 0; --occ) {
@@ -416,11 +409,9 @@ bool make_shrink_tma_plan(int n, int rows, int cols, long long ld, int num_sms, 
         if (R != 0) break;
     }
     if (R == 0) return false;
-    if (occ < 1) occ = 1;
-    p.NT = NT; p.occ = occ;
     p.R = R; p.P = 3 * R; p.Cf = Cf; p.nf = (n + Cf - 1) / Cf; p.KR = KR;
     p.bufstride = (int)(((size_t)p.nf * p.P + 31) / 32 * 32);
-    p.smem_bytes = st_smem_bytes(n, R, Cf, KR, NT);
+    p.smem_bytes = st_smem_bytes(n, R, Cf, KR);
     p.ntile_r = (rows + R - 1) / R;
     p.ntile_c = (cols + 2) / 3;
     p.ntiles = (long long)p.ntile_r * p.ntile_c;
@@ -448,36 +439,29 @@ int make_shrink_tma_maps(const ShrinkTmaPlan& p, const float* D, float* S, float
     return 0;
 }
 
-template <int NT, int MINB>
-static int launch_st(const ShrinkTmaPlan& p, const ShrinkTmaMaps& maps, const ShrinkTmaArgs& a, int mode, cudaStream_t stream) {
+int launch_shrink_tma(const ShrinkTmaPlan& p, const ShrinkTmaMaps& maps, ShrinkBuffers b, const DevState* st, int mode,
+                      int min_rank, cudaStream_t stream) {
+    if (mode == SHRINK_SPILL && !maps.has_U) { set_error("shrink_tma: spill buffer map missing"); return -1; }
+    ShrinkTmaArgs a;
+    a.T = b.T; a.tpart = b.tpart; a.Vr = b.Vr; a.VC = b.VC; a.vstride = b.vstride; a.ld = p.ld; a.n = p.n; a.rows = p.rows;
+    a.cols = p.cols; a.R = p.R; a.P = p.P; a.NQ = p.P / 4; a.NFL = ST_NT / a.NQ; a.Cf = p.Cf; a.nf = p.nf; a.KR = p.KR;
+    a.BS = p.bufstride;
+    a.ntile_r = p.ntile_r; a.ntiles = p.ntiles; a.nclusters = p.grid_clusters; a.st = st; a.part_zz = b.part_zz;
+    a.part_nnz = b.part_nnz; a.part_max = b.part_max; a.mode = mode; a.min_rank = min_rank;
     static unsigned long long attr_devs = 0;      // one bit per device: the attribute is per (function, device)
     if (first_call_on_device(&attr_devs)) {
-        BSUB_CUDA_CHECK(cudaFuncSetAttribute(shrink_tma_kernel<NT, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ST_SMEM_CAP));
+        BSUB_CUDA_CHECK(cudaFuncSetAttribute(shrink_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ST_SMEM_CAP));
     }
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(p.grid_clusters * p.Cf); cfg.blockDim = dim3(NT);
+    cfg.gridDim = dim3(p.grid_clusters * p.Cf); cfg.blockDim = dim3(ST_NT);
     cfg.dynamicSmemBytes = p.smem_bytes; cfg.stream = stream;
     cudaLaunchAttribute at[1];
     at[0].id = cudaLaunchAttributeClusterDimension;
     at[0].val.clusterDim.x = p.Cf; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
     cfg.attrs = at; cfg.numAttrs = 1;
     const CUtensorMap& outmap = (mode == SHRINK_SPILL) ? maps.U : maps.S;
-    BSUB_CUDA_CHECK(cudaLaunchKernelEx(&cfg, shrink_tma_kernel<NT, MINB>, maps.D, maps.S, maps.Y, outmap, a));
+    BSUB_CUDA_CHECK(cudaLaunchKernelEx(&cfg, shrink_tma_kernel, maps.D, maps.S, maps.Y, outmap, a));
     return 0;
-}
-
-int launch_shrink_tma(const ShrinkTmaPlan& p, const ShrinkTmaMaps& maps, ShrinkBuffers b, const DevState* st, int mode,
-                      int min_rank, cudaStream_t stream) {
-    if (mode == SHRINK_SPILL && !maps.has_U) { set_error("shrink_tma: spill buffer map missing"); return -1; }
-    ShrinkTmaArgs a;
-    a.T = b.T; a.tpart = b.tpart; a.Vr = b.Vr; a.VC = b.VC; a.vstride = b.vstride; a.ld = p.ld; a.n = p.n; a.rows = p.rows;
-    a.cols = p.cols; a.R = p.R; a.P = p.P; a.NQ = p.P / 4; a.NFL = p.NT / a.NQ; a.Cf = p.Cf; a.nf = p.nf; a.KR = p.KR;
-    a.BS = p.bufstride;
-    a.ntile_r = p.ntile_r; a.ntiles = p.ntiles; a.nclusters = p.grid_clusters; a.st = st; a.part_zz = b.part_zz;
-    a.part_nnz = b.part_nnz; a.part_max = b.part_max; a.mode = mode; a.min_rank = min_rank;
-    if (p.NT == 512) return launch_st<512, 1>(p, maps, a, mode, stream);
-    if (p.occ >= 3) return launch_st<256, 3>(p, maps, a, mode, stream);
-    return launch_st<256, 2>(p, maps, a, mode, stream);
 }
 
 }  // namespace bsub

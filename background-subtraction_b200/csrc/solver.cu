@@ -372,8 +372,7 @@ int bsub_create(const bsub_config* cfg, bsub_solver** out) {
                 if (s->m % r == 0) { rows = r; cols = (int)(s->m / r); break; }
         }
         s->sp = make_shrink_plan(s->n, rows, cols, s->ld, s->num_sms, cfg->tile_rows, cfg->cluster_frames);
-        s->use_tma = (getenv("BSUB_NO_TMA") == nullptr) &&
-                     make_shrink_tma_plan(s->n, rows, cols, s->ld, s->num_sms, cfg->tile_rows, cfg->cluster_frames, &s->stp);
+        s->use_tma = make_shrink_tma_plan(s->n, rows, cols, s->ld, s->num_sms, cfg->tile_rows, cfg->cluster_frames, &s->stp);
         s->use_stream = s->use_tma && (getenv("BSUB_NO_STREAM") == nullptr) &&
                         make_shrink_stream_plan(s->n, rows, cols, s->ld, s->num_sms, cfg->tile_rows, &s->ssp);
         ALLOC(s->tpart, sizeof(float) * std::max(s->sp.tpart_floats, s->use_tma ? s->stp.tpart_floats : (size_t)0));
@@ -387,7 +386,7 @@ int bsub_create(const bsub_config* cfg, bsub_solver** out) {
         if (s->use_i8) {
             const long long ldq = shrink_stream_ldq(s->ssp);
             s->gip = make_gram_i8_plan(s->n, ldq, s->num_sms);
-            s->gip.m_real = (getenv("BSUB_NO_GRAM_BIAS") == nullptr) ? s->m : 0;
+            s->gip.m_real = s->m;
             s->gip.m_global = s->cfg.m_global;
             std::vector<int4> info; std::vector<int> blkn;
             fill_gram_i8_tables(s->gip, info, blkn);
@@ -420,7 +419,7 @@ int bsub_create(const bsub_config* cfg, bsub_solver** out) {
             default: s->shrink_mode = SHRINK_SPILL; break;
         }
         s->implied_first = s->use_i8 && s->use_stream && s->shrink_mode != SHRINK_SPILL && s->cfg.use_sv_prediction &&
-                           s->cfg.sv0 >= 1 && s->cfg.sv0 <= s->ssp.kcap && getenv("BSUB_NO_IMPLIED_FIRST") == nullptr;
+                           s->cfg.sv0 >= 1 && s->cfg.sv0 <= s->ssp.kcap;
         if (s->shrink_mode == SHRINK_SPILL) { ALLOC(s->U, mat); ALLOC(s->L, mat); cudaMemset(s->U, 0, mat); cudaMemset(s->L, 0, mat); }
 #undef ALLOC
         if (cudaGetLastError() != cudaSuccess) { /* clear sticky-less errors from memset probing */ }
@@ -1122,7 +1121,7 @@ int bsub_mask_stats_local(bsub_solver* s, int phase, void* stream) {
         CK(cudaMemsetAsync(s->comm_max, 0, sizeof(double) * 8, st));
         // one shard holding the whole matrix: max |S| is what the last shrink pass reported; shards need the pass (the
         // per-iteration maximum is not all-reduced)
-        if (s->cfg.m_global == s->m && s->iters_enqueued > 0 && getenv("BSUB_MASK_ABSMAX") == nullptr)
+        if (s->cfg.m_global == s->m && s->iters_enqueued > 0)
             return launch_maxS_from_state(s->st, s->comm_max + 1, st);
         return launch_absmax(s->S, s->ld, s->m, s->n, s->comm_max + 1, st);
     }

@@ -14,9 +14,6 @@ int make_tensor_map_f32(CUtensorMap* map, const void* base, int rank, const uint
 // 8-byte-element tensor map (no swizzle): lets one box row span up to 2 KB of contiguous bytes (boxDim <= 256 elements)
 int make_tensor_map_u64(CUtensorMap* map, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
                         const uint32_t* box);
-// the same with a shared-memory swizzle (inner box extent * 8 bytes <= swizzle_bytes)
-int make_tensor_map_u64_swz(CUtensorMap* map, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
-                            const uint32_t* box, int swizzle_bytes);
 // uint8 tensor map; swizzle_bytes in {0, 32, 64, 128}
 int make_tensor_map_u8(CUtensorMap* map, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
                        const uint32_t* box, int swizzle_bytes);

@@ -50,7 +50,7 @@ O.inexact_alm_lsd(D6, groups=g6, log=olog)
 print("oracle n600 svp", [l['svp'] for l in olog])
 for l in olog[-3:]:
     print("  oracle iter", l['iter'], "sigma*mu", np.round(l['sigma'] * l['mu'], 5))
-for env in ({}, {"BSUB_NO_EIG_FAST": "1"}, {"BSUB_NO_GRAM_BIAS": "1"}, {"BSUB_NO_I8": "1"}, {"BSUB_NO_FLAT": "1"}, {"BSUB_NO_PROJ": "1"}):
+for env in ({}, {"BSUB_NO_EIG_FAST": "1"}, {"BSUB_NO_I8": "1"}, {"BSUB_NO_FLAT": "1"}, {"BSUB_NO_PROJ": "1"}):
     def run():
         dec = B.lsd_decomposition(D6, groups=g6, img_shape=(48, 60))
         return [l['svp'] for l in dec.log()], dec.counters()
@@ -59,7 +59,7 @@ for env in ({}, {"BSUB_NO_EIG_FAST": "1"}, {"BSUB_NO_GRAM_BIAS": "1"}, {"BSUB_NO
 # ---- 3. WaterSurface delta = 1
 Dw, _x, _m = O.normalize_and_center(ws)
 gw = B.get_proximal_flat_groups_nonoverlap((128, 160), (3, 3))
-for env in ({}, {"BSUB_NO_EIG_FAST": "1"}, {"BSUB_NO_GRAM_BIAS": "1"}, {"BSUB_NO_I8": "1"}):
+for env in ({}, {"BSUB_NO_EIG_FAST": "1"}, {"BSUB_NO_I8": "1"}):
     def run():
         dec = B.lsd_decomposition(Dw, groups=gw, delta=1)
         lg = dec.log()

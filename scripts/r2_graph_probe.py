@@ -27,6 +27,6 @@ for rep in range(2 if len(sys.argv) <= 4 else 1):
     torch.cuda.synchronize(); dt = time.perf_counter() - t0
     out = (ctypes.c_int64 * 4)()
     C.check(dec.lib.bsub_debug_graph(dec.h, out))
-    print("%dx%dx%d rep %d ms %.1f iters %d conv %d | prox outer iterations: last call %d, total %d over %d calls, %d calls hit the cap (count factor %s)"
-          % (rows, cols, n, rep, dt * 1e3, st.iter, st.converged, out[0], out[1], out[2], out[3], os.environ.get("BSUB_GRAPH_COUNT_FACTOR", "8")), flush=True)
+    print("%dx%dx%d rep %d ms %.1f iters %d conv %d | prox outer iterations: last call %d, total %d over %d calls, %d calls hit the cap"
+          % (rows, cols, n, rep, dt * 1e3, st.iter, st.converged, out[0], out[1], out[2], out[3]), flush=True)
 print("svp", [l['svp'] for l in dec.log()], "err", ["%.2e" % l['err'] for l in dec.log()])
